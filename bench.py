@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the WEALY retrieval-and-scoring hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision fp16x3|fp16]
-                    [--legs main,c1,c3,c4,c5,f1]
+                    [--legs main,c1,c3,c4,c5,f1] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -36,6 +36,13 @@ The other BASELINE.json configs ride on the same JSON line as extra keys (each a
            the timed code is the oracle port: torch matmul similarity + per-query argsort
            evaluator) on all host cores, on a bounded query sample of the same workload.  This arm
            never loads the CUDA library.
+
+`--dump-outputs DIR`: after the timed steps, what the timed path returned in its last step goes to DIR/<name>.npy
+           (float32 / float64): per-query `aps` and `r1s` and the `sums` {sum AP, sum R1, #scored}.  The inputs are
+           seeded, so two builds run with the same arguments can be compared output for output: `aps` and `r1s`
+           repeat bit for bit, while sum AP is a float64 reduction on the device whose last bits vary from run to run.
+
+The benchmark writes nothing into the tree it runs from (which may be read-only).
 """
 import argparse
 import importlib.util
@@ -48,12 +55,14 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # no __pycache__ in the tree for the modules imported from here on
 
 METRIC = "similarity+MAP eval Gpairs/s at 1/2/4/8 B200 (roofline frac); MAP parity"
 UNIT = "Gpairs/s"
 BASE_N = 100_000
 DIM = 1024
 FALLBACK_PEAKS = {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
 
 
 def load_peaks():
@@ -138,6 +147,30 @@ class ClockSampler(threading.Thread):
         return {"sm_mhz": s[len(s) // 2], "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons)}
 
 
+def dump_outputs(out_dir, per_query, totals, query_rows=None):
+    """Writes `per_query` (name -> [n] tensor) and `totals` (name -> small tensor) to out_dir/<name>.npy, float64 tensors
+    as float64 and the rest as float32.  `query_rows` (the workload's row of each of the n queries, default 0 .. n-1) goes
+    to query_index.npy when given.  Past DUMP_LIMIT_BYTES the per-query arrays keep the same fixed, seeded sample of
+    queries, and query_index.npy says which."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    as_np = lambda t: (t.double() if t.dtype == torch.float64 else t.float()).cpu().numpy()
+    arrays = {k: as_np(v) for k, v in per_query.items()}
+    n = len(next(iter(arrays.values())))
+    rows = None if query_rows is None else np.asarray(query_rows, dtype=np.float64)
+    keep = min(n, (DUMP_LIMIT_BYTES - 64 * 1024) // (sum(a.itemsize for a in arrays.values()) + 8))
+    if keep < n:
+        pick = np.sort(torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].numpy())
+        arrays = {k: a[pick] for k, a in arrays.items()}
+        rows = (np.arange(n, dtype=np.float64) if rows is None else rows)[pick]
+    if rows is not None:
+        arrays["query_index"] = rows
+    arrays.update({k: as_np(v) for k, v in totals.items()})
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def physical_gpu_index(local_rank):
     vis = os.environ.get("CUDA_VISIBLE_DEVICES")
     if vis:
@@ -189,11 +222,13 @@ def run_reference_arm(args):
     for it in range(args.warmup + args.steps):
         lo = (it * sample) % max(1, n_total - sample)
         t0 = time.perf_counter()
-        oev.evaluate_argsort(s["c"][lo:lo + sample], s["i"][lo:lo + sample], s["z"][lo:lo + sample],
-                             s["c"], s["i"], s["z"], dist_fn=dist_fn)
+        aps, r1s = oev.evaluate_argsort(s["c"][lo:lo + sample], s["i"][lo:lo + sample], s["z"][lo:lo + sample],
+                                        s["c"], s["i"], s["z"], dist_fn=dist_fn)[:2]
         dt = time.perf_counter() - t0
         if it >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:   # this arm scores a window of queries per step: the last step's window, with its rows
+        dump_outputs(args.dump_outputs, {"aps": aps, "r1s": r1s}, {}, query_rows=range(lo, lo + aps.numel()))
     sec = sum(times) / len(times)
     value = sample * n_total / sec / 1e9
     line = {
@@ -569,6 +604,8 @@ def run_gpu_arm(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_step = float(t.item()) / args.steps
     value = pairs_total / (ms_step * 1e-3) / 1e9
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"aps": res["aps"], "r1s": res["r1s"]}, {"sums": res["sums"]})
     s_host = res["sums"].double().cpu()
     gpu_map, gpu_mr1 = float(s_host[0] / s_host[2]), float(s_host[1] / s_host[2])
     passes = 3 if args.precision == "fp16x3" else 1
@@ -622,7 +659,7 @@ def run_gpu_arm(args):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    e2e_steps = max(2, min(args.steps, 5))
+    e2e_steps = args.steps
     step_e2e()
     step_e2e()
     single_ms = timed_e2e(lambda: [step_e2e() for _ in range(e2e_steps)]) / e2e_steps
@@ -790,10 +827,19 @@ def run_gpu_arm(args):
         dist.destroy_process_group()
 
 
+def positive_int(text):
+    v = int(text)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {v}")
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=positive_int, default=5,
+                    help="timed steps of the headline workload and of each of its end-to-end forms; the extra legs "
+                         "(c1, c3, c4, c5, f1) time fixed step counts of their own")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--tracks", type=int, default=0,
@@ -806,6 +852,8 @@ def main():
                          "more candidates above the relevant items; diagnostic only)")
     ap.add_argument("--legs", default="main,c1,c3,c4,c5,f1",
                     help="which BASELINE configs to run besides the headline (c1, c3, c4, c5); 'main' = headline only")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (at most 64 MB in all)")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3

@@ -127,6 +127,34 @@ def test_bench_arms_share_one_config():
     assert hasattr(synth, "make_eval_set")
 
 
+def test_bench_dump_stays_under_its_limit_with_a_fixed_sample(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 / float64 .npy files; an output past the size limit keeps the same seeded sample
+    of queries in every run, with the sampled query indices beside it."""
+    import importlib.util
+    ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = importlib.util.spec_from_file_location("_bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    n = 50_000
+    aps, r1s, sums = torch.rand(n), torch.arange(1, n + 1, dtype=torch.float32), torch.tensor([1.0, 2.0, 3.0], dtype=torch.float64)
+    bench.dump_outputs(str(tmp_path / "full"), {"aps": aps, "r1s": r1s}, {"sums": sums})
+    assert sorted(os.listdir(tmp_path / "full")) == ["aps.npy", "r1s.npy", "sums.npy"]
+    assert np.load(tmp_path / "full" / "aps.npy").dtype == np.float32 and np.load(tmp_path / "full" / "sums.npy").dtype == np.float64
+    assert np.array_equal(np.load(tmp_path / "full" / "aps.npy"), aps.numpy())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 64 * 1024 + 160_000)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), {"aps": aps, "r1s": r1s}, {"sums": sums})
+        assert sum(f.stat().st_size for f in (tmp_path / run).iterdir()) <= bench.DUMP_LIMIT_BYTES
+    rows = np.load(tmp_path / "a" / "query_index.npy")
+    assert rows.dtype == np.float64 and 0 < rows.size < n and np.all(np.diff(rows) > 0)
+    for name in ("query_index", "aps", "r1s", "sums"):
+        assert np.array_equal(np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "r1s.npy"), rows.astype(np.float32) + 1)
+    monkeypatch.setattr("sys.argv", ["bench.py", "--steps", "0"])
+    with pytest.raises(SystemExit):
+        bench.main()
+
+
 def test_host_route_is_only_offered_for_one_pinned_matrix(monkeypatch):
     """evaluate() hands embeddings to wealy_eval_run_host only when the device can read them itself: ONE pinned host
     matrix on both sides, big enough for the pipeline to pay; everything else keeps copy-then-compute.  (No GPU here:

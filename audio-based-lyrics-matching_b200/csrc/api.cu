@@ -494,7 +494,19 @@ static int launch_gemm_pair(const Planes& a, const GemmShape& sh, const typename
 // traffic of the single-CTA kernel, which is what bounds these sweeps (WEALY_RECT_PAIR=0 selects the single-CTA kernel).
 template <class Epi>
 static int launch_gemm_rect(int passes, const Planes& a, const Planes& b, GemmShape& sh, const typename Epi::Params& ep,
-                            cudaStream_t s);
+                            cudaStream_t s, int shard_rank = 0, int shard_world = 1);
+
+// Multi-GPU sweeps: restrict a launch shape to the row blocks rb = shard_rank (mod shard_world) -- round-robin, so that
+// the triangle of a symmetric sweep is shared evenly.  Applied to the shape the kernel reads (super row blocks on the
+// CTA-pair core), after any halving.
+static void shard_row_blocks(GemmShape& sh, int shard_rank, int shard_world) {
+  if (shard_world <= 1) return;
+  const int total_owned = sh.n_row_blocks;
+  sh.rb_stride = shard_world;
+  sh.rb_offset = shard_rank;
+  sh.n_row_blocks = shard_rank < total_owned ? (int)ceil_div(total_owned - shard_rank, shard_world) : 0;
+  if (sh.group_rows > sh.n_row_blocks) sh.group_rows = sh.n_row_blocks > 0 ? sh.n_row_blocks : 1;
+}
 
 template <class Epi>
 static int launch_gemm(int passes, const Planes& a, const Planes& b, GemmShape& sh, const typename Epi::Params& ep,
@@ -509,11 +521,16 @@ static int launch_gemm(int passes, const Planes& a, const Planes& b, GemmShape& 
 
 template <class Epi>
 static int launch_gemm_rect(int passes, const Planes& a, const Planes& b, GemmShape& sh, const typename Epi::Params& ep,
-                            cudaStream_t s) {
-  if (env_int("WEALY_RECT_PAIR", 1) == 0 || sh.n_row_blocks < 2) return launch_gemm<Epi>(passes, a, b, sh, ep, s);
+                            cudaStream_t s, int shard_rank, int shard_world) {
+  if (env_int("WEALY_RECT_PAIR", 1) == 0 || sh.n_row_blocks < 2) {
+    GemmShape shs = sh;
+    shard_row_blocks(shs, shard_rank, shard_world);
+    return launch_gemm<Epi>(passes, a, b, shs, ep, s);
+  }
   GemmShape shp = sh;
   shp.n_row_blocks = (sh.n_row_blocks + 1) / 2;  // super row blocks of 256 queries
   shp.group_rows = (sh.group_rows + 1) / 2;
+  shard_row_blocks(shp, shard_rank, shard_world);
   if (passes == 3) {
     if (a.lo == nullptr || b.lo == nullptr) return fail(WEALY_ERR_BAD_ARG, "3-pass contraction needs lo planes");
     shp.k_blocks = (int)(a.d_pad / 32);
@@ -798,6 +815,7 @@ struct wealy_eval_plan {
   bool timed = false;
   bool finished = false;  // the last run included ap_reduce (+ top-k finalize)
   bool last_sym = false;  // the last sweep ran in the clique-sorted view (its counters are in that CSR order)
+  int staged_chunks = 0;  // chunks of the last staged prepare (0 none); > 1: the summed buffer is thr alone
   // wealy_eval_run_host: [0] "planes allocated" on the run's stream, [1 + k] "rows of part k have arrived" on the upload stream
   cudaEvent_t host_ev[1 + 8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   // wealy_eval_plan_create_host: plane rows [early_lo, end) of this matrix are already in flight on the upload stream
@@ -1029,16 +1047,20 @@ static int topk_capacity(int k) {
 // counts are left in the plan's histogram for the caller to sum over ranks (finish == false).
 // chunks > 1 (row f1): every track has `chunks` embeddings (rows t * chunks .. of the matrices), the kS x kS chunk
 // similarities are reduced to one per track pair inside the epilogue (redux: WEALY_REDUX_*), all ids / outputs per track.
+// A sharded chunked sweep (shard_world > 1) takes the row blocks rb = shard_rank (mod shard_world) of the launched shape:
+// the half sweep's pairs score their row and their column query, the rectangle's rows are complete -- either way the
+// counters summed over the ranks are those of the whole sweep.
 template <int kS>
 static int launch_eval_tracks(int passes, const Planes& a, const Planes& b, GemmShape& sh, const EvalParams& ep, cudaStream_t s,
-                              bool sym) {
-  if (!sym) return launch_gemm_rect<EvalTracksEpi<kS>>(passes, a, b, sh, ep, s);
+                              bool sym, int shard_rank, int shard_world) {
+  if (!sym) return launch_gemm_rect<EvalTracksEpi<kS>>(passes, a, b, sh, ep, s, shard_rank, shard_world);
   // chunked all-vs-all: only the tiles that reach above the diagonal, on the CTA-pair core (super row block S = rows
   // [256 S, 256 S + 256) needs column tiles >= S); every track pair scores both its row and its column query
   GemmShape shp = sh;
   shp.n_row_blocks = (sh.n_row_blocks + 1) / 2;
   shp.group_rows = (sh.group_rows + 1) / 2;
   shp.sym = 1;
+  shard_row_blocks(shp, shard_rank, shard_world);
   if (passes == 3) {
     shp.k_blocks = (int)(a.d_pad / 32);
     return launch_gemm_pair<EvalTracksSymEpi<kS>, 3, 32, 8, false>(a, shp, ep, s);
@@ -1051,7 +1073,7 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
                          float* r1s, double* sums, int64_t* topk_idx, float* topk_sim, int shard_rank,
                          int shard_world, bool finish, void* stream, int chunks = 1, int redux = WEALY_REDUX_MIN,
                          const int* q_len = nullptr, const int* c_len = nullptr, bool allow_sym_topk = true, int stage = 0) {
-  // stage (sharded symmetric sweep only): 0 = everything in one call; 1 = prep + the relevant similarities of THIS
+  // stage (sharded all-vs-all sweeps only): 0 = everything in one call; 1 = prep + the relevant similarities of THIS
   // rank's share of the queries, then return (the caller sums the threshold buffer over the ranks); 2 = the sweep,
   // on the planes and thresholds stage 1 left in the plan
   cudaStream_t s = (cudaStream_t)stream;
@@ -1069,6 +1091,8 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
   if (stage != 2 && (!queries_z || !candidates_z)) return fail(WEALY_ERR_BAD_ARG, "null pointer");
   if (stage == 2) {
     if (!p->planes_buf || !p->lvl_thr_buf) return fail(WEALY_ERR_BAD_ARG, "wealy_eval_shard_sweep needs wealy_eval_shard_prepare first");
+    if (chunks > 1 ? p->staged_chunks != chunks : p->staged_chunks > 1)
+      return fail(WEALY_ERR_BAD_ARG, "the staged sweep needs a prepare of the same layout (%d chunks per track)", chunks);
     queries_z = candidates_z = p;  // (not dereferenced: the planes are in the plan)
   }
   if (finish && (!aps || !r1s || !sums)) return fail(WEALY_ERR_BAD_ARG, "null pointer");
@@ -1108,9 +1132,9 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
                         shard_world == 1 && allow_sym_topk && env_int("WEALY_SYM_TOPK", 1) != 0;
   const bool sym = can_sym && (topk == 0 ? (shard_world > 1 || env_int("WEALY_SYM", 1) != 0) : sym_topk);
   // chunked tracks, all-vs-all: the same halving for reductions that give d(q, c) == d(c, q) (min / max / mean)
-  const bool sym_tracks = same && p->same_ids && chunks > 1 && topk == 0 && red_inner == red_outer && shard_world == 1 &&
-                          nq * chunks > 2 * kTileM && env_int("WEALY_SYM_TRACKS", 1) != 0;
-  if (shard_world > 1 && !sym)
+  const bool all_tracks = same && p->same_ids && chunks > 1 && topk == 0;
+  const bool sym_tracks = all_tracks && red_inner == red_outer && nq * chunks > 2 * kTileM && env_int("WEALY_SYM_TRACKS", 1) != 0;
+  if (shard_world > 1 && !sym && !all_tracks)
     return fail(WEALY_ERR_BAD_ARG, "a sharded sweep needs queries == candidates (ids and embeddings) and no top-k");
 
   // operand planes (cached allocation)
@@ -1133,7 +1157,8 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
     CU_TRY(cudaEventCreate(&p->ev1));
     for (cudaEvent_t& e : p->evs) CU_TRY(cudaEventCreate(&e));
   }
-  if (stage != 0 && !(sym && shard_world > 1)) return fail(WEALY_ERR_BAD_ARG, "staged runs belong to the sharded symmetric sweep");
+  if (stage != 0 && !((sym || all_tracks) && shard_world > 1))
+    return fail(WEALY_ERR_BAD_ARG, "staged runs belong to the sharded all-vs-all sweep");
   if (stage != 2) CU_TRY(cudaEventRecord(p->evs[0], s));
   if (stage != 2) {
     W_TRY(launch_prep(queries_z, ld_q, rows_q, d, dtype, kPrepL2AddEps, eps, pq, nullptr, nullptr, 0, nullptr, 0, s,
@@ -1165,10 +1190,18 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
       pos_sort_sorted_kernel<<<blocks, threads, 0, s>>>(p->s_npos, (int)nq, (int)p->s_padded, p->s_off, p->raw, p->thr,
                                                         p->cnt, p->s_lvl, p->s_cinfo, q_lo, q_hi);
     } else if (chunks > 1) {
-      if (nq > 0) pos_thresholds_tracks_kernel<<<(unsigned)nq, threads, 0, s>>>(pq.hi, pq.lo, pc.hi, pc.lo, (int)pq.d_pad, chunks, red_inner,
-                                                              red_outer, red_scale, p->q_i, (int)nq, p->sorted_idx,
-                                                              p->c_i, p->seg_lo, p->seg_len, p->off, p->raw, p->thr,
-                                                              p->lim, p->cnt, q_len, c_len);
+      // stage 1: this rank's contiguous share of the query tracks, on a zeroed thr (its CSR rows are disjoint from the
+      // other ranks', so the sum over the ranks assembles the whole of it); cnt / lim are rebuilt by stage 2
+      int q_lo = 0, q_hi = (int)nq;
+      if (stage == 1) {
+        q_lo = (int)(nq * shard_rank / shard_world);
+        q_hi = (int)(nq * (shard_rank + 1) / shard_world);
+        CU_TRY(cudaMemsetAsync(p->thr, 0, (size_t)(p->total_pairs > 0 ? p->total_pairs : 1) * 4, s));
+      }
+      if (q_hi > q_lo)
+        pos_thresholds_tracks_kernel<<<(unsigned)(q_hi - q_lo), threads, 0, s>>>(
+            pq.hi, pq.lo, pc.hi, pc.lo, (int)pq.d_pad, chunks, red_inner, red_outer, red_scale, p->q_i, (int)nq, p->sorted_idx,
+            p->c_i, p->seg_lo, p->seg_len, p->off, p->raw, p->thr, p->lim, p->cnt, q_len, c_len, q_lo);
     } else if (same && p->same_ids && nq > 0 && env_int("WEALY_KPOS_BLOCKS", 1) != 0) {
       // all-vs-all through the rectangle sweep (top-k requested): the clique-block tensor-core K_pos of the symmetric
       // path on the caller's row order (every unordered pair's operands are read once per 16 x 8 block, not per pair)
@@ -1186,9 +1219,14 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
     CU_TRY(cudaGetLastError());
   }
   if (stage == 1) {
-    p->last_sym = true;
+    p->last_sym = sym;
     p->last_stream = s;
+    p->staged_chunks = chunks;
     return WEALY_OK;
+  }
+  if (stage == 2 && chunks > 1) {
+    track_limits_kernel<<<(unsigned)ceil_div(nq, 256), 256, 0, s>>>(p->off, p->thr, (int)nq, p->lim, p->cnt);
+    CU_TRY(cudaGetLastError());
   }
   // ---- top-k in the symmetric sweep: sampled pre-pass -> per-query lower bound of the k-th best similarity
   float* tk_val = nullptr;
@@ -1318,13 +1356,8 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
       if (sh.group_rows > sh.n_row_blocks) sh.group_rows = std::max(1, sh.n_row_blocks);
     }
   }
-  if (shard_world > 1) {
-    const int total_owned = sh.n_row_blocks;
-    sh.rb_stride = shard_world;
-    sh.rb_offset = shard_rank;
-    sh.n_row_blocks = shard_rank < total_owned ? (int)ceil_div(total_owned - shard_rank, shard_world) : 0;
-    if (sh.group_rows > sh.n_row_blocks) sh.group_rows = sh.n_row_blocks > 0 ? sh.n_row_blocks : 1;
-  }
+  // (chunked tracks: launch_eval_tracks shards the shape it launches, after halving it into super row blocks)
+  if (sym) shard_row_blocks(sh, shard_rank, shard_world);
   if (sym) {
     sh.sym = 1;
     EvalSymParams sp;
@@ -1393,13 +1426,13 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
       W_TRY((launch_gemm_t<EvalSymEpi<3>, 1, 64, 8, 3>(pq, pc, sh, sp, s)));
     }
   } else if (chunks == 2) {
-    W_TRY(launch_eval_tracks<2>(passes, pq, pc, sh, ep, s, sym_tracks));
+    W_TRY(launch_eval_tracks<2>(passes, pq, pc, sh, ep, s, sym_tracks, shard_rank, shard_world));
   } else if (chunks == 4) {
-    W_TRY(launch_eval_tracks<4>(passes, pq, pc, sh, ep, s, sym_tracks));
+    W_TRY(launch_eval_tracks<4>(passes, pq, pc, sh, ep, s, sym_tracks, shard_rank, shard_world));
   } else if (chunks == 8) {
-    W_TRY(launch_eval_tracks<8>(passes, pq, pc, sh, ep, s, sym_tracks));
+    W_TRY(launch_eval_tracks<8>(passes, pq, pc, sh, ep, s, sym_tracks, shard_rank, shard_world));
   } else if (chunks == 16) {
-    W_TRY(launch_eval_tracks<16>(passes, pq, pc, sh, ep, s, sym_tracks));
+    W_TRY(launch_eval_tracks<16>(passes, pq, pc, sh, ep, s, sym_tracks, shard_rank, shard_world));
   } else {
     W_TRY(launch_gemm_rect<EvalEpi>(passes, pq, pc, sh, ep, s));
   }
@@ -1875,9 +1908,51 @@ extern "C" int wealy_eval_shard_prepare(wealy_eval_plan* p, const void* z, int64
 extern "C" int wealy_eval_plan_thresholds(const wealy_eval_plan* p, void** values, int64_t* count) {
   if (!p || !values || !count) return fail(WEALY_ERR_BAD_ARG, "null pointer");
   if (!p->lvl_thr_buf) return fail(WEALY_ERR_BAD_ARG, "the plan is not an all-vs-all plan");
+  if (p->staged_chunks > 1) {  // chunked tracks: the thresholds in the caller's CSR order, nothing else
+    *values = p->thr;
+    *count = p->total_pairs > 0 ? p->total_pairs : 1;
+    return WEALY_OK;
+  }
   *values = p->lvl_thr_buf;
   *count = p->s_padded * 4 + (p->total_pairs > 0 ? p->total_pairs : 1);
   return WEALY_OK;
+}
+
+// Chunked tracks (chunks in {2, 4, 8, 16}, redux WEALY_REDUX_*, lens = NULL or the ragged chunk counts of every track):
+// the same three steps.  min / max / mean take the half sweep, the other reductions (and small sets, WEALY_SYM_TRACKS=0)
+// the rectangle sweep; either way sharded by row blocks.
+static int check_shard_tracks(const wealy_eval_plan* p, int chunks, int shard_rank, int shard_world) {
+  if (!p) return fail(WEALY_ERR_BAD_ARG, "null plan");
+  if (!p->same_ids) return fail(WEALY_ERR_BAD_ARG, "a sharded sweep needs queries == candidates (ids and embeddings) and no top-k");
+  if (chunks != 2 && chunks != 4 && chunks != 8 && chunks != 16)
+    return fail(WEALY_ERR_UNSUPPORTED, "chunked tracks have 2, 4, 8 or 16 chunks, got %d", chunks);
+  if (shard_world < 1 || shard_rank < 0 || shard_rank >= shard_world) return fail(WEALY_ERR_BAD_ARG, "bad shard %d/%d", shard_rank, shard_world);
+  return WEALY_OK;
+}
+
+extern "C" int wealy_eval_sweep_shard_tracks(wealy_eval_plan* p, const void* z, int64_t ld, int64_t d, int dtype, float eps,
+                                             int passes, int chunks, int redux, const int32_t* lens, int shard_rank,
+                                             int shard_world, void* stream) {
+  W_TRY(check_shard_tracks(p, chunks, shard_rank, shard_world));
+  return eval_run_impl(p, z, ld, z, ld, d, dtype, eps, passes, 0, nullptr, nullptr, nullptr, nullptr, nullptr, shard_rank,
+                       shard_world, false, stream, chunks, redux, lens, lens);
+}
+
+extern "C" int wealy_eval_shard_prepare_tracks(wealy_eval_plan* p, const void* z, int64_t ld, int64_t d, int dtype, float eps,
+                                               int passes, int chunks, int redux, const int32_t* lens, int shard_rank,
+                                               int shard_world, void* stream) {
+  W_TRY(check_shard_tracks(p, chunks, shard_rank, shard_world));
+  if (shard_world < 2) return fail(WEALY_ERR_BAD_ARG, "staged sweeps are for two or more ranks");
+  return eval_run_impl(p, z, ld, z, ld, d, dtype, eps, passes, 0, nullptr, nullptr, nullptr, nullptr, nullptr, shard_rank,
+                       shard_world, false, stream, chunks, redux, lens, lens, true, 1);
+}
+
+extern "C" int wealy_eval_shard_sweep_tracks(wealy_eval_plan* p, int64_t d, int passes, int chunks, int redux,
+                                             const int32_t* lens, int shard_rank, int shard_world, void* stream) {
+  W_TRY(check_shard_tracks(p, chunks, shard_rank, shard_world));
+  if (shard_world < 2) return fail(WEALY_ERR_BAD_ARG, "staged sweeps are for two or more ranks");
+  return eval_run_impl(p, nullptr, 0, nullptr, 0, d, WEALY_F32, 0.f, passes, 0, nullptr, nullptr, nullptr, nullptr, nullptr,
+                       shard_rank, shard_world, false, stream, chunks, redux, lens, lens, true, 2);
 }
 
 extern "C" int wealy_eval_shard_sweep(wealy_eval_plan* p, int64_t d, int passes, int shard_rank, int shard_world, void* stream) {

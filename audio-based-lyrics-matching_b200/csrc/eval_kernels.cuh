@@ -149,17 +149,17 @@ __device__ __forceinline__ void mma_16x8x16(float (&c)[4], const unsigned (&a)[4
 // are candidate chunks -- 16 / kS whole candidates per tile for kS <= 8 (eight two-chunk tracks, two eight-chunk
 // tracks), one for kS = 16 -- and the 8 tile COLUMNS the query's chunks (two tiles for kS = 16), so a warp reads the
 // query's rows once for all the candidates of its tile.  Two accumulators take alternate k windows (the dependent MMA
-// chain is what bounds a warp).
+// chain is what bounds a warp).  Block b takes query track q_lo + b (a multi-GPU run gives every rank a share).
 __global__ void __launch_bounds__(256) pos_thresholds_tracks_kernel(
     const __half* __restrict__ q_hi, const __half* __restrict__ q_lo, const __half* __restrict__ c_hi,
     const __half* __restrict__ c_lo, int d_pad, int ks, int red_inner, int red_outer, float red_scale,
     const int* __restrict__ q_i, int nq, const int* __restrict__ sorted_idx, const int* __restrict__ c_i,
     const int* __restrict__ seg_lo, const int* __restrict__ seg_len, const long long* __restrict__ off,
     float* __restrict__ raw, float* __restrict__ thr, float* __restrict__ lim, int* __restrict__ cnt,
-    const int* __restrict__ q_len, const int* __restrict__ c_len) {
+    const int* __restrict__ q_len, const int* __restrict__ c_len, int q_first) {
   // its 8 warps take the relevant candidates tile by tile, round-robin (a clique of 160 versions is a handful of
   // sequential contractions per warp); slots of the query's CSR row are handed out by a shared counter
-  const int q = (int)blockIdx.x;
+  const int q = q_first + (int)blockIdx.x;
   const int lane = (int)(threadIdx.x & 31), warp = (int)(threadIdx.x >> 5);
   __shared__ int n_sh;
   if (threadIdx.x == 0) n_sh = 0;
@@ -270,6 +270,20 @@ __global__ void __launch_bounds__(256) pos_thresholds_tracks_kernel(
     cnt[q] = n;
     lim[q] = n > 0 ? thr[o] : __int_as_float(0x7f800000);
   }
+}
+
+// Multi-GPU staged K_pos of chunked tracks: after the ranks' threshold shares have been summed, every rank rebuilds the
+// per-query values the sweep reads from the CSR offsets and the assembled thresholds, exactly as
+// pos_thresholds_tracks_kernel writes them (a query's relevant candidates are the npos[q] = off[q + 1] - off[q]
+// non-self members of its clique).  Integers never travel through the float all-reduce.
+__global__ void track_limits_kernel(const long long* __restrict__ off, const float* __restrict__ thr, int nq,
+                                    float* __restrict__ lim, int* __restrict__ cnt) {
+  const int q = (int)(blockIdx.x * blockDim.x + threadIdx.x);
+  if (q >= nq) return;
+  const long long o = off[q];
+  const int n = (int)(off[q + 1] - o);
+  cnt[q] = n;
+  lim[q] = n > 0 ? thr[o] : __int_as_float(0x7f800000);
 }
 
 // ---------------------------------------------------------------------------------------------------------

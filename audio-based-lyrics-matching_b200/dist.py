@@ -7,7 +7,8 @@ Two schemes:
   corpus and sweeps the row blocks rb = rank (mod world) of the SAME symmetric problem (only tiles above the
   diagonal, each element scoring its row and its column query).  A rank therefore holds partial rank counts for
   ALL queries; the one real exchange step of the path is an all-reduce (SUM) of those int32 counters -- the
-  "rank counts merged over NCCL" of the north star -- after which every rank owns the complete AP / R1.
+  "rank counts merged over NCCL" of the north star -- after which every rank owns the complete AP / R1.  Chunked
+  tracks ([N, s, D], SURVEY.md 8(f) row f1) shard the chunked sweep the same way for min / max / mean.
 * general queries vs corpus -- `evaluate_sharded`: queries are independent units, so rank r scores the contiguous
   query slice shard_range(Nq, r, world) against the whole (replicated) corpus with the single-GPU fused kernel and
   the data path needs no collective.  The only exchange is the result merge: one all-reduce of {sum AP, sum R1,
@@ -58,27 +59,28 @@ def gather_rows(local, n_total, group=None):
 
 
 def upload_sharded(z_host, device, group=None):
-    """Host embeddings -> the full [n, d] matrix on every rank's device without every rank pulling the whole corpus
-    over PCIe: rank r uploads only its contiguous 1/world slice of the rows (pinned host memory -> HBM), then ONE
-    all-gather over NVLink / NVSwitch replicates the corpus.  Host traffic per rank drops from n*d to n*d/world
-    bytes (8 ranks x 1.16 GB through one host bridge at 282k x 1024 was 2/3 of the end-to-end step)."""
+    """Host embeddings -> the full [n, d] matrix (or [n, s, d] chunked tracks) on every rank's device without every rank
+    pulling the whole corpus over PCIe: rank r uploads only its contiguous 1/world slice of the rows (whole tracks;
+    pinned host memory -> HBM), then ONE all-gather over NVLink / NVSwitch replicates the corpus.  Host traffic per rank
+    drops from n*d to n*d/world bytes (8 ranks x 1.16 GB through one host bridge at 282k x 1024 was 2/3 of the
+    end-to-end step)."""
     on = dist.is_available() and dist.is_initialized()
     world = dist.get_world_size(group) if on else 1
     rank = dist.get_rank(group) if on else 0
-    n, d = z_host.shape
+    n, row = z_host.shape[0], tuple(z_host.shape[1:])
     if world == 1:
         return z_host.to(device, non_blocking=True)
     chunk = -(-n // world)
     lo, hi = min(rank * chunk, n), min((rank + 1) * chunk, n)
-    mine = torch.zeros((chunk, d), dtype=z_host.dtype, device=device) if hi - lo < chunk else \
-        torch.empty((chunk, d), dtype=z_host.dtype, device=device)
+    mine = torch.zeros((chunk,) + row, dtype=z_host.dtype, device=device) if hi - lo < chunk else \
+        torch.empty((chunk,) + row, dtype=z_host.dtype, device=device)
     if hi > lo:
         mine[: hi - lo].copy_(z_host[lo:hi], non_blocking=True)
-    full = torch.empty((world * chunk, d), dtype=z_host.dtype, device=device)
+    full = torch.empty((world * chunk,) + row, dtype=z_host.dtype, device=device)
     try:
         dist.all_gather_into_tensor(full, mine, group=group)
     except (RuntimeError, NotImplementedError):      # backends without the flat variant (CPU tests)
-        dist.all_gather(list(full.view(world, chunk, d).unbind(0)), mine, group=group)
+        dist.all_gather(list(full.view((world, chunk) + row).unbind(0)), mine, group=group)
     return full[:n]
 
 
@@ -94,26 +96,56 @@ def _agree(flag, device, group=None):
 STAGED_MIN_WORLD = 4
 
 
-def sharded_step(plan, z, rank, world, *, eps=1e-6, precision=None, group=None):
+def _chunks_per_track(z, chunks, redux, q_chunks):
+    """Chunks per track of `z` ([N, s, D], or [N * s, D] with chunks=s; 1 for plain [N, D] embeddings).  Every rank
+    passes the same arguments, so whatever this refuses is refused on every rank, before any collective."""
+    from . import _native as N
+    shape = tuple(torch.as_tensor(z).shape)
+    s = shape[1] if len(shape) == 3 else (1 if chunks is None else int(chunks))
+    if len(shape) == 3 and chunks is not None and int(chunks) != s:
+        raise ValueError(f"chunks={chunks}, but z holds {s} chunks per track")
+    if s not in (1, 2, 4, 8, 16):
+        raise NotImplementedError("chunks per track must be 1, 2, 4, 8 or 16")
+    if redux not in N.REDUX:
+        raise NotImplementedError(f"redux {redux!r} is not fused into the evaluation (min / max / mean / meanmin / minmean)")
+    if q_chunks is not None and s == 1:
+        raise ValueError("chunk counts need chunked tracks")
+    return s
+
+
+def query_slice(queries_z, q_chunks, lo, hi, chunks=None):
+    """Query tracks [lo, hi) of `queries_z` ([N, D], [N, s, D], or [N * s, D] with chunks=s) and their chunk counts."""
+    s = 1 if (queries_z.ndim == 3 or chunks is None) else int(chunks)
+    return queries_z[lo * s:hi * s], None if q_chunks is None else torch.as_tensor(q_chunks)[lo:hi]
+
+
+def sharded_step(plan, z, rank, world, *, eps=1e-6, precision=None, group=None, redux="min", q_chunks=None, chunks=None):
     """The multi-GPU all-vs-all sweep up to (not including) finish(): the relevant similarities are computed once across
     the ranks (each rank its share of the queries; one all-reduce of floats assembles them -- every element has a single
     non-zero contribution, so the sum is exact), every rank sweeps the row blocks rank (mod world) of the symmetric
-    problem, and the per-(query, relevant item) rank counters are summed (the second all-reduce)."""
+    problem, and the per-(query, relevant item) rank counters are summed (the second all-reduce).  Chunked tracks
+    (`chunks`, `redux`, `q_chunks` as in EvalPlan.run) take the row-block-sharded chunked sweep the same way."""
+    kw = dict(eps=eps, precision=precision, redux=redux, q_chunks=q_chunks, chunks=chunks)
     if world >= STAGED_MIN_WORLD:
-        plan.shard_prepare(z, rank, world, eps=eps, precision=precision)
+        plan.shard_prepare(z, rank, world, **kw)
         dist.all_reduce(plan.thresholds_tensor(), op=dist.ReduceOp.SUM, group=group)
         plan.shard_sweep(rank, world)
     else:
         # two or three ranks: recomputing the relevant similarities on every rank (0.5 ms at 141k tracks) costs less
         # than the extra collective (measured at N = 2: 23.1 vs 23.5 ms per step)
-        plan.sweep_shard(z, rank, world, eps=eps, precision=precision)
+        plan.sweep_shard(z, rank, world, **kw)
     dist.all_reduce(plan.counts_tensor(), op=dist.ReduceOp.SUM, group=group)
 
 
-def evaluate_all_vs_all(c, i, z, *, precision=None, eps=1e-6, group=None, plan=None, allow_empty=False, topk=None):
+def evaluate_all_vs_all(c, i, z, *, precision=None, eps=1e-6, group=None, plan=None, allow_empty=False, topk=None,
+                        chunks=None, redux="min", q_chunks=None):
     """All-vs-all evaluation of one set (clique ids c, version ids i, embeddings z) over all ranks of `group`.
     Every rank passes the full tensors (host embeddings are uploaded 1/world per rank and all-gathered over
     NVLink).  -> dict(map, mr1, count, aps, r1s, plan); identical on every rank.
+
+    Chunked tracks (SURVEY.md 8(f) row f1): z [N, s, D] (or [N * s, D] with chunks=s), `redux` and ragged `q_chunks`
+    as in EvalPlan.run.  min / max / mean shard the chunked sweep by row blocks, like plain embeddings; meanmin /
+    minmean (d(q, c) != d(c, q), so no half sweep) take the query-partitioned scheme below.
 
     topk: per-query top-k lists are per-query state, not additive counters, so with more than one rank they take the
     query-partitioned scheme (`evaluate_sharded`: every rank scores its slice of the queries against the replicated
@@ -125,11 +157,12 @@ def evaluate_all_vs_all(c, i, z, *, precision=None, eps=1e-6, group=None, plan=N
     on = dist.is_available() and dist.is_initialized()
     rank = dist.get_rank(group) if on else 0
     world = dist.get_world_size(group) if on else 1
-    if topk and world > 1:
+    s = _chunks_per_track(z, chunks, redux, q_chunks)
+    if world > 1 and (topk or (s > 1 and redux in ("meanmin", "minmean"))):
         if not torch.as_tensor(z).is_cuda:
             z = upload_sharded(torch.as_tensor(z), torch.device("cuda", torch.cuda.current_device()), group)
         return evaluate_sharded(c, i, z, c, i, z, topk=topk, precision=precision, eps=eps, group=group,
-                                allow_empty=allow_empty)
+                                allow_empty=allow_empty, chunks=chunks, redux=redux, q_chunks=q_chunks, c_chunks=q_chunks)
     side = None
     if world > 1 and not torch.as_tensor(z).is_cuda:
         # 1/world of the rows per rank + NVLink all-gather, issued on a side stream BEFORE the id plan is built: the
@@ -149,9 +182,11 @@ def evaluate_all_vs_all(c, i, z, *, precision=None, eps=1e-6, group=None, plan=N
         raise ValueError(f"{plan.queries_without_relevant} queries have no relevant candidate "
                          "(every clique needs >= 2 versions; pass allow_empty=True to score the rest)")
     if world == 1:
-        res = plan.run(z, z, eps=eps, precision=precision, allow_empty=allow_empty, topk=topk)
+        res = plan.run(z, z, eps=eps, precision=precision, allow_empty=allow_empty, topk=topk, chunks=chunks, redux=redux,
+                       q_chunks=q_chunks)
     else:
-        sharded_step(plan, z, rank, world, eps=eps, precision=precision, group=group)
+        sharded_step(plan, z, rank, world, eps=eps, precision=precision, group=group, redux=redux, q_chunks=q_chunks,
+                     chunks=chunks)
         res = plan.finish()
     s = res["sums"].cpu()                                            # one 24-byte device -> host read
     n = max(float(s[2]), 1.0)
@@ -163,9 +198,13 @@ def evaluate_all_vs_all(c, i, z, *, precision=None, eps=1e-6, group=None, plan=N
 
 
 def evaluate_sharded(queries_c, queries_i, queries_z, candidates_c, candidates_i, candidates_z, *, topk=None,
-                     precision=None, eps=1e-6, gather=True, group=None, plan=None, allow_empty=False):
+                     precision=None, eps=1e-6, gather=True, group=None, plan=None, allow_empty=False, chunks=None,
+                     redux="min", q_chunks=None, c_chunks=None):
     """Every rank passes the FULL query / candidate tensors (or its own copy of them); rank r
     scores its slice.  Returns dict(map, mr1, count[, aps, r1s, topk_idx, topk_sim]) on every rank.
+
+    Chunked tracks: `chunks`, `redux` and the ragged `q_chunks` / `c_chunks` as in EvalPlan.run; rank r passes the chunk
+    counts of its query slice, `c_chunks` whole.
 
     A rank whose slice is empty (world > Nq) contributes nothing; a query without relevant candidates raises
     ValueError on EVERY rank (agreed on before the merge collectives) unless allow_empty."""
@@ -173,6 +212,11 @@ def evaluate_sharded(queries_c, queries_i, queries_z, candidates_c, candidates_i
     on = dist.is_available() and dist.is_initialized()
     rank = dist.get_rank(group) if on else 0
     world = dist.get_world_size(group) if on else 1
+    _chunks_per_track(queries_z, chunks, redux, q_chunks if q_chunks is not None else c_chunks)
+    if (q_chunks is None) != (c_chunks is None):
+        if queries_z is not candidates_z:
+            raise ValueError("q_chunks and c_chunks go together")
+        q_chunks = c_chunks = q_chunks if c_chunks is None else c_chunks
     nq = len(queries_c)
     lo, hi = shard_range(nq, rank, world)
     device = plan.device if plan is not None else torch.device("cuda", torch.cuda.current_device())
@@ -186,7 +230,9 @@ def evaluate_sharded(queries_c, queries_i, queries_z, candidates_c, candidates_i
                          "pass allow_empty=True to score the rest)")
     k = 0 if topk is None else min(int(topk), len(candidates_c))
     if hi > lo:
-        res = plan.run(queries_z[lo:hi], candidates_z, topk=topk, eps=eps, precision=precision, allow_empty=allow_empty)
+        qz, ql = query_slice(queries_z, q_chunks, lo, hi, chunks)
+        res = plan.run(qz, candidates_z, topk=topk, eps=eps, precision=precision, allow_empty=allow_empty, chunks=chunks,
+                       redux=redux, q_chunks=ql, c_chunks=c_chunks)
     else:                                                            # empty shard: neutral contribution
         res = {"aps": torch.empty(0, dtype=torch.float32, device=device),
                "r1s": torch.empty(0, dtype=torch.float32, device=device),

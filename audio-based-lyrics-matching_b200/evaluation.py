@@ -79,40 +79,72 @@ class EvalPlan:
             pass
 
     # ---- multi-GPU all-vs-all: symmetric sweep sharded by row blocks, rank counts summed over ranks ----
-    def sweep_shard(self, z, shard_rank, shard_world, *, eps=1e-6, precision=None):
-        """Sweep this rank's share (row blocks = shard_rank mod shard_world) of the symmetric all-vs-all
-        problem; the plan must have been built with queries == candidates."""
+    def _shard_input(self, z, chunks, redux, q_chunks):
+        """-> (z [rows, D] on the device, chunks per track, device int32 chunk counts or None) for the sharded entries;
+        chunked tracks come as [N, s, D] or as [N * s, D] with chunks=s, as in run()."""
         z = _to_device(z, self.device)
         if z.dtype == torch.float64:
             z = z.float()
-        assert z.ndim == 2 and z.shape[0] == self.nq == self.nc
+        if z.ndim == 3:
+            assert chunks is None or int(chunks) == z.shape[1]
+            chunks = z.shape[1]
+            z = z.reshape(-1, z.shape[-1])
+        s = 1 if chunks is None else int(chunks)
+        if s not in (1, 2, 4, 8, 16):
+            raise NotImplementedError("chunks per track must be 1, 2, 4, 8 or 16")
+        if redux not in N.REDUX:
+            raise NotImplementedError(f"redux {redux!r} is not fused into the evaluation (min / max / mean / meanmin / minmean)")
+        if q_chunks is not None and s == 1:
+            raise ValueError("chunk counts need chunked tracks")
+        assert z.ndim == 2 and z.shape[0] == self.nq * s and self.nq == self.nc
         if z.stride(1) != 1:
             z = z.contiguous()
-        with torch.cuda.device(self.device):
-            N.check(N.lib.wealy_eval_sweep_shard(
-                self._handle, z.data_ptr(), z.stride(0), z.shape[1], N.dtype_code(z.dtype), float(eps),
-                passes_of(precision), int(shard_rank), int(shard_world), N.stream_ptr(self.device)))
-        self._keepalive = z
+        lens = None
+        if q_chunks is not None:
+            lens = torch.as_tensor(q_chunks).to(self.device, torch.int32).contiguous()
+            assert lens.shape == (self.nq,)
+        return z, s, lens
 
-    def shard_prepare(self, z, shard_rank, shard_world, *, eps=1e-6, precision=None):
-        """Stage 1 of the sharded sweep: planes of the whole corpus, thresholds of THIS rank's share of the queries.
-        Then sum thresholds_tensor() over the ranks and call shard_sweep()."""
-        z = _to_device(z, self.device)
-        if z.dtype == torch.float64:
-            z = z.float()
-        assert z.ndim == 2 and z.shape[0] == self.nq == self.nc
-        if z.stride(1) != 1:
-            z = z.contiguous()
-        self._shard_dim, self._shard_passes = z.shape[1], passes_of(precision)
+    def sweep_shard(self, z, shard_rank, shard_world, *, eps=1e-6, precision=None, redux="min", q_chunks=None, chunks=None):
+        """Sweep this rank's share (row blocks = shard_rank mod shard_world) of the symmetric all-vs-all
+        problem; the plan must have been built with queries == candidates.  Chunked tracks ([N, s, D], or [N * s, D]
+        with chunks=s; `redux`, ragged `q_chunks` as in run()) take the row-block-sharded chunked sweep."""
+        z, s, lens = self._shard_input(z, chunks, redux, q_chunks)
         with torch.cuda.device(self.device):
-            N.check(N.lib.wealy_eval_shard_prepare(
-                self._handle, z.data_ptr(), z.stride(0), z.shape[1], N.dtype_code(z.dtype), float(eps), self._shard_passes,
-                int(shard_rank), int(shard_world), N.stream_ptr(self.device)))
-        self._keepalive = z
+            if s == 1:
+                N.check(N.lib.wealy_eval_sweep_shard(
+                    self._handle, z.data_ptr(), z.stride(0), z.shape[1], N.dtype_code(z.dtype), float(eps),
+                    passes_of(precision), int(shard_rank), int(shard_world), N.stream_ptr(self.device)))
+            else:
+                N.check(N.lib.wealy_eval_sweep_shard_tracks(
+                    self._handle, z.data_ptr(), z.stride(0), z.shape[1], N.dtype_code(z.dtype), float(eps),
+                    passes_of(precision), s, N.REDUX[redux], None if lens is None else lens.data_ptr(), int(shard_rank),
+                    int(shard_world), N.stream_ptr(self.device)))
+        self._keepalive = (z, lens)
+
+    def shard_prepare(self, z, shard_rank, shard_world, *, eps=1e-6, precision=None, redux="min", q_chunks=None,
+                      chunks=None):
+        """Stage 1 of the sharded sweep: planes of the whole corpus, thresholds of THIS rank's share of the queries.
+        Then sum thresholds_tensor() over the ranks and call shard_sweep() (which reuses this call's layout)."""
+        z, s, lens = self._shard_input(z, chunks, redux, q_chunks)
+        self._shard_dim, self._shard_passes = z.shape[1], passes_of(precision)
+        self._shard_tracks = (s, redux, lens)
+        with torch.cuda.device(self.device):
+            if s == 1:
+                N.check(N.lib.wealy_eval_shard_prepare(
+                    self._handle, z.data_ptr(), z.stride(0), z.shape[1], N.dtype_code(z.dtype), float(eps),
+                    self._shard_passes, int(shard_rank), int(shard_world), N.stream_ptr(self.device)))
+            else:
+                N.check(N.lib.wealy_eval_shard_prepare_tracks(
+                    self._handle, z.data_ptr(), z.stride(0), z.shape[1], N.dtype_code(z.dtype), float(eps),
+                    self._shard_passes, s, N.REDUX[redux], None if lens is None else lens.data_ptr(), int(shard_rank),
+                    int(shard_world), N.stream_ptr(self.device)))
+        self._keepalive = (z, lens)
 
     def thresholds_tensor(self):
-        """float32 view (no copy) of {lowest thresholds, all thresholds}: what a multi-GPU run all-reduces (SUM) between
-        shard_prepare() and shard_sweep()."""
+        """float32 view (no copy) of {lowest thresholds, all thresholds} (after a chunked shard_prepare(): the thresholds
+        alone, in the CSR order of ranks()): what a multi-GPU run all-reduces (SUM) between shard_prepare() and
+        shard_sweep()."""
         ptr, n = ctypes.c_void_p(), ctypes.c_int64()
         N.check(N.lib.wealy_eval_plan_thresholds(self._handle, ctypes.byref(ptr), ctypes.byref(n)))
 
@@ -120,13 +152,28 @@ class EvalPlan:
             __cuda_array_interface__ = {"shape": (n.value,), "typestr": "<f4", "data": (ptr.value, False), "version": 2}
         return torch.as_tensor(_Dev(), device=self.device)
 
-    def shard_sweep(self, shard_rank, shard_world):
-        """Stage 2: this rank's row blocks of the symmetric sweep on the planes / thresholds stage 1 left in the plan."""
+    def shard_sweep(self, shard_rank, shard_world, *, redux=None, q_chunks=None, chunks=None):
+        """Stage 2: this rank's row blocks of the symmetric sweep on the planes / thresholds stage 1 left in the plan.
+        redux / q_chunks / chunks default to what shard_prepare() was given; a different redux or chunks raises
+        ValueError (the thresholds were computed for those)."""
         if not hasattr(self, "_shard_dim"):
             raise AssertionError("shard_sweep() needs shard_prepare() first")
+        s, red, lens = self._shard_tracks
+        if (chunks is not None and int(chunks) != s) or (redux is not None and redux != red):
+            raise ValueError(f"shard_prepare() ran with chunks={s}, redux={red!r}")
+        if q_chunks is not None:
+            lens = torch.as_tensor(q_chunks).to(self.device, torch.int32).contiguous()
+            assert lens.shape == (self.nq,)
+            self._shard_tracks = (s, red, lens)
         with torch.cuda.device(self.device):
-            N.check(N.lib.wealy_eval_shard_sweep(self._handle, self._shard_dim, self._shard_passes, int(shard_rank),
-                                                 int(shard_world), N.stream_ptr(self.device)))
+            if s == 1:
+                N.check(N.lib.wealy_eval_shard_sweep(self._handle, self._shard_dim, self._shard_passes, int(shard_rank),
+                                                     int(shard_world), N.stream_ptr(self.device)))
+            else:
+                N.check(N.lib.wealy_eval_shard_sweep_tracks(
+                    self._handle, self._shard_dim, self._shard_passes, s, N.REDUX[red],
+                    None if lens is None else lens.data_ptr(), int(shard_rank), int(shard_world),
+                    N.stream_ptr(self.device)))
 
     def counts_tensor(self):
         """int32 view (no copy) of the plan's per-(query, relevant item) rank counters: the buffer a

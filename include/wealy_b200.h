@@ -183,6 +183,26 @@ int wealy_eval_shard_prepare(wealy_eval_plan* plan, const void* z, int64_t ld, i
                              int shard_rank, int shard_world, void* stream);
 int wealy_eval_plan_thresholds(const wealy_eval_plan* plan, void** values, int64_t* count);
 int wealy_eval_shard_sweep(wealy_eval_plan* plan, int64_t d, int passes, int shard_rank, int shard_world, void* stream);
+/* Multi-GPU all-vs-all of CHUNKED tracks (z [n * chunks, d], chunks in {2, 4, 8, 16}, redux WEALY_REDUX_*; lens NULL for
+ * full tracks, else the device int32 [n] ragged chunk counts, used for both sides as in wealy_eval_run_ragged).  The
+ * same protocol as above: every rank sweeps the row blocks rb = shard_rank (mod shard_world) of the chunked sweep --
+ * the half sweep for min / max / mean, the rectangle for meanmin / minmean (or WEALY_SYM_TRACKS=0) -- then the counts
+ * are summed over the ranks and wealy_eval_finish yields the per-track AP / R1.  No top-k; queries must be the
+ * candidates (WEALY_ERR_BAD_ARG otherwise), other chunk counts WEALY_ERR_UNSUPPORTED.
+ * Staged form: _prepare_tracks computes the relevant track similarities of this rank's contiguous share of the query
+ * tracks, [n r / w, n (r + 1) / w), into a zeroed buffer; after _prepare_tracks, wealy_eval_plan_thresholds returns that
+ * buffer alone: `count` = total_pairs floats, query q's sorted thresholds at [offsets[q], offsets[q + 1]) of
+ * wealy_eval_plan_ranks' CSR offsets (after the vector _prepare it returns {lowest thresholds, all thresholds}).  The
+ * caller sums it over the ranks; _sweep_tracks rebuilds the per-query counts and limits from it on every rank, then
+ * sweeps the rank's row blocks.  d / passes / chunks / redux / lens of the two stages must agree. */
+int wealy_eval_sweep_shard_tracks(wealy_eval_plan* plan, const void* z, int64_t ld, int64_t d, int dtype, float eps,
+                                  int passes, int chunks, int redux, const int32_t* lens, int shard_rank, int shard_world,
+                                  void* stream);
+int wealy_eval_shard_prepare_tracks(wealy_eval_plan* plan, const void* z, int64_t ld, int64_t d, int dtype, float eps,
+                                    int passes, int chunks, int redux, const int32_t* lens, int shard_rank, int shard_world,
+                                    void* stream);
+int wealy_eval_shard_sweep_tracks(wealy_eval_plan* plan, int64_t d, int passes, int chunks, int redux, const int32_t* lens,
+                                  int shard_rank, int shard_world, void* stream);
 int wealy_eval_finish(wealy_eval_plan* plan, float* aps, float* r1s, double* sums, void* stream);
 /* Per-item ranks of the last run -- the quantities AP and R1 are made of.  offsets [nq + 1] int64 (CSR over the
  * caller's queries; offsets[nq] = total_pairs of wealy_eval_plan_info), ranks / sims [total_pairs]: for every query its

@@ -68,6 +68,9 @@ SIGNATURES = {
     "wealy_eval_shard_prepare_tracks": (c_int, [c_vp, c_vp, c_i64, c_i64, c_int, c_f32, c_int, c_int, c_int, c_vp, c_int,
                                                 c_int, c_vp]),
     "wealy_eval_shard_sweep_tracks": (c_int, [c_vp, c_i64, c_int, c_int, c_int, c_vp, c_int, c_int, c_vp]),
+    "wealy_eval_sweep_shard_topk": (c_int, [c_vp, c_vp, c_i64, c_i64, c_int, c_f32, c_int, c_int, c_int, c_int, c_vp, c_vp,
+                                            c_vp, c_vp]),
+    "wealy_eval_topk_merge": (c_int, [c_vp, c_vp, c_vp, c_int, c_i64, c_int, c_vp, c_vp, c_vp, c_vp]),
     "wealy_eval_plan_counts": (c_int, [c_vp, ctypes.POINTER(c_vp), ctypes.POINTER(c_i64)]),
     "wealy_eval_finish": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp]),
     "wealy_eval_plan_ranks": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp]),

@@ -813,7 +813,7 @@ struct wealy_eval_plan {
   // ... and the stages around it: [0] before prep, [1] before K_pos, [2] after ap_reduce, [3] after the top-k finalize
   cudaEvent_t evs[4] = {nullptr, nullptr, nullptr, nullptr};
   bool timed = false;
-  bool finished = false;  // the last run included ap_reduce (+ top-k finalize)
+  bool finished = false;  // the last run recorded the events after ap_reduce and the top-k finalize (evs[2], evs[3])
   bool last_sym = false;  // the last sweep ran in the clique-sorted view (its counters are in that CSR order)
   int staged_chunks = 0;  // chunks of the last staged prepare (0 none); > 1: the summed buffer is thr alone
   // wealy_eval_run_host: [0] "planes allocated" on the run's stream, [1 + k] "rows of part k have arrived" on the upload stream
@@ -1072,10 +1072,14 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
                          int64_t ld_c, int64_t d, int dtype, float eps, int passes, int topk, float* aps,
                          float* r1s, double* sums, int64_t* topk_idx, float* topk_sim, int shard_rank,
                          int shard_world, bool finish, void* stream, int chunks = 1, int redux = WEALY_REDUX_MIN,
-                         const int* q_len = nullptr, const int* c_len = nullptr, bool allow_sym_topk = true, int stage = 0) {
+                         const int* q_len = nullptr, const int* c_len = nullptr, bool allow_sym_topk = true, int stage = 0,
+                         int* local_idx = nullptr, int* local_cnt = nullptr) {
   // stage (sharded all-vs-all sweeps only): 0 = everything in one call; 1 = prep + the relevant similarities of THIS
   // rank's share of the queries, then return (the caller sums the threshold buffer over the ranks); 2 = the sweep,
   // on the planes and thresholds stage 1 left in the plan
+  // local_cnt != NULL (wealy_eval_sweep_shard_topk): the symmetric top-k sweep over this rank's row blocks, its lists
+  // finalized locally into topk_sim / local_idx / local_cnt; the rank counters stay in the plan (finish == false)
+  const bool local = local_cnt != nullptr;
   cudaStream_t s = (cudaStream_t)stream;
   if (!p) return fail(WEALY_ERR_BAD_ARG, "null plan");
   if (p->early_lo >= 0) {
@@ -1100,7 +1104,7 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
   if (d <= 0) return fail(WEALY_ERR_BAD_ARG, "bad embedding size %lld", (long long)d);
   if (passes != 1 && passes != 3) return fail(WEALY_ERR_BAD_ARG, "passes must be 1 or 3");
   if (topk < 0 || topk > 800) return fail(WEALY_ERR_UNSUPPORTED, "topk must be in [0, 800], got %d", topk);
-  if (topk > 0 && (!topk_idx || !topk_sim)) return fail(WEALY_ERR_BAD_ARG, "topk outputs are null");
+  if (topk > 0 && (!(local ? (void*)local_idx : (void*)topk_idx) || !topk_sim)) return fail(WEALY_ERR_BAD_ARG, "topk outputs are null");
   const int64_t nq = p->nq, nc = p->nc;
   const bool same = (queries_z == candidates_z && nq == nc && ld_q == ld_c);
   if (chunks != 1 && chunks != 2 && chunks != 4 && chunks != 8 && chunks != 16)
@@ -1128,12 +1132,15 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
   // sweep appends what lies above the bound to per-query lists in both directions.  Worth it (and statistically sound)
   // for large sets and moderate k; everything else keeps the rectangle sweep with its streaming top-k.
   const bool sym_topk = can_sym && topk > 0 && topk <= 128 && nq >= env_int("WEALY_SYM_TOPK_MIN_ROWS", 16384) &&
-                        nq >= 192ll * topk && finish &&
-                        shard_world == 1 && allow_sym_topk && env_int("WEALY_SYM_TOPK", 1) != 0;
+                        nq >= 192ll * topk && (local || (finish && shard_world == 1)) &&
+                        allow_sym_topk && env_int("WEALY_SYM_TOPK", 1) != 0;
   const bool sym = can_sym && (topk == 0 ? (shard_world > 1 || env_int("WEALY_SYM", 1) != 0) : sym_topk);
   // chunked tracks, all-vs-all: the same halving for reductions that give d(q, c) == d(c, q) (min / max / mean)
   const bool all_tracks = same && p->same_ids && chunks > 1 && topk == 0;
   const bool sym_tracks = all_tracks && red_inner == red_outer && nq * chunks > 2 * kTileM && env_int("WEALY_SYM_TRACKS", 1) != 0;
+  if (local && !sym_topk)
+    return fail(WEALY_ERR_UNSUPPORTED, "the sharded top-k sweep needs queries == candidates (ids and embeddings), plain "
+                "embeddings, k <= 128 and N >= max(WEALY_SYM_TOPK_MIN_ROWS, 192 k), got N = %lld, k = %d", (long long)nq, topk);
   if (shard_world > 1 && !sym && !all_tracks)
     return fail(WEALY_ERR_BAD_ARG, "a sharded sweep needs queries == candidates (ids and embeddings) and no top-k");
 
@@ -1439,6 +1446,18 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
   CU_TRY(cudaEventRecord(p->ev1, s));
   p->timed = true;
   p->finished = finish;
+
+  if (local) {
+    // (stage events: ap_reduce stays empty -- it runs in wealy_eval_finish once the counters are summed --, topk_finalize
+    //  times the local finalize)
+    CU_TRY(cudaEventRecord(p->evs[2], s));
+    topk_sym_local_kernel<<<(unsigned)ceil_div(rows_q * 32, 128), 128, 0, s>>>(tk_val, tk_idx, tk_cnt, tk_cap2, (int)rows_q, (int)nq,
+                                                                              topk, p->sorted_idx, topk_sim, local_idx, local_cnt);
+    CU_TRY(cudaGetLastError());
+    CU_TRY(cudaEventRecord(p->evs[3], s));
+    p->finished = true;
+    return WEALY_OK;
+  }
 
   if (finish) {
     const int threads = 256;
@@ -1966,6 +1985,42 @@ extern "C" int wealy_eval_sweep_shard(wealy_eval_plan* p, const void* z, int64_t
                                       int passes, int shard_rank, int shard_world, void* stream) {
   return eval_run_impl(p, z, ld, z, ld, d, dtype, eps, passes, 0, nullptr, nullptr, nullptr, nullptr, nullptr,
                        shard_rank, shard_world, false, stream);
+}
+
+// ... with top-k lists: the same sweep with the symmetric top-k epilogue, this rank's lists finalized locally (caller's
+// row order; cnt -1 = overflow); eligibility depends on the arguments and the plan's ids only, so every rank gets the
+// same answer before any work.  world * k <= 1024: the merge takes a query's lists of all ranks in one warp pass.
+extern "C" int wealy_eval_sweep_shard_topk(wealy_eval_plan* p, const void* z, int64_t ld, int64_t d, int dtype, float eps,
+                                           int passes, int k, int shard_rank, int shard_world, float* val, int32_t* idx,
+                                           int32_t* cnt, void* stream) {
+  if (k < 1 || k > 128) return fail(WEALY_ERR_UNSUPPORTED, "the sharded top-k sweep needs 1 <= k <= 128, got %d", k);
+  if ((int64_t)shard_world * k > 1024)
+    return fail(WEALY_ERR_UNSUPPORTED, "the sharded top-k merge needs world * k <= 1024, got %d x %d", shard_world, k);
+  if (!p || !z || !val || !idx || !cnt) return fail(WEALY_ERR_BAD_ARG, "null pointer");
+  return eval_run_impl(p, z, ld, z, ld, d, dtype, eps, passes, k, nullptr, nullptr, nullptr, nullptr, val, shard_rank,
+                       shard_world, false, stream, 1, WEALY_REDUX_MIN, nullptr, nullptr, true, 0, idx, cnt);
+}
+
+// The k best of every query's lists of all ranks (val / idx [world][n][k], cnt [world][n]: the local lists of the ranks,
+// each restricted to the same n queries) -> out_idx / out_sim [n][k]; *fail += the queries whose lists overflowed or
+// hold fewer than k entries together.
+extern "C" int wealy_eval_topk_merge(const float* val, const int32_t* idx, const int32_t* cnt, int world, int64_t n, int k,
+                                     int64_t* out_idx, float* out_sim, int32_t* fail_count, void* stream) {
+  cudaStream_t s = (cudaStream_t)stream;
+  if (world < 1 || n < 0 || k < 1) return fail(WEALY_ERR_BAD_ARG, "bad merge shape: %d lists of [%lld][%d]", world, (long long)n, k);
+  if (k > 128 || (int64_t)world * k > 1024)
+    return fail(WEALY_ERR_UNSUPPORTED, "the top-k merge needs k <= 128 and world * k <= 1024, got %d x %d", world, k);
+  if (n == 0) return WEALY_OK;
+  if (!val || !idx || !cnt || !out_idx || !out_sim || !fail_count) return fail(WEALY_ERR_BAD_ARG, "null pointer");
+  const unsigned blocks = (unsigned)ceil_div(n * 32, 128);
+  const int L = world * k;
+  long long* oi = reinterpret_cast<long long*>(out_idx);
+  if (L <= 128) topk_merge_kernel<4><<<blocks, 128, 0, s>>>(val, idx, cnt, world, n, k, oi, out_sim, fail_count);
+  else if (L <= 256) topk_merge_kernel<8><<<blocks, 128, 0, s>>>(val, idx, cnt, world, n, k, oi, out_sim, fail_count);
+  else if (L <= 512) topk_merge_kernel<16><<<blocks, 128, 0, s>>>(val, idx, cnt, world, n, k, oi, out_sim, fail_count);
+  else topk_merge_kernel<32><<<blocks, 128, 0, s>>>(val, idx, cnt, world, n, k, oi, out_sim, fail_count);
+  CU_TRY(cudaGetLastError());
+  return WEALY_OK;
 }
 
 // ... the per-(query, relevant item) rank counts are then summed over the ranks by the caller (an all-reduce of

@@ -155,9 +155,41 @@ __device__ __noinline__ void select_topk_exact(float* val, int* idx, int n, int 
   __syncwarp();
 }
 
+// The min(k, m) best of a list of m <= cap entries (plane rows) moved to its front, their plane rows translated to the
+// caller's indices (the selection itself never looks at indices, so that equal similarities are ordered like the
+// rectangle path orders them).  Returns min(k, m).
+__device__ __forceinline__ int sym_list_best(float* sv, int* si, int m, int k, const int* __restrict__ perm, int lane) {
+  // (lists are sized mean + 8 sigma: most hold far fewer entries than `cap`, so the selection is instantiated for the
+  //  list's length, and its bisection stops at the first prefix that exactly k entries reach)
+  if (m > k) {
+    if (m <= 256) select_topk_exact<8>(sv, si, m, k, lane);
+    else if (m <= 512) select_topk_exact<16>(sv, si, m, k, lane);
+    else if (m <= 768) select_topk_exact<24>(sv, si, m, k, lane);
+    else select_topk_exact<32>(sv, si, m, k, lane);
+  }
+  const int kk = m < k ? m : k;
+  __syncwarp();
+  for (int e = lane; e < kk; e += 32) si[e] = perm[spread_sorted_of(si[e])];
+  __syncwarp();
+  return kk;
+}
+
+// position of entry e among the kk entries of a list in the output order: descending similarity, ties -> lower caller
+// index (like a stable ascending-distance argsort)
+__device__ __forceinline__ int sym_list_rank(const float* sv, const int* si, int kk, int e) {
+  const float ve = sv[e];
+  const int ie = si[e];
+  int r = 0;
+  for (int f = 0; f < kk; ++f) {
+    const float vf = sv[f];
+    r += (vf > ve) || (vf == ve && si[f] < ie);
+  }
+  return r;
+}
+
 // finalize: one warp per plane row (query).  Its list holds every candidate above beta (plane rows); select the k best,
-// order them (descending similarity, ties -> lower caller index, like a stable ascending-distance argsort) and write
-// them at the caller's row.  Lists that overflowed or hold fewer than k entries are reported in `fail`.
+// order them and write them at the caller's row.  Lists that overflowed or hold fewer than k entries are reported in
+// `fail`.
 __global__ void __launch_bounds__(128) topk_sym_finalize_kernel(float* __restrict__ tk_val, int* __restrict__ tk_idx,
                                                                 const int* __restrict__ tk_cnt, int cap, int n_rows, int n,
                                                                 int k, const int* __restrict__ perm,
@@ -176,29 +208,127 @@ __global__ void __launch_bounds__(128) topk_sym_finalize_kernel(float* __restric
   }
   float* sv = tk_val + (long long)p * cap;
   int* si = tk_idx + (long long)p * cap;
-  // (lists are sized mean + 8 sigma: most hold far fewer entries than `cap`, so the selection is instantiated for the
-  //  list's length, and its bisection stops at the first prefix that exactly k entries reach)
-  if (m > k) {
-    if (m <= 256) select_topk_exact<8>(sv, si, m, k, lane);
-    else if (m <= 512) select_topk_exact<16>(sv, si, m, k, lane);
-    else if (m <= 768) select_topk_exact<24>(sv, si, m, k, lane);
-    else select_topk_exact<32>(sv, si, m, k, lane);
+  sym_list_best(sv, si, m, k, perm, lane);
+  for (int e = lane; e < k; e += 32) {
+    const int r = sym_list_rank(sv, si, k, e);
+    out_idx[q * k + r] = si[e];
+    out_sim[q * k + r] = sv[e];
+  }
+}
+
+// Sharded sweep (wealy_eval_sweep_shard_topk): the local finalize.  A rank's list of query q holds the candidates above
+// beta_q that ITS row blocks found; the min(k, m) best of it go to the caller's row q in the order above, padded with
+// (-inf, -1), and cnt[q] = m (-1: the list overflowed).  A list shorter than k is no failure here -- the other ranks hold
+// the rest; topk_merge_kernel judges the union.
+__global__ void __launch_bounds__(128) topk_sym_local_kernel(float* __restrict__ tk_val, int* __restrict__ tk_idx,
+                                                             const int* __restrict__ tk_cnt, int cap, int n_rows, int n, int k,
+                                                             const int* __restrict__ perm, float* __restrict__ out_val,
+                                                             int* __restrict__ out_idx, int* __restrict__ out_cnt) {
+  const int p = (int)((blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5);
+  const int lane = (int)(threadIdx.x & 31);
+  if (p >= n_rows) return;
+  const int srow = spread_sorted_of(p);
+  if (srow >= n) return;
+  const long long q = perm[srow];
+  const int m = tk_cnt[p];
+  if (lane == 0) out_cnt[q] = m > cap ? -1 : m;
+  float* sv = tk_val + (long long)p * cap;
+  int* si = tk_idx + (long long)p * cap;
+  const int kk = m > cap ? 0 : sym_list_best(sv, si, m, k, perm, lane);
+  for (int e = lane; e < k; e += 32) {
+    if (e < kk) {
+      const int r = sym_list_rank(sv, si, kk, e);
+      out_idx[q * k + r] = si[e];
+      out_val[q * k + r] = sv[e];
+    } else {
+      out_idx[q * k + e] = -1;
+      out_val[q * k + e] = __int_as_float(0xff800000);
+    }
+  }
+}
+
+// Merge of the sharded lists (wealy_eval_topk_merge), one warp per query q: its `world` lists of k entries (val / idx
+// [world][n][k], cnt [world][n]) -> the k best, by descending similarity, ties -> lower index.  Every entry becomes one
+// 64-bit key {order key of the similarity, ~(index + 1)}, unique but for the (-inf, -1) padding (whose copies are
+// identical), so the k largest keys -- found by a bisection like select_topk_exact's, on 64 bits -- and their order do
+// not depend on the order of the lists.  Adds 1 to `fail` where a list overflowed (cnt -1) or the lists hold fewer than
+// k entries together.  world * k <= 32 * kPerLane, k <= 128.
+template <int kPerLane>
+__global__ void __launch_bounds__(128) topk_merge_kernel(const float* __restrict__ val, const int* __restrict__ idx,
+                                                         const int* __restrict__ cnt, int world, long long n, int k,
+                                                         long long* __restrict__ out_idx, float* __restrict__ out_sim,
+                                                         int* __restrict__ fail) {
+  constexpr unsigned kFull = 0xffffffffu;
+  __shared__ unsigned long long skey_all[4][128];
+  const long long q = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+  const int lane = (int)(threadIdx.x & 31);
+  if (q >= n) return;
+  unsigned long long* sk = skey_all[threadIdx.x >> 5];
+  int total = 0;
+  bool over = false;
+  for (int w = lane; w < world; w += 32) {
+    const int c = cnt[(long long)w * n + q];
+    over |= c < 0;
+    total += c < 0 ? 0 : c;
+  }
+  total = __reduce_add_sync(kFull, total);
+  over = __any_sync(kFull, over);
+  if (lane == 0 && (over || total < k)) atomicAdd(fail, 1);
+  const int L = world * k;
+  unsigned long long key[kPerLane];
+#pragma unroll
+  for (int j = 0; j < kPerLane; ++j) {
+    const int e = j * 32 + lane;
+    key[j] = 0ull;  // below every entry's key (the order key of -inf is 0x007fffff)
+    if (e < L) {
+      const int w = e / k;
+      const long long o = ((long long)w * n + q) * k + (e - w * k);
+      key[j] = ((unsigned long long)float_order_key(val[o]) << 32) | (unsigned)~(unsigned)(idx[o] + 1);
+    }
+  }
+  unsigned long long T = 0ull;
+  for (int b = 63; b >= 0; --b) {
+    const unsigned long long cand = T | (1ull << b);
+    int c = 0;
+#pragma unroll
+    for (int j = 0; j < kPerLane; ++j) c += key[j] >= cand;
+    c = __reduce_add_sync(kFull, c);
+    if (c >= k) T = cand;  // warp-uniform
+    if (c == k) break;
+  }
+  int g = 0, e_q = 0;
+#pragma unroll
+  for (int j = 0; j < kPerLane; ++j) {
+    g += key[j] > T;
+    e_q += key[j] == T;
+  }
+  int gi = g, qi = e_q;  // inclusive scans over lanes
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const int tg = __shfl_up_sync(kFull, gi, o);
+    const int tq = __shfl_up_sync(kFull, qi, o);
+    if (lane >= o) { gi += tg; qi += tq; }
+  }
+  int pg = gi - g;
+  int pq = __shfl_sync(kFull, gi, 31) + (qi - e_q);
+#pragma unroll
+  for (int j = 0; j < kPerLane; ++j) {
+    if (key[j] > T) sk[pg++] = key[j];
+    else if (key[j] == T) {
+      if (pq < k) sk[pq] = key[j];
+      ++pq;
+    }
   }
   __syncwarp();
-  // plane row -> caller index for the k survivors (the selection itself never looks at indices), so that equal
-  // similarities are ordered like the rectangle path orders them
-  for (int e = lane; e < k; e += 32) si[e] = perm[spread_sorted_of(si[e])];
-  __syncwarp();
   for (int e = lane; e < k; e += 32) {
-    const float ve = sv[e];
-    const int ie = si[e];
+    const unsigned long long ke = sk[e];
     int r = 0;
     for (int f = 0; f < k; ++f) {
-      const float vf = sv[f];
-      r += (vf > ve) || (vf == ve && si[f] < ie);
+      const unsigned long long kf = sk[f];
+      r += (kf > ke) || (kf == ke && f < e);
     }
-    out_idx[q * k + r] = ie;
-    out_sim[q * k + r] = ve;
+    out_idx[q * k + r] = (long long)(int)(~(unsigned)ke) - 1;
+    out_sim[q * k + r] = float_from_order_key((unsigned)(ke >> 32));
   }
 }
 

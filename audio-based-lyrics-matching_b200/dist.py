@@ -8,7 +8,9 @@ Two schemes:
   diagonal, each element scoring its row and its column query).  A rank therefore holds partial rank counts for
   ALL queries; the one real exchange step of the path is an all-reduce (SUM) of those int32 counters -- the
   "rank counts merged over NCCL" of the north star -- after which every rank owns the complete AP / R1.  Chunked
-  tracks ([N, s, D], SURVEY.md 8(f) row f1) shard the chunked sweep the same way for min / max / mean.
+  tracks ([N, s, D], SURVEY.md 8(f) row f1) shard the chunked sweep the same way for min / max / mean.  Top-k lists
+  (per-query state, not counters) are finalized locally, exchanged with one all-to-all so that rank r holds every
+  rank's lists of its query slice, merged there and all-gathered.
 * general queries vs corpus -- `evaluate_sharded`: queries are independent units, so rank r scores the contiguous
   query slice shard_range(Nq, r, world) against the whole (replicated) corpus with the single-GPU fused kernel and
   the data path needs no collective.  The only exchange is the result merge: one all-reduce of {sum AP, sum R1,
@@ -84,6 +86,48 @@ def upload_sharded(z_host, device, group=None):
     return full[:n]
 
 
+def exchange_topk(val, idx, cnt, group=None):
+    """Every rank's local top-k lists of ALL queries (val [n, k] float32, idx [n, k] int32, cnt [n] int32, as
+    EvalPlan.sweep_shard_topk returns them) -> the lists of every rank for THIS rank's query slice
+    shard_range(n, rank, world): (val [world, n_r, k], idx [world, n_r, k], cnt [world, n_r]), list w from rank w.
+    The rows are already laid out by destination (slices are contiguous), so one all_to_all_single of the three arrays
+    packed side by side ([n, 2 k + 1] int32) moves them; gloo stages through the host, as gather_rows does."""
+    world = dist.get_world_size(group)
+    rank = dist.get_rank(group)
+    n, k = val.shape
+    sizes = [hi - lo for lo, hi in (shard_range(n, r, world) for r in range(world))]
+    packed = torch.cat([val.view(torch.int32), idx, cnt[:, None]], dim=1)
+    via_host = packed.is_cuda and dist.get_backend(group) == "gloo"
+    src = packed.cpu() if via_host else packed
+    recv = torch.empty((world * sizes[rank], 2 * k + 1), dtype=torch.int32, device=src.device)
+    dist.all_to_all_single(recv, src, output_split_sizes=[sizes[rank]] * world, input_split_sizes=sizes, group=group)
+    recv = recv.to(val.device).view(world, sizes[rank], 2 * k + 1)
+    return (recv[..., :k].contiguous().view(torch.float32), recv[..., k:2 * k].contiguous(),
+            recv[..., 2 * k].contiguous())
+
+
+def _sym_sharded_topk(plan, z, rank, world, k, *, eps, precision, group):
+    """All-vs-all top-k on the row-block-sharded symmetric sweep: every rank sweeps its row blocks with the top-k
+    epilogue (sampled bounds computed identically on every rank), the rank counters are summed, the local lists of every
+    query slice are exchanged (exchange_topk) and merged on the slice's rank, the merged slices all-gathered.
+    -> (dict(aps, r1s, sums, topk_idx, topk_sim), "sym_sharded"); (None, "query_sharded") where the call is not eligible
+    (the same on every rank: the decision reads only arguments and ids), (None, "query_sharded_fallback") where some
+    rank's merge found a list that overflowed or ended short of k."""
+    from .evaluation import merge_topk
+    try:
+        loc = plan.sweep_shard_topk(z, rank, world, k, eps=eps, precision=precision)
+    except NotImplementedError:
+        return None, "query_sharded"
+    dist.all_reduce(plan.counts_tensor(), op=dist.ReduceOp.SUM, group=group)
+    tk_idx, tk_sim, failed = merge_topk(*exchange_topk(loc["val"], loc["idx"], loc["cnt"], group))
+    if _agree(failed, plan.device, group):
+        return None, "query_sharded_fallback"
+    res = plan.finish()
+    res["topk_idx"] = gather_rows(tk_idx, plan.nq, group)
+    res["topk_sim"] = gather_rows(tk_sim, plan.nq, group)
+    return res, "sym_sharded"
+
+
 def _agree(flag, device, group=None):
     """MAX of a small non-negative integer over the ranks: every rank learns whether ANY rank wants to raise."""
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
@@ -147,9 +191,14 @@ def evaluate_all_vs_all(c, i, z, *, precision=None, eps=1e-6, group=None, plan=N
     as in EvalPlan.run.  min / max / mean shard the chunked sweep by row blocks, like plain embeddings; meanmin /
     minmean (d(q, c) != d(c, q), so no half sweep) take the query-partitioned scheme below.
 
-    topk: per-query top-k lists are per-query state, not additive counters, so with more than one rank they take the
-    query-partitioned scheme (`evaluate_sharded`: every rank scores its slice of the queries against the replicated
-    corpus with the streaming top-k, the lists are all-gathered) -> also topk_idx / topk_sim.
+    topk -> also topk_idx / topk_sim and, with more than one rank, topk_path.  Top-k lists are per-query state, not
+    additive counters: where the single-GPU run takes the symmetric top-k sweep (plain [N, D] embeddings, k <= 128,
+    N >= max(16384, 192 k)) and world * k <= 1024, every rank sweeps its row blocks with the top-k epilogue, the rank
+    counters are summed, each rank merges every rank's lists of its query slice (one all-to-all) and the merged slices
+    are all-gathered (topk_path "sym_sharded").  Otherwise -- and, on every rank, when a merge finds a list that
+    overflowed or ended short of k ("query_sharded_fallback") -- the query-partitioned scheme (`evaluate_sharded`:
+    every rank scores its slice of the queries against the replicated corpus with the streaming top-k, the lists are
+    all-gathered; "query_sharded").
 
     Like EvalPlan.run, a query without any relevant candidate raises ValueError unless allow_empty -- on every
     rank (all ranks build the same id plan), before the first collective."""
@@ -158,11 +207,14 @@ def evaluate_all_vs_all(c, i, z, *, precision=None, eps=1e-6, group=None, plan=N
     rank = dist.get_rank(group) if on else 0
     world = dist.get_world_size(group) if on else 1
     s = _chunks_per_track(z, chunks, redux, q_chunks)
-    if world > 1 and (topk or (s > 1 and redux in ("meanmin", "minmean"))):
+    if world > 1 and s > 1 and (topk or redux in ("meanmin", "minmean")):
         if not torch.as_tensor(z).is_cuda:
             z = upload_sharded(torch.as_tensor(z), torch.device("cuda", torch.cuda.current_device()), group)
-        return evaluate_sharded(c, i, z, c, i, z, topk=topk, precision=precision, eps=eps, group=group,
-                                allow_empty=allow_empty, chunks=chunks, redux=redux, q_chunks=q_chunks, c_chunks=q_chunks)
+        out = evaluate_sharded(c, i, z, c, i, z, topk=topk, precision=precision, eps=eps, group=group,
+                               allow_empty=allow_empty, chunks=chunks, redux=redux, q_chunks=q_chunks, c_chunks=q_chunks)
+        if topk:
+            out["topk_path"] = "query_sharded"
+        return out
     side = None
     if world > 1 and not torch.as_tensor(z).is_cuda:
         # 1/world of the rows per rank + NVLink all-gather, issued on a side stream BEFORE the id plan is built: the
@@ -173,7 +225,8 @@ def evaluate_all_vs_all(c, i, z, *, precision=None, eps=1e-6, group=None, plan=N
         side.wait_stream(torch.cuda.current_stream(device))
         with torch.cuda.stream(side):
             z = upload_sharded(torch.as_tensor(z), device, group)
-    if plan is None:
+    own = plan is None
+    if own:
         plan = EvalPlan(c, i, c, i)
     if side is not None:
         torch.cuda.current_stream(plan.device).wait_stream(side)
@@ -184,6 +237,16 @@ def evaluate_all_vs_all(c, i, z, *, precision=None, eps=1e-6, group=None, plan=N
     if world == 1:
         res = plan.run(z, z, eps=eps, precision=precision, allow_empty=allow_empty, topk=topk, chunks=chunks, redux=redux,
                        q_chunks=q_chunks)
+    elif topk:
+        res, path = _sym_sharded_topk(plan, z, rank, world, min(int(topk), plan.nq), eps=eps, precision=precision,
+                                      group=group)
+        if res is None:
+            if own:
+                plan.close()
+            out = evaluate_sharded(c, i, z, c, i, z, topk=topk, precision=precision, eps=eps, group=group,
+                                   allow_empty=allow_empty)
+            out["topk_path"] = path
+            return out
     else:
         sharded_step(plan, z, rank, world, eps=eps, precision=precision, group=group, redux=redux, q_chunks=q_chunks,
                      chunks=chunks)
@@ -194,6 +257,8 @@ def evaluate_all_vs_all(c, i, z, *, precision=None, eps=1e-6, group=None, plan=N
            "plan": plan}
     if topk and "topk_idx" in res:
         out["topk_idx"], out["topk_sim"] = res["topk_idx"], res["topk_sim"]
+    if topk and world > 1:
+        out["topk_path"] = path
     return out
 
 

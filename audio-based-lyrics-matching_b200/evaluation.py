@@ -122,6 +122,27 @@ class EvalPlan:
                     int(shard_world), N.stream_ptr(self.device)))
         self._keepalive = (z, lens)
 
+    def sweep_shard_topk(self, z, shard_rank, shard_world, k, *, eps=1e-6, precision=None):
+        """sweep_shard() with top-k lists: this rank's row blocks of the symmetric top-k sweep (plain [N, D] embeddings;
+        the sampled per-query bounds are computed on every rank, identically).  The rank counters stay in the plan (sum
+        counts_tensor() over the ranks, then finish()); returns this rank's local lists dict(val [N, k] float32,
+        idx [N, k] int32, cnt [N] int32): per query the min(k, m) best of its m local candidates, by descending
+        similarity, ties to the lower index, padded with (-inf, -1); cnt = m, or -1 where the list overflowed.  Merge
+        the lists of all ranks with merge_topk().  Raises NotImplementedError, before any work and alike on every rank,
+        where the single-GPU run would not take the symmetric top-k sweep or shard_world * k > 1024."""
+        z, _, _ = self._shard_input(z, None, "min", None)
+        k = int(k)
+        val = torch.empty((self.nq, max(k, 0)), dtype=torch.float32, device=self.device)
+        idx = torch.empty((self.nq, max(k, 0)), dtype=torch.int32, device=self.device)
+        cnt = torch.empty(self.nq, dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            N.check(N.lib.wealy_eval_sweep_shard_topk(
+                self._handle, z.data_ptr(), z.stride(0), z.shape[1], N.dtype_code(z.dtype), float(eps),
+                passes_of(precision), k, int(shard_rank), int(shard_world), val.data_ptr(), idx.data_ptr(), cnt.data_ptr(),
+                N.stream_ptr(self.device)))
+        self._keepalive = z
+        return {"val": val, "idx": idx, "cnt": cnt}
+
     def shard_prepare(self, z, shard_rank, shard_world, *, eps=1e-6, precision=None, redux="min", q_chunks=None,
                       chunks=None):
         """Stage 1 of the sharded sweep: planes of the whole corpus, thresholds of THIS rank's share of the queries.
@@ -326,6 +347,29 @@ class EvalPlan:
         if k:
             out["topk_idx"], out["topk_sim"] = tk_idx, tk_sim
         return out
+
+
+def merge_topk(val, idx, cnt):
+    """Merge the local top-k lists of `world` ranks (EvalPlan.sweep_shard_topk), restricted to the same n queries:
+    val [world, n, k] float32, idx [world, n, k] int32, cnt [world, n] int32 on one CUDA device ->
+    (topk_idx [n, k] int64, topk_sim [n, k] float32, failed): per query the k best of its world * k entries, by
+    descending similarity, ties to the lower index, whatever the order of the world lists.  `failed` counts the queries
+    whose lists overflowed (cnt -1) or hold fewer than k entries together: their lists are not the k best (recompute
+    them).  Synchronises the stream once (to read `failed`).  k <= 128 and world * k <= 1024."""
+    assert val.ndim == 3 and idx.shape == val.shape and cnt.shape == val.shape[:2]
+    assert val.is_cuda and idx.is_cuda and cnt.is_cuda
+    world, n, k = val.shape
+    device = val.device
+    val = val.to(torch.float32).contiguous()
+    idx = idx.to(torch.int32).contiguous()
+    cnt = cnt.to(torch.int32).contiguous()
+    out_idx = torch.empty((n, k), dtype=torch.long, device=device)
+    out_sim = torch.empty((n, k), dtype=torch.float32, device=device)
+    fail = torch.zeros(1, dtype=torch.int32, device=device)
+    with torch.cuda.device(device):
+        N.check(N.lib.wealy_eval_topk_merge(val.data_ptr(), idx.data_ptr(), cnt.data_ptr(), world, n, k,
+                                            out_idx.data_ptr(), out_sim.data_ptr(), fail.data_ptr(), N.stream_ptr(device)))
+    return out_idx, out_sim, int(fail.item())
 
 
 def evaluate(queries_c, queries_i, queries_z, candidates_c, candidates_i, candidates_z, *, topk=None, mode="cos",

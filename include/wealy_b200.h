@@ -203,6 +203,28 @@ int wealy_eval_shard_prepare_tracks(wealy_eval_plan* plan, const void* z, int64_
                                     void* stream);
 int wealy_eval_shard_sweep_tracks(wealy_eval_plan* plan, int64_t d, int passes, int chunks, int redux, const int32_t* lens,
                                   int shard_rank, int shard_world, void* stream);
+/* Multi-GPU all-vs-all WITH top-k lists (plain [n, d] embeddings, queries == candidates).  Every rank calls
+ * wealy_eval_sweep_shard_topk: the normalisation, the relevant similarities and the sampled per-query bounds of the
+ * single-GPU symmetric top-k sweep run on every rank (identical on all of them), then the symmetric top-k sweep over the
+ * row blocks rb = shard_rank (mod shard_world).  The rank counts stay in the plan (sum them over the ranks, then
+ * wealy_eval_finish, as above); the rank's candidate lists are finalized locally: val / idx [n][k] (device float32 /
+ * int32, the caller's row q, caller indices) hold the min(k, m) best of query q's m local candidates, by descending
+ * similarity, ties to the lower index, padded with (-inf, -1); cnt [n] = m, or -1 where the list overflowed.  A list
+ * shorter than k is no failure: the other ranks hold the rest.  WEALY_ERR_UNSUPPORTED, before any work, unless the
+ * single-GPU call would take the symmetric top-k sweep (same ids, k <= 128, n >= max(WEALY_SYM_TOPK_MIN_ROWS, 192 k),
+ * WEALY_SYM_TOPK != 0) and shard_world * k <= 1024; the decision reads only the arguments and the plan's ids, so every
+ * rank reaches the same one.  wealy_eval_plan_last_topk_path reports 1, stage_ms' top-k finalize the local finalize.
+ * wealy_eval_topk_merge then merges, per query, the lists of all ranks -- val / idx [world][n][k], cnt [world][n], as
+ * sweep_shard_topk wrote them, each restricted to the same n queries (rank r typically receives every rank's rows of
+ * its own query slice) -- into out_idx (int64) / out_sim [n][k]: the k best of the world * k entries, by descending
+ * similarity, ties to the lower index, whatever the order of the world lists.  It ADDS to the device int32 *fail the
+ * number of queries with a count of -1 or counts summing to less than k; for those the lists do not hold the k best,
+ * and the caller recomputes them (e.g. with queries partitioned over the ranks).  k <= 128, world * k <= 1024. */
+int wealy_eval_sweep_shard_topk(wealy_eval_plan* plan, const void* z, int64_t ld, int64_t d, int dtype, float eps,
+                                int passes, int k, int shard_rank, int shard_world, float* val, int32_t* idx, int32_t* cnt,
+                                void* stream);
+int wealy_eval_topk_merge(const float* val, const int32_t* idx, const int32_t* cnt, int world, int64_t n, int k,
+                          int64_t* out_idx, float* out_sim, int32_t* fail, void* stream);
 int wealy_eval_finish(wealy_eval_plan* plan, float* aps, float* r1s, double* sums, void* stream);
 /* Per-item ranks of the last run -- the quantities AP and R1 are made of.  offsets [nq + 1] int64 (CSR over the
  * caller's queries; offsets[nq] = total_pairs of wealy_eval_plan_info), ranks / sims [total_pairs]: for every query its
@@ -217,7 +239,8 @@ int wealy_eval_plan_last_sweep_ms(const wealy_eval_plan* plan, float* ms);
  * 4-byte overflow flag), 2 the rectangle sweep with its streaming top-k, 3 = 1 failed its check and 2 recomputed.  */
 int wealy_eval_plan_last_topk_path(const wealy_eval_plan* plan, int* path);
 /* the same for the stages of the last run: ms[5] = {prep (normalise + fp16 split), K_pos (relevant similarities +
- * counter reset), fused sweep, ap_reduce, top-k finalize}; the last two are 0 after wealy_eval_sweep_shard.  */
+ * counter reset), fused sweep, ap_reduce, top-k finalize}; the last two are 0 after wealy_eval_sweep_shard, ap_reduce
+ * is 0 after wealy_eval_sweep_shard_topk.  */
 int wealy_eval_plan_stage_ms(const wealy_eval_plan* plan, float* ms);
 void wealy_eval_plan_destroy(wealy_eval_plan* plan);
 

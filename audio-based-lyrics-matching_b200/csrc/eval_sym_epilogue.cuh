@@ -11,12 +11,12 @@
 //   * in registers for the thread's own row,
 //   * in a per-tile shared-memory slot for the tile's 256 columns (one 6 KB bulk copy issued by the TMA thread
 //     together with the operand tiles; completion on an mbarrier, no CTA barrier per tile),
-// and the buckets 0 .. kLv-2 are counted directly: popc of mask differences into per-thread registers (rows),
-// 32x32 bit-matrix transposes + popc + one RED per (column, bucket) (columns).  Only elements above the kLv-th
+// and the buckets 0 .. kLv-2 are counted directly (clean tiles: chunk32_clean, counts of compares for the rows and, after
+// a transpose of the chunk through shared memory, for the columns; dirty tiles: popc of mask differences for the rows,
+// 32x32 bit-matrix transposes + popc for the columns), with one RED per (column, bucket).  Only elements above the kLv-th
 // threshold (~1 % of the pairs on SHS100K-shaped data, 7 % pass the first) go through the warp queue, where a
 // self-describing entry (value, threshold range, counter index) is binned by a binary search 32 x 2 at a time.
-// Dirty tiles run the same code with a validity mask built from the ids (64 shuffles per chunk) and the
-// diagonal test col > row.
+// Dirty tiles apply a validity mask built from the ids (64 shuffles per chunk) and the diagonal test col > row.
 //
 // Row order inside the sweep: every row / column index in this file is a PLANE row.  The planes, lvl and cinfo store
 // each 128-row block of the sorted order with its rows dealt round-robin to the four TMEM lane quadrants
@@ -308,6 +308,130 @@ struct EvalSymEpi {
       st.dirty |= rbi < p.n_row_blocks ? (int)__ldg(p.dirty + (size_t)rbi * p.n_col_tiles + t) : 1;
   }
 
+  // Counting compares.  set.gt.f32.f32 is one FSET writing 1.0f (0x3f800000 = 127 << 23) or 0; summed as INTEGERS,
+  // two per IADD3, k of them give 127 k << 23 (mod 2^32), and k < 512 comes back through the inverse of 127 mod 512
+  // (383).  The usual (s > t) ? 1 : 0 compiles to FSETP + SEL, one instruction more per compare.
+  __device__ static __forceinline__ unsigned gt_one(float a, float b) {
+    float r;
+    asm("set.gt.f32.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
+    return __float_as_uint(r);
+  }
+  __device__ static __forceinline__ unsigned ones_count(unsigned sum) { return ((sum >> 23) * 383u) & 511u; }
+  // m |= bit if a > b: FSETP + a predicated LOP3 (the ternary form compiles to FSETP + SEL + half an IADD3)
+  __device__ static __forceinline__ void set_if_gt(unsigned& m, float a, float b, unsigned bit) {
+    asm("{\n.reg .pred p;\nsetp.gt.f32 p, %1, %2;\n@p or.b32 %0, %0, %3;\n}" : "+r"(m) : "f"(a), "f"(b), "r"(bit));
+  }
+
+  // Clean tile (no ids, no diagonal, no top-k): the same counts as the dense masks of chunk32 with a quarter fewer
+  // instructions per element (SASS of EvalSymEpi<4>: about 620 instead of 830 per 32 x 32 chunk, queue excluded).  Both directions rely on the thresholds being ascending (t_j <= t_{j+1}, the
+  // K_pos sort), so that an element above level j+1 is above level j too: bucket j holds c_j - c_{j+1} elements,
+  // c_j = #{s > t_j}, and levels 0 .. kLv-2 need COUNTS only (gt_one: FSET + half an IADD3 each).  A mask is built for the
+  // last level alone (it feeds the queue).
+  //   * rows: the thread's row against its thresholds in registers;
+  //   * columns: the chunk is transposed through the warp's staging area, 16 columns at a time (lane = column
+  //     16 h + lane % 16, rows 16 (lane / 16) .. +16), so that a lane compares against ITS column's thresholds held
+  //     in registers -- no broadcast load per element, no bit transposes of the bucket masks.  The two row halves
+  //     of a column meet in one shuffle of byte-packed bucket counts; only the last level's mask goes back to the
+  //     row layout (one bit transpose) for the queue.
+  __device__ static __forceinline__ void chunk32_clean(const Params& p, RowState& st, int col0, const uint32_t (&acc)[32],
+                                                       const EpiCtx& ctx, const float4* lv, const uint2* cinf, int lane) {
+    constexpr int kCnt = kLv - 1;  // counted levels
+    unsigned nr[kCnt];             // c_j of the row, as sums of gt_one
+    unsigned dr = 0u;
+#pragma unroll
+    for (int j = 0; j < kCnt; ++j) nr[j] = 0u;
+#pragma unroll
+    for (int e = 0; e < 32; ++e) {
+      const float s = __uint_as_float(acc[e]);
+#pragma unroll
+      for (int j = 0; j < kCnt; ++j) nr[j] += gt_one(s, st.t[j]);
+      set_if_gt(dr, s, st.t[kCnt], 1u << e);
+    }
+#pragma unroll
+    for (int j = 0; j < kCnt - 1; ++j) st.rc[j] += ones_count(nr[j] - nr[j + 1]);
+    st.rc[kCnt - 1] += ones_count(nr[kCnt - 1]) - (unsigned)__popc(dr);
+
+    // columns.  Staging layout of half h: element (row r, column 16 h + e) at e * 32 + (r ^ 4 (e % 8)): the lanes'
+    // stores of one column hit 32 banks, and the 16-byte loads of four rows of a column stay contiguous and spread
+    // over the banks of each 8-lane phase
+    float* stg = stage(ctx);
+    const int cc = lane & 15, r0 = lane & 16;
+    unsigned cpk = 0u, cdm = 0u;  // lane's column (col0 + lane): bucket counts (one byte per counted level), deep rows
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+#pragma unroll
+      for (int e = 0; e < 16; ++e) stg[e * 32 + (lane ^ ((e & 7) << 2))] = __uint_as_float(acc[h * 16 + e]);
+      __syncwarp();
+      const float4 tc = lv[h * 16 + cc];
+      const float* src = stg + cc * 32;
+      const int sw = (cc & 7) << 2;
+      unsigned nc[kCnt];
+      unsigned dch = 0u;
+#pragma unroll
+      for (int j = 0; j < kCnt; ++j) nc[j] = 0u;
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        const float4 q = *reinterpret_cast<const float4*>(src + ((r0 + 4 * k) ^ sw));
+        const float v4[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+#pragma unroll
+          for (int j = 0; j < kCnt; ++j) nc[j] += gt_one(v4[i], lvl_of(tc, j));
+          set_if_gt(dch, v4[i], lvl_of(tc, kCnt), 1u << (4 * k + i));
+        }
+      }
+      __syncwarp();  // (every lane has read the half before the next one, or the queue push, overwrites it)
+      unsigned pk = (ones_count(nc[kCnt - 1]) - (unsigned)__popc(dch)) << (8 * (kCnt - 1));
+#pragma unroll
+      for (int j = 0; j < kCnt - 1; ++j) pk += ones_count(nc[j] - nc[j + 1]) << (8 * j);
+      pk += __shfl_xor_sync(0xffffffffu, pk, 16);  // <= 32 per byte
+      const unsigned other = __shfl_xor_sync(0xffffffffu, dch, 16);
+      if ((lane >> 4) == h) {
+        cpk = pk;
+        cdm = r0 ? (other | (dch << 16)) : (dch | (other << 16));
+      }
+    }
+    if (cpk != 0u) {
+      const unsigned coff = cinf[lane].x;
+#pragma unroll
+      for (int j = 0; j < kCnt; ++j) {
+        const unsigned n = (cpk >> (8 * j)) & 0xffu;
+        if (n != 0u) atomicAdd(p.hist + coff + j, n);
+      }
+    }
+    const unsigned dc = __any_sync(0xffffffffu, cdm != 0u) ? bit_transpose32(cdm, lane) : 0u;
+    enqueue(p, st, ctx, acc, dr, dc, 0u, 0u, cinf, col0, lane);
+  }
+
+  // ---- elements above the kLv-th threshold (and top-k candidates): queue
+  __device__ static __forceinline__ void enqueue(const Params& p, RowState& st, const EpiCtx& ctx, const uint32_t (&acc)[32],
+                                                 unsigned dr, unsigned dc, unsigned tkr, unsigned tkc, const uint2* cinf,
+                                                 int col0, int lane) {
+    constexpr unsigned kFull = 0xffffffffu;
+    if (!__any_sync(kFull, (dr | dc | tkr | tkc) != 0u)) return;
+    const int mine = __popc(dr) + __popc(dc) + __popc(tkr) + __popc(tkc);
+    const int incl = warp_incl_scan(mine, lane);
+    const int total = __shfl_sync(kFull, incl, 31);
+    if (st.qn + total > kQueueCap) drain(p, st, ctx);
+    if (total <= kQueueCap) {
+      push(st, ctx, acc, dr, dc, cinf, st.qn + incl - mine, tkr, tkc, col0);
+      st.qn += total;
+    } else {
+      // a chunk denser than the whole queue: kQueueCap / 64 columns (<= kQueueCap entries) at a time
+      constexpr int kBatchCols = kQueueCap / (kTopk ? 128 : 64);
+      static_assert(kBatchCols >= 1 && 32 % kBatchCols == 0, "queue capacity: 64 (128 with top-k) .. 2048, a power of two");
+#pragma unroll 1
+      for (int g = 0; g < 32 / kBatchCols; ++g) {
+        const unsigned sel = ((1u << kBatchCols) - 1u) << (kBatchCols * g);
+        const int mine_g = __popc(dr & sel) + __popc(dc & sel) + __popc(tkr & sel) + __popc(tkc & sel);
+        const int incl_g = warp_incl_scan(mine_g, lane);
+        push(st, ctx, acc, dr & sel, dc & sel, cinf, incl_g - mine_g, tkr & sel, tkc & sel, col0);
+        st.qn = __shfl_sync(kFull, incl_g, 31);
+        drain(p, st, ctx);
+      }
+    }
+  }
+
   __device__ static __forceinline__ void chunk32(const Params& p, RowState& st, int row, int col0,
                                                  const uint32_t (&acc)[32], const GemmShape& sh, const EpiCtx& ctx) {
     constexpr unsigned kFull = 0xffffffffu;
@@ -315,6 +439,12 @@ struct EvalSymEpi {
     (void)row;
     const float4* lv = reinterpret_cast<const float4*>(ctx.col_slot) + (col0 & (kTileN - 1));
     const uint2* cinf = reinterpret_cast<const uint2*>(ctx.col_slot + kLvlBytes) + (col0 & (kTileN - 1));
+    if constexpr (!kTopk) {
+      if (!st.dirty) {
+        chunk32_clean(p, st, col0, acc, ctx, lv, cinf, lane);
+        return;
+      }
+    }
 
     unsigned m[kLv], mc[kLv];
     unsigned tkr = 0u, tkc = 0u;  // kTopk: elements above the row's / the column's top-k bound
@@ -380,30 +510,7 @@ struct EvalSymEpi {
       }
     }
 
-    // ---- deeper elements (and top-k candidates): queue
-    const unsigned dr = m[kLv - 1], dc = mc[kLv - 1];
-    if (!__any_sync(kFull, (dr | dc | tkr | tkc) != 0u)) return;
-    const int mine = __popc(dr) + __popc(dc) + __popc(tkr) + __popc(tkc);
-    const int incl = warp_incl_scan(mine, lane);
-    const int total = __shfl_sync(kFull, incl, 31);
-    if (st.qn + total > kQueueCap) drain(p, st, ctx);
-    if (total <= kQueueCap) {
-      push(st, ctx, acc, dr, dc, cinf, st.qn + incl - mine, tkr, tkc, col0);
-      st.qn += total;
-    } else {
-      // a chunk denser than the whole queue: kQueueCap / 64 columns (<= kQueueCap entries) at a time
-      constexpr int kBatchCols = kQueueCap / (kTopk ? 128 : 64);
-      static_assert(kBatchCols >= 1 && 32 % kBatchCols == 0, "queue capacity: 64 (128 with top-k) .. 2048, a power of two");
-#pragma unroll 1
-      for (int g = 0; g < 32 / kBatchCols; ++g) {
-        const unsigned sel = ((1u << kBatchCols) - 1u) << (kBatchCols * g);
-        const int mine_g = __popc(dr & sel) + __popc(dc & sel) + __popc(tkr & sel) + __popc(tkc & sel);
-        const int incl_g = warp_incl_scan(mine_g, lane);
-        push(st, ctx, acc, dr & sel, dc & sel, cinf, incl_g - mine_g, tkr & sel, tkc & sel, col0);
-        st.qn = __shfl_sync(kFull, incl_g, 31);
-        drain(p, st, ctx);
-      }
-    }
+    enqueue(p, st, ctx, acc, m[kLv - 1], mc[kLv - 1], tkr, tkc, cinf, col0, lane);
   }
 
   __device__ static __forceinline__ void tile_end(const Params& p, RowState& st, const GemmShape&, const EpiCtx& ctx) {

@@ -83,20 +83,33 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
 #define WEALY_DEADLOCK_CYCLES (4000000000ll)  // ~2 s at 2 GHz: a stuck pipeline traps instead of hanging the GPU
 #endif
 
-// Spin on the barrier phase.  try_wait suspends in hardware for a bounded time, so the loop is
-// cheap; the clock check turns a protocol bug into a trap (reported as a CUDA error) instead of
-// a hang that would take the whole GPU box down.
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  if (mbar_try_wait(bar, parity)) return;
-  const long long t0 = clock64();
+// The deadlock clock of a waiting thread: read once per kClockPolls failed polls, not per poll (the poll loops are a
+// fifth of the symmetric sweep's executed instructions).  The first read starts the count, so a wait that ends within
+// kClockPolls polls reads no clock at all; a stuck protocol still traps within seconds.
+constexpr int kClockPolls = 2048;
+struct DeadlockClock {
+  long long t0 = 0;
   int polls = 0;
-  while (!mbar_try_wait(bar, parity)) {
-    if ((++polls & 63) == 0 && clock64() - t0 > WEALY_DEADLOCK_CYCLES) {
-      printf("wealy: mbarrier deadlock block=%d thread=%d bar=0x%x parity=%u\n", (int)blockIdx.x,
-             (int)threadIdx.x, smem_u32(bar), parity);
+  __device__ __forceinline__ void tick(const char* what, uint64_t* bar, uint32_t parity) {
+    if (++polls < kClockPolls) return;
+    polls = 0;
+    const long long now = clock64();
+    if (t0 == 0) {
+      t0 = now;
+    } else if (now - t0 > WEALY_DEADLOCK_CYCLES) {
+      printf("wealy: %s deadlock block=%d thread=%d bar=0x%x parity=%u\n", what, (int)blockIdx.x, (int)threadIdx.x,
+             smem_u32(bar), parity);
       __trap();
     }
   }
+};
+
+// Spin on the barrier phase.  try_wait suspends in hardware for a bounded time; the clock check turns a protocol bug
+// into a trap (reported as a CUDA error) instead of a hang that would take the whole GPU box down.
+__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
+  if (mbar_try_wait(bar, parity)) return;
+  DeadlockClock clk;
+  while (!mbar_try_wait(bar, parity)) clk.tick("mbarrier", bar, parity);
 }
 
 // The same for a whole warp: one lane polls, the others wait at the warp barrier (32x fewer polling lanes)
@@ -241,29 +254,26 @@ __device__ __forceinline__ void mbar_arrive_cluster_relaxed(uint32_t cluster_add
 __device__ __forceinline__ void st_cluster_u32(uint32_t cluster_addr, uint32_t v) {
   asm volatile("st.shared::cluster.u32 [%0], %1;" ::"r"(cluster_addr), "r"(v) : "memory");
 }
+__device__ __forceinline__ bool mbar_try_wait_cluster(uint64_t* bar, uint32_t parity) {
+  uint32_t ok;
+  // (with the suspend-time hint of mbar_try_wait: an un-hinted poll loop was 25 % of the pair kernel's instructions)
+  asm volatile(
+      "{\n"
+      ".reg .pred P;\n"
+      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P, [%1], %2, %3;\n"
+      "selp.u32 %0, 1, 0, P;\n"
+      "}\n"
+      : "=r"(ok)
+      : "r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)(WEALY_WAIT_HINT_NS > 0 ? WEALY_WAIT_HINT_NS : 1))
+      : "memory");
+  return ok != 0;
+}
+
 // wait with cluster-scope acquire: the barrier is signalled by the peer CTA
 __device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-  const long long t0 = clock64();
-  int polls = 0;
-  while (true) {
-    uint32_t ok;
-    // (with the suspend-time hint of mbar_try_wait: an un-hinted poll loop was 25 % of the pair kernel's instructions)
-    asm volatile(
-        "{\n"
-        ".reg .pred P;\n"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P, [%1], %2, %3;\n"
-        "selp.u32 %0, 1, 0, P;\n"
-        "}\n"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)(WEALY_WAIT_HINT_NS > 0 ? WEALY_WAIT_HINT_NS : 1))
-        : "memory");
-    if (ok) return;
-    if ((++polls & 63) == 0 && clock64() - t0 > WEALY_DEADLOCK_CYCLES) {
-      printf("wealy: cluster mbarrier deadlock block=%d thread=%d bar=0x%x parity=%u\n", (int)blockIdx.x,
-             (int)threadIdx.x, smem_u32(bar), parity);
-      __trap();
-    }
-  }
+  if (mbar_try_wait_cluster(bar, parity)) return;
+  DeadlockClock clk;
+  while (!mbar_try_wait_cluster(bar, parity)) clk.tick("cluster mbarrier", bar, parity);
 }
 
 // a whole warp waiting on a cluster-scope barrier: one lane polls (see mbar_wait_warp)

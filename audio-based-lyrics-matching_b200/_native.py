@@ -79,7 +79,10 @@ SIGNATURES = {
     "wealy_eval_plan_stage_ms": (c_int, [c_vp, ctypes.POINTER(c_f32)]),
     "wealy_eval_plan_destroy": (None, [c_vp]),
     "wealy_masked_reduce": (c_int, [c_vp, c_vp, c_i64, c_i64, c_int, c_int, c_f32, c_f32, c_vp, c_vp]),
+    "wealy_masked_reduce_backward": (c_int, [c_vp, c_vp, c_i64, c_i64, c_int, c_int, c_f32, c_f32, c_int, c_vp, c_vp, c_vp]),
     "wealy_distance_redux": (c_int, [c_vp, c_vp, c_i64, c_int, c_int, c_int, c_int, c_int, c_int, c_f32, c_f32, c_vp, c_vp]),
+    "wealy_distance_redux_backward": (c_int, [c_vp, c_vp, c_i64, c_int, c_int, c_int, c_int, c_int, c_int, c_f32, c_f32, c_vp,
+                                              c_vp, c_vp]),
     "wealy_mean_pool": (c_int, [c_vp, c_vp, c_i64, c_i64, c_i64, c_int, c_vp, c_int, c_vp]),
     "wealy_segment_mean": (c_int, [c_vp, c_vp, c_i64, c_i64, c_int, c_vp, c_vp]),
     "wealy_triplet_mine": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp]),

@@ -2100,6 +2100,39 @@ extern "C" int wealy_masked_reduce(const void* x, const uint8_t* mask, int64_t r
   }
 }
 
+template <typename T, typename A>
+static int launch_masked_backward(const void* x, const unsigned char* mask, int64_t rows, int64_t cols, int op, int full,
+                                  float fill, float eps, const void* g, void* dx, cudaStream_t s) {
+  if (cols <= 2048 || rows >= 4096) {
+    const int threads = 256;
+    const unsigned blocks = (unsigned)ceil_div(rows * 32, threads);
+    masked_reduce_backward_warp_kernel<T, A><<<blocks, threads, 0, s>>>((const T*)x, mask, rows, cols, op, full, (A)fill, (A)eps,
+                                                                        (const T*)g, (T*)dx);
+  } else {
+    masked_reduce_backward_block_kernel<T, A><<<(unsigned)rows, 1024, 0, s>>>((const T*)x, mask, rows, cols, op, full, (A)fill,
+                                                                              (A)eps, (const T*)g, (T*)dx);
+  }
+  CU_TRY(cudaGetLastError());
+  return WEALY_OK;
+}
+
+extern "C" int wealy_masked_reduce_backward(const void* x, const uint8_t* mask, int64_t rows, int64_t cols, int dtype, int op,
+                                            float fill, float eps, int full, const void* g, void* dx, void* stream) {
+  if (rows < 0 || cols < 0) return fail(WEALY_ERR_BAD_ARG, "bad shape rows=%lld cols=%lld", (long long)rows, (long long)cols);
+  if (rows == 0 || cols == 0) return WEALY_OK;
+  if (!x || !g || !dx) return fail(WEALY_ERR_BAD_ARG, "null pointer");
+  if (op < WEALY_MASKED_SUM || op > WEALY_MASKED_MAX) return fail(WEALY_ERR_BAD_ARG, "unknown masked op %d", op);
+  if (rows > 2000000000ll) return fail(WEALY_ERR_UNSUPPORTED, "too many rows");
+  cudaStream_t s = (cudaStream_t)stream;
+  switch (dtype) {
+    case WEALY_F32: return launch_masked_backward<float, float>(x, mask, rows, cols, op, full, fill, eps, g, dx, s);
+    case WEALY_F16: return launch_masked_backward<__half, float>(x, mask, rows, cols, op, full, fill, eps, g, dx, s);
+    case WEALY_BF16: return launch_masked_backward<__nv_bfloat16, float>(x, mask, rows, cols, op, full, fill, eps, g, dx, s);
+    case WEALY_F64: return launch_masked_backward<double, double>(x, mask, rows, cols, op, full, fill, eps, g, dx, s);
+    default: return fail(WEALY_ERR_BAD_ARG, "unknown element type %d", dtype);
+  }
+}
+
 // a4: distance_tensor_redux (lib/tensor_ops.py:288-373) in one launch -- csrc/redux_kernels.cuh
 extern "C" int wealy_distance_redux(const void* dist, const uint8_t* mask, int64_t pairs, int s1, int s2, int dtype, int op,
                                     int karg, int symmetric, float eps, float inf, void* out, void* stream) {
@@ -2120,6 +2153,33 @@ extern "C" int wealy_distance_redux(const void* dist, const uint8_t* mask, int64
     default: return fail(WEALY_ERR_BAD_ARG, "unknown element type %d", dtype);
   }
 #undef WEALY_RDX
+  CU_TRY(cudaGetLastError());
+  return WEALY_OK;
+}
+
+extern "C" int wealy_distance_redux_backward(const void* dist, const uint8_t* mask, int64_t pairs, int s1, int s2, int dtype, int op,
+                                             int karg, int symmetric, float eps, float inf, const void* g, void* ddist, void* stream) {
+  if (pairs < 0 || s1 < 1 || s2 < 1) return fail(WEALY_ERR_BAD_ARG, "bad shape pairs=%lld s1=%d s2=%d", (long long)pairs, s1, s2);
+  if (s1 > kReduxMaxS || s2 > kReduxMaxS) return fail(WEALY_ERR_UNSUPPORTED, "more than %d chunks per track", kReduxMaxS);
+  if (op < WEALY_RDX_MIN || op > WEALY_RDX_BPWR) return fail(WEALY_ERR_BAD_ARG, "unknown redux op %d", op);
+  if (pairs == 0) return WEALY_OK;
+  if (!dist || !g || !ddist) return fail(WEALY_ERR_BAD_ARG, "null pointer");
+  if (pairs > 3ll * 2000000000ll) return fail(WEALY_ERR_UNSUPPORTED, "too many pairs");
+  cudaStream_t s = (cudaStream_t)stream;
+#define WEALY_RDX_BWD(T, A)                                                                                                          \
+  redux_pairs_backward_kernel<T, A><<<(unsigned)ceil_div(pairs, redux_bwd_warps<A>()), 32 * redux_bwd_warps<A>(), 0, s>>>(          \
+      (const T*)dist, mask, (long long)pairs, s1, s2, op, karg, symmetric, (A)eps, (A)inf, (const T*)g, (T*)ddist)
+  switch (dtype) {
+    case WEALY_F32: WEALY_RDX_BWD(float, float); break;
+    case WEALY_F16: WEALY_RDX_BWD(__half, float); break;
+    case WEALY_BF16: WEALY_RDX_BWD(__nv_bfloat16, float); break;
+    case WEALY_F64:
+      if (pairs > 2000000000ll) return fail(WEALY_ERR_UNSUPPORTED, "too many pairs");
+      WEALY_RDX_BWD(double, double);
+      break;
+    default: return fail(WEALY_ERR_BAD_ARG, "unknown element type %d", dtype);
+  }
+#undef WEALY_RDX_BWD
   CU_TRY(cudaGetLastError());
   return WEALY_OK;
 }

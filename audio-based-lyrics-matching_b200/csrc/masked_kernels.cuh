@@ -101,4 +101,126 @@ __global__ void __launch_bounds__(1024) masked_reduce_block_kernel(const T* __re
   }
 }
 
+// ---- backward: dx = g[row] * w_e, the weights fixed by the forward's selection (rerun here, no index output) ----
+//   sum: 1 on included entries;  mean: 1 / max(count, eps) on included entries;
+//   min / max over given dims: one-hot on the FIRST extreme of the filled row (excluded entries hold `fill`, a NaN is
+//     the extreme), dropped when that entry is excluded -- the caller orders the columns so that "first" is the
+//     reference's order (it reduces the dims one at a time with torch.min(d));
+//   min / max with dim=None (full != 0): torch.min() spreads the gradient evenly over every position equal to the
+//     extreme (NaN: every NaN), excluded positions included in the count, their share dropped.
+// Arithmetic in A (float, double for float64 inputs); dx in x's dtype.
+template <typename A, typename T>
+__device__ __forceinline__ A ld_acc(const T* p, long long i) {
+  if constexpr (sizeof(A) == 8) return (A)p[i]; else return (A)to_f32<T>(p[i]);
+}
+template <typename T, typename A>
+__device__ __forceinline__ void st_acc(T* p, long long i, A v) {
+  if constexpr (sizeof(A) == 8) p[i] = (T)v; else p[i] = from_f32<T>((float)v);
+}
+
+template <typename A>
+__device__ __forceinline__ bool same_value(A a, A b) { return a == b || (a != a && b != b); }
+
+// a strictly more extreme than b (a NaN beats every number)
+template <typename A>
+__device__ __forceinline__ bool beats(A a, A b, bool take_min) {
+  if (a != a) return b == b;
+  return take_min ? a < b : a > b;
+}
+
+template <typename A>
+struct MaskedSel {
+  A cnt;          // included entries (mean)
+  A v;            // extreme of the filled row (min / max)
+  long long idx;  // its first position
+  long long ties; // positions equal to it
+  __device__ __forceinline__ void take(A w, long long i, long long t, bool take_min) {
+    if (beats(w, v, take_min)) { v = w; idx = i; ties = t; }
+    else if (same_value(w, v)) { ties += t; idx = i < idx ? i : idx; }
+  }
+  __device__ __forceinline__ void warp_merge(bool take_min) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
+      const A ov = __shfl_xor_sync(0xffffffffu, v, o);
+      const long long oi = __shfl_xor_sync(0xffffffffu, idx, o), ot = __shfl_xor_sync(0xffffffffu, ties, o);
+      take(ov, oi, ot, take_min);
+    }
+  }
+};
+
+template <typename T, typename A>
+__device__ __forceinline__ void masked_sel_visit(MaskedSel<A>& s, const T* __restrict__ x, const unsigned char* __restrict__ mask,
+                                                 long long base, long long c, int op, A fill) {
+  const bool excluded = mask != nullptr && mask[base + c] != 0;
+  if (op == kMMean) { s.cnt += excluded ? (A)0 : (A)1; return; }
+  s.take(excluded ? fill : ld_acc<A>(x, base + c), c, 1, op == kMMin);
+}
+
+template <typename T, typename A>
+__device__ __forceinline__ void masked_grad_write(const MaskedSel<A>& s, const T* __restrict__ x,
+                                                  const unsigned char* __restrict__ mask, long long base, long long c, int op,
+                                                  int full, A fill, A eps, A g, T* __restrict__ dx) {
+  const bool excluded = mask != nullptr && mask[base + c] != 0;
+  A d;
+  if (op == kMSum) d = g * (excluded ? (A)0 : (A)1);
+  else if (op == kMMean) d = (g / (s.cnt > eps ? s.cnt : eps)) * (excluded ? (A)0 : (A)1);
+  else if (!full) d = (c == s.idx && !excluded) ? g : (A)0;
+  else d = (!excluded && same_value(ld_acc<A>(x, base + c), s.v)) ? g / (A)s.ties : (A)0;
+  st_acc<T>(dx, base + c, d);
+}
+
+template <typename A>
+__device__ __forceinline__ MaskedSel<A> masked_sel_init(int op) {
+  const A inf = (A)__int_as_float(0x7f800000);
+  return MaskedSel<A>{(A)0, op == kMMin ? inf : -inf, 0x7fffffffffffffffll, 0};
+}
+
+// one warp per row
+template <typename T, typename A>
+__global__ void __launch_bounds__(256) masked_reduce_backward_warp_kernel(const T* __restrict__ x,
+                                                                          const unsigned char* __restrict__ mask, long long rows,
+                                                                          long long cols, int op, int full, A fill, A eps,
+                                                                          const T* __restrict__ g, T* __restrict__ dx) {
+  const long long row = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+  const int lane = (int)(threadIdx.x & 31);
+  if (row >= rows) return;
+  const long long base = row * cols;
+  MaskedSel<A> s = masked_sel_init<A>(op);
+  if (op != kMSum) {
+    for (long long c = lane; c < cols; c += 32) masked_sel_visit<T, A>(s, x, mask, base, c, op, fill);
+    s.warp_merge(op == kMMin);
+  }
+  const A gr = ld_acc<A>(g, row);
+  for (long long c = lane; c < cols; c += 32) masked_grad_write<T, A>(s, x, mask, base, c, op, full, fill, eps, gr, dx);
+}
+
+// one block per row (long rows)
+template <typename T, typename A>
+__global__ void __launch_bounds__(1024) masked_reduce_backward_block_kernel(const T* __restrict__ x,
+                                                                            const unsigned char* __restrict__ mask, long long rows,
+                                                                            long long cols, int op, int full, A fill, A eps,
+                                                                            const T* __restrict__ g, T* __restrict__ dx) {
+  __shared__ MaskedSel<A> s_sel[32];
+  const long long row = blockIdx.x;
+  const long long base = row * cols;
+  const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
+  MaskedSel<A> s = masked_sel_init<A>(op);
+  if (op != kMSum) {
+    for (long long c = threadIdx.x; c < cols; c += blockDim.x) masked_sel_visit<T, A>(s, x, mask, base, c, op, fill);
+    s.warp_merge(op == kMMin);
+    if (l == 0) s_sel[w] = s;
+    __syncthreads();
+    if (w == 0) {
+      s = l < (int)(blockDim.x >> 5) ? s_sel[l] : masked_sel_init<A>(op);
+      s.warp_merge(op == kMMin);
+      if (l == 0) s_sel[0] = s;
+    }
+    __syncthreads();
+    s = s_sel[0];
+  }
+  const A gr = ld_acc<A>(g, row);
+  for (long long c = threadIdx.x; c < cols; c += blockDim.x) masked_grad_write<T, A>(s, x, mask, base, c, op, full, fill, eps, gr, dx);
+}
+
 }  // namespace wealy

@@ -27,9 +27,11 @@ enum ReduxOp : int { kRdxMin = 0, kRdxMax = 1, kRdxMean = 2, kRdxMinMean = 3, kR
 constexpr int kReduxMaxS = 32;  // chunks per track on either side
 
 // One strategy on the block held in shared memory: x[i * ld_i + j * ld_j] (i < n1 rows, j < n2 columns), mk likewise.
-template <typename A>
+// kGrad: the backward reuses the forward's selection and adds scale * w_e (out = sum_e w_e x_e) to wt[i * ld_i + j * ld_j]
+// for the entries it selected; the forward's arithmetic is the same in both instantiations.
+template <typename A, bool kGrad = false>
 __device__ A redux_block(int op, int karg, const A* x, unsigned char* mk, int n1, int n2, int ld_i, int ld_j, A eps, A inf_, int lane,
-                         A* agg /*[32]*/, A* work /*[1024]*/) {
+                         A* agg /*[32]*/, A* work /*[1024]*/, A* wt = nullptr, A scale = 0) {
   constexpr unsigned kFull = 0xffffffffu;
   const int n = n1 * n2;
   auto at = [&](int i, int j) { return x[i * ld_i + j * ld_j]; };
@@ -55,6 +57,8 @@ __device__ A redux_block(int op, int karg, const A* x, unsigned char* mk, int n1
     }
     return v;
   };
+  auto same = [](A a, A b) { return a == b || (a != a && b != b); };
+  auto add_w = [&](int i, int j, A v) { wt[i * ld_i + j * ld_j] += v; };
   if (op == kRdxMin || op == kRdxMax) {
     A v = op == kRdxMin ? inf_ : -inf_;
     bool any = false;
@@ -64,7 +68,19 @@ __device__ A redux_block(int op, int karg, const A* x, unsigned char* mk, int n1
       if (w != w) { v = w; any = true; }
       else if (!any) v = op == kRdxMin ? (w < v ? w : v) : (w > v ? w : v);
     }
-    return op == kRdxMin ? wmin(v) : wmax(v);
+    v = op == kRdxMin ? wmin(v) : wmax(v);
+    if constexpr (kGrad) {
+      // one-hot on the first extreme in row-major order of the (oriented) block, dropped when it is excluded
+      int first = n;
+      for (int e = lane; e < n && first == n; e += 32) {
+        const int i = e / n2, j = e - i * n2;
+        if (same(ex(i, j) ? (op == kRdxMin ? inf_ : -inf_) : at(i, j), v)) first = e;
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) first = min(first, __shfl_xor_sync(kFull, first, o));
+      if (lane == 0 && first < n && !ex(first / n2, first % n2)) add_w(first / n2, first % n2, scale);
+    }
+    return v;
   }
   if (op == kRdxMean) {
     A s = 0, c = 0;
@@ -76,6 +92,13 @@ __device__ A redux_block(int op, int karg, const A* x, unsigned char* mk, int n1
     }
     s = wsum(s);
     c = wsum(c);
+    if constexpr (kGrad) {
+      const A q = scale / (c > eps ? c : eps);
+      for (int e = lane; e < n; e += 32) {
+        const int i = e / n2, j = e - i * n2;
+        if (!ex(i, j)) add_w(i, j, q);
+      }
+    }
     return s / (c > eps ? c : eps);
   }
   if (op == kRdxMinMean || op == kRdxMeanMin) {
@@ -105,7 +128,18 @@ __device__ A redux_block(int op, int karg, const A* x, unsigned char* mk, int n1
     if (op == kRdxMinMean) {
       // min over the rows that have an included entry (their mean stands at every included position)
       A v = (lane < n1 && cnt > 0) ? r : inf_;
-      return wmin(v);
+      v = wmin(v);
+      if constexpr (kGrad) {
+        // the first row with an included entry whose mean is the minimum: 1 / max(cnt_i, eps) on its included entries
+        const unsigned rows = __ballot_sync(kFull, lane < n1 && cnt > 0 && same(r, v));
+        if (rows) {
+          const int i = __ffs(rows) - 1;
+          const A ci = __shfl_sync(kFull, cnt, i);
+          const A q = scale / (ci > eps ? ci : eps);
+          if (lane < n2 && !ex(i, lane)) add_w(i, lane, q);
+        }
+      }
+      return v;
     }
     // mean of the row minima, every row weighted by its number of included entries
     A s = lane < n1 ? (cnt > 0 ? cnt * r : (A)0 * r) : (A)0;
@@ -114,6 +148,14 @@ __device__ A redux_block(int op, int karg, const A* x, unsigned char* mk, int n1
     }
     s = wsum(s);
     const A c = wsum(lane < n1 ? cnt : (A)0);
+    if constexpr (kGrad) {
+      // the reference broadcasts the row minima against the mask: row i's first argmin carries cnt_i / max(C, eps)
+      if (lane < n1 && cnt > 0) {
+        int j = 0;
+        while (j < n2 && !same(ex(lane, j) ? inf_ : at(lane, j), r)) ++j;
+        if (j < n2 && !ex(lane, j)) add_w(lane, j, scale * cnt / (c > eps ? c : eps));
+      }
+    }
     return s / (c > eps ? c : eps);
   }
   if (op == kRdxBest || op == kRdxWorst) {
@@ -125,6 +167,7 @@ __device__ A redux_block(int op, int karg, const A* x, unsigned char* mk, int n1
     }
     __syncwarp();
     A s = 0, c = 0;
+    unsigned kept = 0;  // (kGrad) bit e / 32: this lane's entry e was selected and is included
     for (int e = lane; e < n; e += 32) {
       const A v = work[e];
       int rank = 0;
@@ -137,11 +180,17 @@ __device__ A redux_block(int op, int karg, const A* x, unsigned char* mk, int n1
         const bool excluded = op == kRdxBest ? (v >= inf_) : (v >= -inf_);
         s += excluded ? (A)0 * v : v;
         c += excluded ? (A)0 : (A)1;
+        if constexpr (kGrad) kept |= excluded ? 0u : 1u << (e >> 5);
       }
     }
     __syncwarp();
     s = wsum(s);
     c = wsum(c);
+    if constexpr (kGrad) {
+      const A q = scale / (c > eps ? c : eps);
+      for (int e = lane; e < n; e += 32)
+        if ((kept >> (e >> 5)) & 1u) add_w(e / n2, e - (e / n2) * n2, q);
+    }
     return s / (c > eps ? c : eps);
   }
   // ---- bpwr: greedy best pairs without replacement (the block is already jittered by the caller)
@@ -192,6 +241,11 @@ __device__ A redux_block(int op, int karg, const A* x, unsigned char* mk, int n1
     }
     s = wsum(s);
     c = wsum(c);
+    if constexpr (kGrad) {
+      const A q = scale / (c > eps ? c : eps);
+      for (int e = lane; e < n; e += 32)
+        if (picked[e]) add_w(e / n2, e - (e / n2) * n2, q);
+    }
     (void)agg;
     return s / (c > eps ? c : eps);
   }
@@ -199,6 +253,29 @@ __device__ A redux_block(int op, int karg, const A* x, unsigned char* mk, int n1
 
 template <typename A>
 __host__ __device__ constexpr int redux_warps() { return sizeof(A) == 8 ? 2 : 4; }  // static shared memory: 2 x 1024 A + 2 x 1024 bytes per warp
+
+// The strategy on one staged block (xs, ms = working mask, ms0 = the caller's mask), "s" prefix included.  bpwr works on
+// the orientation with the fewer rows (the reference transposes when s2 < s1).  kGrad: the weights go to wt (zeroed).
+template <typename A, bool kGrad = false>
+__device__ __forceinline__ A redux_pair(int op, int karg, int symmetric, const A* xs, unsigned char* ms, const unsigned char* ms0,
+                                        int s1, int s2, A eps, A inf_, int lane, A* ag, A* ws, A* wt = nullptr) {
+  const int n = s1 * s2;
+  const bool bp = op == kRdxBpwr;
+  const A scale = symmetric ? (A)0.5 : (A)1;
+  auto run = [&](bool transposed) {
+    const bool t = transposed != (bp && ((transposed ? s1 : s2) < (transposed ? s2 : s1)));
+    const int n1 = t ? s2 : s1, n2 = t ? s1 : s2;
+    return redux_block<A, kGrad>(op, karg, xs, ms, n1, n2, t ? 1 : s2, t ? s2 : 1, eps, inf_, lane, ag, ws, wt, scale);
+  };
+  A r = run(false);
+  if (symmetric) {
+    __syncwarp();
+    for (int e = lane; e < n; e += 32) ms[e] = ms0[e];  // (bpwr edits its mask)
+    __syncwarp();
+    r = (A)0.5 * (r + run(true));
+  }
+  return r;
+}
 
 template <typename T, typename A>
 __global__ void __launch_bounds__(128) redux_pairs_kernel(const T* __restrict__ dist, const unsigned char* __restrict__ mask,
@@ -221,22 +298,48 @@ __global__ void __launch_bounds__(128) redux_pairs_kernel(const T* __restrict__ 
     ms[w][e] = ms0[w][e];
   }
   __syncwarp();
-  // bpwr works on the orientation with the fewer rows (the reference transposes when s2 < s1)
-  const bool bp = op == kRdxBpwr;
-  auto run = [&](bool transposed) {
-    const bool t = transposed != (bp && ((transposed ? s1 : s2) < (transposed ? s2 : s1)));
-    const int n1 = t ? s2 : s1, n2 = t ? s1 : s2;
-    return redux_block<A>(op, karg, xs[w], ms[w], n1, n2, t ? 1 : s2, t ? s2 : 1, eps, inf_, lane, ag[w], ws[w]);
-  };
-  A r = run(false);
-  if (symmetric) {
-    __syncwarp();
-    for (int e = lane; e < n; e += 32) ms[w][e] = ms0[w][e];  // (bpwr edits its mask)
-    __syncwarp();
-    r = (A)0.5 * (r + run(true));
-  }
+  const A r = redux_pair<A>(op, karg, symmetric, xs[w], ms[w], ms0[w], s1, s2, eps, inf_, lane, ag[w], ws[w]);
   if (lane == 0) {
     if constexpr (sizeof(A) == 8) out[pair] = (T)r; else out[pair] = from_f32<T>((float)r);
+  }
+}
+
+// The backward of one track pair: d dist[pair][e] = g[pair] * w_e, w_e written by the forward's selection (redux_block<A, true>)
+// rerun on the same (jittered, for bpwr) block.  One warp per pair like the forward; the weights take a third block of
+// shared memory, so a CTA holds one warp fewer (float) / one warp (double) to stay within the 48 KB of static shared memory.
+template <typename A>
+__host__ __device__ constexpr int redux_bwd_warps() { return sizeof(A) == 8 ? 1 : 3; }
+
+template <typename T, typename A>
+__global__ void __launch_bounds__(96) redux_pairs_backward_kernel(const T* __restrict__ dist, const unsigned char* __restrict__ mask,
+                                                                  long long pairs, int s1, int s2, int op, int karg, int symmetric,
+                                                                  A eps, A inf_, const T* __restrict__ g, T* __restrict__ dx) {
+  constexpr int kW = redux_bwd_warps<A>();
+  __shared__ A xs[kW][kReduxMaxS * kReduxMaxS];
+  __shared__ A ws[kW][kReduxMaxS * kReduxMaxS];
+  __shared__ A wt[kW][kReduxMaxS * kReduxMaxS];
+  __shared__ unsigned char ms[kW][kReduxMaxS * kReduxMaxS];
+  __shared__ unsigned char ms0[kW][kReduxMaxS * kReduxMaxS];
+  __shared__ A ag[kW][32];
+  const int w = (int)(threadIdx.x >> 5), lane = (int)(threadIdx.x & 31);
+  const long long pair = blockIdx.x * (long long)kW + w;
+  if (pair >= pairs) return;
+  const int n = s1 * s2;
+  const T* src = dist + pair * n;
+  for (int e = lane; e < n; e += 32) {
+    if constexpr (sizeof(A) == 8) xs[w][e] = (A)src[e]; else xs[w][e] = (A)to_f32<T>(src[e]);
+    ms0[w][e] = mask ? (unsigned char)(mask[pair * n + e] != 0) : 0;
+    ms[w][e] = ms0[w][e];
+    wt[w][e] = 0;
+  }
+  __syncwarp();
+  redux_pair<A, true>(op, karg, symmetric, xs[w], ms[w], ms0[w], s1, s2, eps, inf_, lane, ag[w], ws[w], wt[w]);
+  __syncwarp();
+  A gp;
+  if constexpr (sizeof(A) == 8) gp = (A)g[pair]; else gp = (A)to_f32<T>(g[pair]);
+  T* d = dx + pair * n;
+  for (int e = lane; e < n; e += 32) {
+    if constexpr (sizeof(A) == 8) d[e] = (T)(gp * wt[w][e]); else d[e] = from_f32<T>((float)(gp * wt[w][e]));
   }
 }
 

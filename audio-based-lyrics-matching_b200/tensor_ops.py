@@ -12,12 +12,22 @@ float64 inputs return float64 like the reference: they take a CUDA-core double-p
 torch ops): cos / cossim / dot / dotsim and the euclidean family (sqeuc / nsqeuc / fro / nfro / euc / neuc
 with p = 2, pairwise_euclidean_distance_matrix) run their two gradient products on the same contraction
 core.  cdist with p != 2 is not a contraction and raises NotImplementedError (WEALY_ERR_UNSUPPORTED).
+
+  msum / mmean / mmin / mmax / mrand / mbest / mworst                lib/tensor_ops.py:182-282
+  distance_tensor_redux(dist, redux, mask=None, ...)                lib/tensor_ops.py:288-373
+
+are differentiable too, with the gradient the reference's autograd gives (first order, with respect to x / dist, not
+the mask): every result is a sum of w_e * x_e with weights fixed by a discrete selection, and the backward kernels
+(wealy_masked_reduce_backward, wealy_distance_redux_backward) rerun that selection with the reference's tie rules --
+first extreme for min / max over given dims (the last dim reduced is the most significant), an even split over the
+ties for dim=None, the fused redux's own choice at best-k boundary ties.  Without grad they launch only the forward.
 Inputs must be CUDA tensors -- there is no CPU fallback.
 """
 import ctypes
 import os
 
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import _native as N
 
@@ -316,13 +326,57 @@ _INF = float("inf")
 _OPS = {"sum": 0, "mean": 1, "min": 2, "max": 3}
 
 
+def _masked_launch(xp, mp, op, fill, eps):
+    """wealy_masked_reduce over the columns of the contiguous [rows, cols] xp (mp: its uint8 mask or None) -> [rows]."""
+    rows, cols = xp.shape
+    out = torch.empty(rows, dtype=xp.dtype, device=xp.device)
+    if rows and cols == 0:
+        out.fill_({0: 0.0, 1: 0.0, 2: _INF, 3: -_INF}[op])
+    elif rows:
+        with torch.cuda.device(xp.device):
+            N.check(N.lib.wealy_masked_reduce(xp.data_ptr(), mp.data_ptr() if mp is not None else None, rows, cols,
+                                              N.dtype_code(xp.dtype, allow_f64=True), op, float(fill), float(eps),
+                                              out.data_ptr(), N.stream_ptr(xp.device)))
+    return out
+
+
+class _MaskedReduce(torch.autograd.Function):
+    """msum / mmean / mmin / mmax under autograd: dx = g * w, the weights of the forward's selection, rerun by
+    wealy_masked_reduce_backward (csrc/masked_kernels.cuh).  `full`: dim=None, where torch.min() spreads the gradient
+    over every tied position instead of the first one."""
+
+    @staticmethod
+    def forward(ctx, xp, mp, op, fill, eps, full):
+        ctx.save_for_backward(xp, mp)
+        ctx.cfg = (op, fill, eps, full)
+        return _masked_launch(xp.detach(), mp, op, fill, eps)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        xp, mp = ctx.saved_tensors
+        op, fill, eps, full = ctx.cfg
+        rows, cols = xp.shape
+        dx = torch.empty_like(xp, memory_format=torch.contiguous_format)
+        if rows and cols:
+            g = g.to(xp.dtype).contiguous()
+            with torch.cuda.device(xp.device):
+                N.check(N.lib.wealy_masked_reduce_backward(
+                    xp.data_ptr(), mp.data_ptr() if mp is not None else None, rows, cols,
+                    N.dtype_code(xp.dtype, allow_f64=True), op, float(fill), float(eps), int(full), g.data_ptr(),
+                    dx.data_ptr(), N.stream_ptr(xp.device)))
+        return dx, None, None, None, None, None
+
+
 def _reduce(x, mask, dim, keepdim, op, fill=0.0, eps=1e-7):
     N.require_cuda(x)
-    code = N.dtype_code(x.dtype, allow_f64=True)
+    N.dtype_code(x.dtype, allow_f64=True)
+    grad = x.requires_grad and torch.is_grad_enabled()
     if mask is not None:
         N.require_cuda(mask)
         # like the reference's `included * x` / `torch.where(mask, ctt, x)`, x and mask broadcast together
-        # (minmean / meanmin reduce an already-reduced x against the full-size mask)
+        # (minmean / meanmin reduce an already-reduced x against the full-size mask); under autograd the expand's
+        # backward sums dx back to x's shape
         x, mask = torch.broadcast_tensors(x, mask)
     nd = x.ndim
     if dim is None:
@@ -330,7 +384,17 @@ def _reduce(x, mask, dim, keepdim, op, fill=0.0, eps=1e-7):
     else:
         red = sorted({d % nd for d in ((dim,) if isinstance(dim, int) else tuple(dim))})
     kept = [d for d in range(nd) if d not in red]
-    order = kept + red
+    cols_order = red
+    if grad and dim is not None and op in (_OPS["min"], _OPS["max"]):
+        # the reference reduces the dims one at a time in the caller's order, each taking the first extreme: the last
+        # dim reduced is the most significant for ties.  Flatten the columns in that order so that the kernel's
+        # "first extreme" is the reference's (the value itself does not depend on the order)
+        cols_order = []
+        for d in ((dim,) if isinstance(dim, int) else tuple(dim)):
+            if d % nd not in cols_order:
+                cols_order.append(d % nd)
+        cols_order = cols_order[::-1]
+    order = kept + cols_order
     kept_shape = [x.shape[d] for d in kept]
     rows = 1
     for s_ in kept_shape:
@@ -342,14 +406,10 @@ def _reduce(x, mask, dim, keepdim, op, fill=0.0, eps=1e-7):
     mp = None
     if mask is not None:
         mp = mask.permute(order).contiguous().to(torch.uint8)
-    out = torch.empty(rows, dtype=x.dtype, device=x.device)
-    if rows and cols == 0:
-        out.fill_({0: 0.0, 1: 0.0, 2: _INF, 3: -_INF}[op])
-    elif rows:
-        with torch.cuda.device(x.device):
-            N.check(N.lib.wealy_masked_reduce(xp.data_ptr(), mp.data_ptr() if mp is not None else None, rows, cols,
-                                              code, op, float(fill), float(eps), out.data_ptr(),
-                                              N.stream_ptr(x.device)))
+    if grad:
+        out = _MaskedReduce.apply(xp.view(rows, cols), mp, op, fill, eps, dim is None)
+    else:
+        out = _masked_launch(xp.view(rows, cols), mp, op, fill, eps)
     out = out.view(kept_shape)
     if keepdim:
         for d in red:
@@ -428,21 +488,57 @@ def _redux_plan(redux):
     return None
 
 
+def _redux_launch(d, m, plan, eps, inf):
+    """wealy_distance_redux on the contiguous (b1, b2, s1, s2) block d (m: its uint8 mask or None) -> (b1, b2)."""
+    op, karg, sym = plan
+    b1, b2, s1, s2 = d.shape
+    out = torch.empty((b1, b2), dtype=d.dtype, device=d.device)
+    with torch.cuda.device(d.device):
+        N.check(N.lib.wealy_distance_redux(d.data_ptr(), m.data_ptr() if m is not None else None, b1 * b2, s1, s2,
+                                           N.dtype_code(d.dtype, allow_f64=True), op, min(karg, 1 << 30), sym, float(eps),
+                                           float(inf), out.data_ptr(), N.stream_ptr(d.device)))
+    return out
+
+
+class _ReduxFused(torch.autograd.Function):
+    """distance_tensor_redux on the fused path under autograd: d dist = g * w, the weights of the strategy's selection,
+    rerun by wealy_distance_redux_backward on the same block (for bpwr the jittered one, whose jitter has gradient 1)."""
+
+    @staticmethod
+    def forward(ctx, d, m, plan, eps, inf):
+        ctx.save_for_backward(d, m)
+        ctx.cfg = (plan, eps, inf)
+        return _redux_launch(d.detach(), m, plan, eps, inf)
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        d, m = ctx.saved_tensors
+        (op, karg, sym), eps, inf = ctx.cfg
+        b1, b2, s1, s2 = d.shape
+        dd = torch.empty_like(d, memory_format=torch.contiguous_format)
+        g = g.to(d.dtype).contiguous()
+        with torch.cuda.device(d.device):
+            N.check(N.lib.wealy_distance_redux_backward(
+                d.data_ptr(), m.data_ptr() if m is not None else None, b1 * b2, s1, s2,
+                N.dtype_code(d.dtype, allow_f64=True), op, min(karg, 1 << 30), sym, float(eps), float(inf), g.data_ptr(),
+                dd.data_ptr(), N.stream_ptr(d.device)))
+        return dd, None, None, None, None
+
+
 def _redux_fused(dist, plan, mask, eps, inf):
     """One launch of the fused kernel (csrc/redux_kernels.cuh) -> (b1, b2, 1, 1)."""
-    op, karg, sym = plan
     b1, b2, s1, s2 = dist.shape
-    if op == 7:                                         # bpwr: the reference's tie jitter (lib/tensor_ops.py:318)
+    if plan[0] == 7:                                    # bpwr: the reference's tie jitter (lib/tensor_ops.py:318)
         dist = dist + eps * torch.rand_like(dist)
     d = dist.contiguous()
     m = None
     if mask is not None:
         m = torch.broadcast_to(mask, dist.shape).contiguous().to(torch.uint8)
-    out = torch.empty((b1, b2), dtype=dist.dtype, device=dist.device)
-    with torch.cuda.device(dist.device):
-        N.check(N.lib.wealy_distance_redux(d.data_ptr(), m.data_ptr() if m is not None else None, b1 * b2, s1, s2,
-                                           N.dtype_code(dist.dtype, allow_f64=True), op, min(karg, 1 << 30), sym, float(eps),
-                                           float(inf), out.data_ptr(), N.stream_ptr(dist.device)))
+    if dist.requires_grad and torch.is_grad_enabled():
+        out = _ReduxFused.apply(d, m, plan, eps, inf)
+    else:
+        out = _redux_launch(d, m, plan, eps, inf)
     return out.view(b1, b2, 1, 1)
 
 

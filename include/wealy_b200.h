@@ -255,6 +255,14 @@ void wealy_eval_plan_destroy(wealy_eval_plan* plan);
 #define WEALY_MASKED_MAX 3
 int wealy_masked_reduce(const void* x, const uint8_t* mask, int64_t rows, int64_t cols, int dtype, int op, float fill,
                         float eps, void* out, void* stream);
+/* Gradient of wealy_masked_reduce: dx [rows, cols] (x's dtype) = g[row] * w, g [rows] in x's dtype, the same x / mask /
+ * op / fill / eps as the forward.  w: sum 1, mean 1 / max(count, eps) on included entries (0 on excluded ones); min / max
+ * with full == 0: 1 on the FIRST extreme of the filled row (a NaN is the extreme; 0 if that entry is excluded) -- order
+ * the columns so that the reference's tie (the last dim it reduces is the most significant) is the first; full != 0
+ * (dim=None, torch.min() of the whole tensor): 1 / t on every included entry equal to the extreme, t = the number of
+ * positions equal to it, excluded ones counted.                                                                    */
+int wealy_masked_reduce_backward(const void* x, const uint8_t* mask, int64_t rows, int64_t cols, int dtype, int op,
+                                 float fill, float eps, int full, const void* g, void* dx, void* stream);
 
 /* ---- a4: multi-chunk distance reduction -----------------------------------------------------
  * Replaces lib/tensor_ops.py:288-373 `distance_tensor_redux(dist, redux, mask, ...)`: dist [pairs, s1, s2] contiguous
@@ -273,6 +281,14 @@ int wealy_masked_reduce(const void* x, const uint8_t* mask, int64_t rows, int64_
 #define WEALY_RDX_BPWR 7
 int wealy_distance_redux(const void* dist, const uint8_t* mask, int64_t pairs, int s1, int s2, int dtype, int op, int karg,
                          int symmetric, float eps, float inf, void* out, void* stream);
+/* Gradient of wealy_distance_redux: ddist [pairs, s1, s2] (dist's dtype) = g[pair] * w, g [pairs] in dist's dtype, the
+ * same dist (for WEALY_RDX_BPWR the jittered one the forward saw) / mask / op / karg / symmetric / eps / inf.  The
+ * strategy's selection is rerun; w is what the reference's autograd gives (DESIGN.md section 1, row a4): min / max
+ * one-hot on the first extreme in row-major order, mean 1 / max(count, eps), minmean 1 / max(cnt_i, eps) on the first
+ * minimal row, meanmin cnt_i / max(C, eps) on every row's first argmin, best-k / bpwr 1 / max(c, eps) on the selected
+ * entries, worst-k 0; excluded entries 0; symmetric: the mean of the weights of the block and of its transpose.     */
+int wealy_distance_redux_backward(const void* dist, const uint8_t* mask, int64_t pairs, int s1, int s2, int dtype, int op,
+                                  int karg, int symmetric, float eps, float inf, const void* g, void* ddist, void* stream);
 
 /* ---- f3 / f4: the steps either side of the path (SURVEY.md section 8(f)) --------------------------
  * wealy_mean_pool: lib/layers.py:6-30 MeanPool.  x [b, c, t] contiguous, mask [b, t] bytes (non-zero = VALID) or

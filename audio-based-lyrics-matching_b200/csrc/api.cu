@@ -397,7 +397,7 @@ static void fill_shape(GemmShape& sh, int64_t m, int64_t n, int64_t d_pad, int b
   sh.n_col_tiles = (int)ceil_div(n, kTileN);
   // enough units for ~16 rounds of the persistent grid (tail quantisation < 4 %), but never more
   // chunks than column tiles; CTAs resident together sweep the same chunk (L2 reuse of candidates)
-  const int64_t target_units = (int64_t)num_sms() * env_int("WEALY_ROUNDS", 16);
+  const int64_t target_units = (int64_t)num_sms() * 16;
   int64_t chunks = ceil_div(target_units, sh.n_row_blocks > 0 ? sh.n_row_blocks : 1);
   // short units (a few column tiles) keep the CTAs that share candidate tiles within one unit of each other
   if (tiles_per_unit > 0 && chunks < ceil_div(sh.n_col_tiles, tiles_per_unit)) chunks = ceil_div(sh.n_col_tiles, tiles_per_unit);
@@ -409,8 +409,7 @@ static void fill_shape(GemmShape& sh, int64_t m, int64_t n, int64_t d_pad, int b
   sh.n_col_chunks = (int)ceil_div(sh.n_col_tiles, sh.tiles_per_chunk);
   if (sh.n_col_chunks < 1) sh.n_col_chunks = 1;
   // row blocks per scheduling group: the CTAs resident together cover group_rows row blocks x all chunks
-  int gr = env_int("WEALY_GROUP_ROWS", 0);
-  if (gr <= 0) gr = num_sms() / (sh.n_col_chunks < 4 ? sh.n_col_chunks : 4);  // ~4 chunks in flight per group
+  int gr = num_sms() / (sh.n_col_chunks < 4 ? sh.n_col_chunks : 4);  // ~4 chunks in flight per group
   if (gr < 1) gr = 1;
   if (gr > sh.n_row_blocks) gr = sh.n_row_blocks > 0 ? sh.n_row_blocks : 1;
   sh.group_rows = gr;
@@ -423,10 +422,13 @@ static void fill_shape(GemmShape& sh, int64_t m, int64_t n, int64_t d_pad, int b
   sh.skip0 = sh.skip1 = 0;
 }
 
-template <class Epi, int kPasses, int kBlockK, int kEpiWarps, int kMaxStages = 8>
+// column tiles per unit of the evaluation sweeps (4 and 16 measured the same at C2, within 0.1 ms)
+constexpr int kEvalTilesPerUnit = 8;
+
+template <class Epi, int kPasses, int kBlockK, int kEpiWarps>
 static int launch_gemm_t(const Planes& a, const Planes& b, const GemmShape& sh, const typename Epi::Params& ep,
                          cudaStream_t s) {
-  using SM = GemmSmem<kPasses, kBlockK, kMaxStages>;
+  using SM = GemmSmem<kPasses, kBlockK>;
   GemmTmaps maps;
   memset(&maps, 0, sizeof(maps));
   W_TRY(make_plane_tmap(&maps.a_hi, a.hi, a.rows, a.d_pad, kTileM, kBlockK));
@@ -438,7 +440,7 @@ static int launch_gemm_t(const Planes& a, const Planes& b, const GemmShape& sh, 
     maps.a_lo = maps.a_hi;
     maps.b_lo = maps.b_hi;
   }
-  auto kern = gemm_kernel<Epi, kPasses, kBlockK, kEpiWarps, kMaxStages>;
+  auto kern = gemm_kernel<Epi, kPasses, kBlockK, kEpiWarps>;
   constexpr int kSmemBytes = SM::total(kEpiWarps, Epi::kWarpScratchBytes, Epi::kCtaScratchBytes);
   static_assert(kSmemBytes <= 227 * 1024, "shared memory budget");
   CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
@@ -453,7 +455,7 @@ static int launch_gemm_t(const Planes& a, const Planes& b, const GemmShape& sh, 
 }
 
 // CTA-pair kernel (gemm_core2.cuh): sh.n_row_blocks / group_rows / rb_stride / rb_offset are in SUPER row blocks
-template <class Epi, int kPasses, int kBlockK, int kEpiWarps = 8, bool kDyn = false>
+template <class Epi, int kPasses, int kBlockK, int kEpiWarps = 8>
 static int launch_gemm_pair(const Planes& a, const GemmShape& sh, const typename Epi::Params& ep, cudaStream_t s,
                             const Planes* b_planes = nullptr, int max_pairs = 0) {
   constexpr int kStages = 4;
@@ -473,7 +475,7 @@ static int launch_gemm_pair(const Planes& a, const GemmShape& sh, const typename
     maps.a_lo = maps.a_hi;
     maps.b_lo = maps.b_hi;
   }
-  auto kern = gemm_pair_kernel<Epi, kPasses, kBlockK, kEpiWarps, kStages, kDyn>;
+  auto kern = gemm_pair_kernel<Epi, kPasses, kBlockK, kEpiWarps, kStages>;
   constexpr int kSmemBytes = SM::total(kEpiWarps, Epi::kWarpScratchBytes, Epi::kCtaScratchBytes);
   static_assert(kSmemBytes <= 227 * 1024, "shared memory budget");
   CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
@@ -491,7 +493,8 @@ static int launch_gemm_pair(const Planes& a, const GemmShape& sh, const typename
 
 // Rectangle sweeps (queries != corpus, streaming top-k, chunked tracks) on the CTA-pair core: 256 x 256 tiles per pair
 // of SMs, each SM loads its 128 query rows and half of the tile's candidate rows -- 2/3 of the L2 -> shared-memory
-// traffic of the single-CTA kernel, which is what bounds these sweeps (WEALY_RECT_PAIR=0 selects the single-CTA kernel).
+// traffic of the single-CTA kernel, which is what bounds these sweeps (DESIGN.md §4).  A single row block stays on the
+// single-CTA kernel.
 template <class Epi>
 static int launch_gemm_rect(int passes, const Planes& a, const Planes& b, GemmShape& sh, const typename Epi::Params& ep,
                             cudaStream_t s, int shard_rank = 0, int shard_world = 1);
@@ -522,7 +525,7 @@ static int launch_gemm(int passes, const Planes& a, const Planes& b, GemmShape& 
 template <class Epi>
 static int launch_gemm_rect(int passes, const Planes& a, const Planes& b, GemmShape& sh, const typename Epi::Params& ep,
                             cudaStream_t s, int shard_rank, int shard_world) {
-  if (env_int("WEALY_RECT_PAIR", 1) == 0 || sh.n_row_blocks < 2) {
+  if (sh.n_row_blocks < 2) {
     GemmShape shs = sh;
     shard_row_blocks(shs, shard_rank, shard_world);
     return launch_gemm<Epi>(passes, a, b, shs, ep, s);
@@ -534,9 +537,9 @@ static int launch_gemm_rect(int passes, const Planes& a, const Planes& b, GemmSh
   if (passes == 3) {
     if (a.lo == nullptr || b.lo == nullptr) return fail(WEALY_ERR_BAD_ARG, "3-pass contraction needs lo planes");
     shp.k_blocks = (int)(a.d_pad / 32);
-    return launch_gemm_pair<Epi, 3, 32, 8, false>(a, shp, ep, s, &b);
+    return launch_gemm_pair<Epi, 3, 32, 8>(a, shp, ep, s, &b);
   }
-  if (passes == 1) return launch_gemm_pair<Epi, 1, 64, 8, false>(a, shp, ep, s, &b);
+  if (passes == 1) return launch_gemm_pair<Epi, 1, 64, 8>(a, shp, ep, s, &b);
   return fail(WEALY_ERR_BAD_ARG, "passes must be 1 or 3, got %d", passes);
 }
 
@@ -1063,9 +1066,52 @@ static int launch_eval_tracks(int passes, const Planes& a, const Planes& b, Gemm
   shard_row_blocks(shp, shard_rank, shard_world);
   if (passes == 3) {
     shp.k_blocks = (int)(a.d_pad / 32);
-    return launch_gemm_pair<EvalTracksSymEpi<kS>, 3, 32, 8, false>(a, shp, ep, s);
+    return launch_gemm_pair<EvalTracksSymEpi<kS>, 3, 32, 8>(a, shp, ep, s);
   }
-  return launch_gemm_pair<EvalTracksSymEpi<kS>, 1, 64, 8, false>(a, shp, ep, s);
+  return launch_gemm_pair<EvalTracksSymEpi<kS>, 1, 64, 8>(a, shp, ep, s);
+}
+
+// EvalSymParams of a plan's symmetric sweep; `sh` is fill_shape's shape of all N rows (128-row blocks).  The top-k fields
+// stay zero.
+static EvalSymParams sym_params(const wealy_eval_plan* p, const GemmShape& sh) {
+  EvalSymParams sp;
+  memset(&sp, 0, sizeof(sp));
+  sp.lvl = p->s_lvl;
+  sp.cinfo = p->s_cinfo;
+  sp.s_c = p->sorted_c;
+  sp.s_i = p->s_i;
+  sp.thr = p->thr;
+  sp.hist = p->hist;
+  sp.dirty = p->s_dirty;
+  sp.n_col_tiles = sh.n_col_tiles;
+  sp.n_row_blocks = sh.n_row_blocks;
+  sp.total_pairs = (unsigned)p->total_pairs;
+  return sp;
+}
+
+// The symmetric all-vs-all sweep (EvalSymEpi on the CTA-pair core), for every run that takes it: plain, sharded, staged,
+// top-k and the parts of a host run.  `sh` is the launch shape in super row blocks of 256 rows, already restricted to the
+// caller's row blocks (shard, part); max_pairs > 0 caps the CTA pairs (SMs left to another resident kernel).
+static int launch_sym_sweep(int passes, bool topk, const Planes& pq, GemmShape sh, const EvalSymParams& sp, cudaStream_t s,
+                            int max_pairs = 0) {
+  // the two CTAs of a pair take the even / odd rows of the super row block, which splits the epilogue work of a clique
+  // evenly between the coupled epilogues (sh.sym bit 1)
+  sh.sym = 1 | 2;
+  if (passes == 3) sh.k_blocks = (int)(pq.d_pad / 32);
+  if (topk) {
+    // (8 epilogue warps: the top-k epilogue needs 160 registers per thread)
+    if (passes == 3) return launch_gemm_pair<EvalSymEpi<3, 256, 4096, true>, 3, 32, 8>(pq, sh, sp, s, nullptr, max_pairs);
+    return launch_gemm_pair<EvalSymEpi<3, 256, 4096, true>, 1, 64, 8>(pq, sh, sp, s, nullptr, max_pairs);
+  }
+  // the plain sweep measured best with about half as many super row blocks per scheduling group as there are CTA pairs
+  // -- 37 instead of 19 on 148 SMs: 431-443 against 422-436 Gpairs/s at C2 on two boxes (56 .. 74 row blocks the same
+  // within the noise, 18 and 296 clearly worse)
+  sh.group_rows = std::max(1, std::min(num_sms() / 4, sh.n_row_blocks));
+  // three epilogue warps per TMEM lane quadrant (the pair's epilogue is the co-limiter; 16 warps were measured worse).
+  // Dense threshold levels, 3 passes: 4 (C2: 23.45 ms per step against 23.2-23.4 with 3 -- the same --, MAP-0.1 data:
+  // 43.7 against 49.1 ms; 2 levels: 24.0-24.2 / 56.9 ms)
+  if (passes == 3) return launch_gemm_pair<EvalSymEpi<4>, 3, 32, 12>(pq, sh, sp, s, nullptr, max_pairs);
+  return launch_gemm_pair<EvalSymEpi<3>, 1, 64, 12>(pq, sh, sp, s, nullptr, max_pairs);
 }
 
 static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q, const void* candidates_z,
@@ -1134,7 +1180,7 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
   const bool sym_topk = can_sym && topk > 0 && topk <= 128 && nq >= env_int("WEALY_SYM_TOPK_MIN_ROWS", 16384) &&
                         nq >= 192ll * topk && (local || (finish && shard_world == 1)) &&
                         allow_sym_topk && env_int("WEALY_SYM_TOPK", 1) != 0;
-  const bool sym = can_sym && (topk == 0 ? (shard_world > 1 || env_int("WEALY_SYM", 1) != 0) : sym_topk);
+  const bool sym = can_sym && (topk == 0 || sym_topk);
   // chunked tracks, all-vs-all: the same halving for reductions that give d(q, c) == d(c, q) (min / max / mean)
   const bool all_tracks = same && p->same_ids && chunks > 1 && topk == 0;
   const bool sym_tracks = all_tracks && red_inner == red_outer && nq * chunks > 2 * kTileM && env_int("WEALY_SYM_TRACKS", 1) != 0;
@@ -1209,7 +1255,7 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
         pos_thresholds_tracks_kernel<<<(unsigned)(q_hi - q_lo), threads, 0, s>>>(
             pq.hi, pq.lo, pc.hi, pc.lo, (int)pq.d_pad, chunks, red_inner, red_outer, red_scale, p->q_i, (int)nq, p->sorted_idx,
             p->c_i, p->seg_lo, p->seg_len, p->off, p->raw, p->thr, p->lim, p->cnt, q_len, c_len, q_lo);
-    } else if (same && p->same_ids && nq > 0 && env_int("WEALY_KPOS_BLOCKS", 1) != 0) {
+    } else if (same && p->same_ids && nq > 0) {
       // all-vs-all through the rectangle sweep (top-k requested): the clique-block tensor-core K_pos of the symmetric
       // path on the caller's row order (every unordered pair's operands are read once per 16 x 8 block, not per pair)
       CU_TRY(cudaMemsetAsync(p->cnt, 0, (size_t)nq * 4, s));
@@ -1309,7 +1355,7 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
   GemmShape sh;
   // top-k keeps <= 4 candidate lists per query (column chunks x epilogue warps per row)
   const bool rect_topk = topk > 0 && !sym_topk;
-  fill_shape(sh, rq, rc, pq.d_pad, 64, rect_topk ? (4 / halves) : (1 << 20), rect_topk ? 0 : env_int("WEALY_TILES_PER_UNIT", 8));
+  fill_shape(sh, rq, rc, pq.d_pad, 64, rect_topk ? (4 / halves) : (1 << 20), rect_topk ? 0 : kEvalTilesPerUnit);
   const int parts = sh.n_col_chunks * halves;
   const int cap = rect_topk ? topk_capacity(topk) : 0;
 
@@ -1347,91 +1393,18 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
     CU_TRY(cudaMemsetAsync(ep.cand_cnt, 0, (size_t)parts * nq * 4, s));
   }
   CU_TRY(cudaEventRecord(p->ev0, s));
-  // CTA-pair (cta_group::2) kernel: the default for the symmetric sweep (half the B-operand shared-memory traffic;
-  // WEALY_SYM_PAIR=0 selects the single-CTA kernel)
-  const bool pair = sym && env_int("WEALY_SYM_PAIR", 1) != 0;
-  const int total_rb = sh.n_row_blocks;
-  if (pair) {
-    // the pair kernel works on super row blocks (two adjacent row blocks per CTA pair)
-    sh.n_row_blocks = (total_rb + 1) / 2;
-    sh.group_rows = (sh.group_rows + 1) / 2;
-    // the plain (no top-k) sweep measured best with about half as many super row blocks per scheduling group as there
-    // are CTA pairs -- 37 instead of 19 on 148 SMs: 431-443 against 422-436 Gpairs/s at C2 on two boxes (56 .. 74 row
-    // blocks the same within the noise, 18 and 296 clearly worse)
-    if (!sym_topk && env_int("WEALY_GROUP_ROWS", 0) <= 0) {
-      sh.group_rows = std::max(1, num_sms() / 4);
-      if (sh.group_rows > sh.n_row_blocks) sh.group_rows = std::max(1, sh.n_row_blocks);
-    }
-  }
-  // (chunked tracks: launch_eval_tracks shards the shape it launches, after halving it into super row blocks)
-  if (sym) shard_row_blocks(sh, shard_rank, shard_world);
   if (sym) {
-    sh.sym = 1;
-    EvalSymParams sp;
-    memset(&sp, 0, sizeof(sp));
-    sp.lvl = p->s_lvl;
-    sp.cinfo = p->s_cinfo;
-    sp.s_c = p->sorted_c;
-    sp.s_i = p->s_i;
-    sp.thr = p->thr;
-    sp.hist = p->hist;
-    sp.dirty = p->s_dirty;
-    sp.n_col_tiles = sh.n_col_tiles;
-    sp.n_row_blocks = total_rb;
-    sp.total_pairs = (unsigned)p->total_pairs;
+    EvalSymParams sp = sym_params(p, sh);
     sp.beta = tk_beta;
     sp.tk_val = tk_val;
     sp.tk_idx = tk_idx;
     sp.tk_cnt = tk_cnt;
     sp.tk_cap = tk_cap2;
-    const int lv = env_int("WEALY_SYM_LEVELS", 3);  // 3 measured best at C2 (2: 26.8 ms, 3: 25.5 ms, 4: 25.9 ms per step)
-    if (sym_topk && pair) {
-      // (8 epilogue warps: the top-k epilogue needs 160 registers per thread)
-      if (env_int("WEALY_PAIR_INTERLEAVE", 1) != 0) sh.sym |= 2;
-      if (passes == 3) {
-        sh.k_blocks = (int)(pq.d_pad / 32);
-        W_TRY((launch_gemm_pair<EvalSymEpi<3, 256, 4096, true>, 3, 32, 8, true>(pq, sh, sp, s)));
-      } else {
-        W_TRY((launch_gemm_pair<EvalSymEpi<3, 256, 4096, true>, 1, 64, 8, true>(pq, sh, sp, s)));
-      }
-    } else if (sym_topk) {
-      if (passes == 3) {
-        sh.k_blocks = (int)(pq.d_pad / 32);
-        W_TRY((launch_gemm_t<EvalSymEpi<3, 256, 4096, true>, 3, 32, 8, 3>(pq, pc, sh, sp, s)));
-      } else {
-        W_TRY((launch_gemm_t<EvalSymEpi<3, 256, 4096, true>, 1, 64, 8, 3>(pq, pc, sh, sp, s)));
-      }
-    } else if (pair) {
-      if (env_int("WEALY_PAIR_INTERLEAVE", 1) != 0) sh.sym |= 2;
-      // three epilogue warps per TMEM lane quadrant (the pair's epilogue is the co-limiter; 16 warps were measured worse);
-      // WEALY_PAIR_DYN: the warps of a quadrant claim 32-column chunks dynamically instead of owning fixed ones
-      const bool w12 = env_int("WEALY_PAIR_EPI_WARPS", 12) == 12;
-      const bool dyn = env_int("WEALY_PAIR_DYN", 1) != 0;
-      if (passes == 3) {
-        sh.k_blocks = (int)(pq.d_pad / 32);
-        // dense threshold levels on the pair core: 4 (C2: 23.45 ms per step against 23.2-23.4 with 3 -- the same --, MAP-0.1
-        // data: 43.7 against 49.1 ms; 2 levels: 24.0-24.2 / 56.9 ms)
-        const int lvp = env_int("WEALY_SYM_LEVELS", 4);
-        if (dyn && w12 && lvp == 2) W_TRY((launch_gemm_pair<EvalSymEpi<2>, 3, 32, 12, true>(pq, sh, sp, s)));
-        else if (dyn && w12 && lvp == 4) W_TRY((launch_gemm_pair<EvalSymEpi<4>, 3, 32, 12, true>(pq, sh, sp, s)));
-        else if (dyn && w12) W_TRY((launch_gemm_pair<EvalSymEpi<3>, 3, 32, 12, true>(pq, sh, sp, s)));
-        else if (dyn) W_TRY((launch_gemm_pair<EvalSymEpi<3>, 3, 32, 8, true>(pq, sh, sp, s)));
-        else if (w12) W_TRY((launch_gemm_pair<EvalSymEpi<3>, 3, 32, 12>(pq, sh, sp, s)));
-        else W_TRY((launch_gemm_pair<EvalSymEpi<3>, 3, 32>(pq, sh, sp, s)));
-      } else {
-        if (dyn && w12) W_TRY((launch_gemm_pair<EvalSymEpi<3>, 1, 64, 12, true>(pq, sh, sp, s)));
-        else if (dyn) W_TRY((launch_gemm_pair<EvalSymEpi<3>, 1, 64, 8, true>(pq, sh, sp, s)));
-        else if (w12) W_TRY((launch_gemm_pair<EvalSymEpi<3>, 1, 64, 12>(pq, sh, sp, s)));
-        else W_TRY((launch_gemm_pair<EvalSymEpi<3>, 1, 64>(pq, sh, sp, s)));
-      }
-    } else if (passes == 3) {
-      sh.k_blocks = (int)(pq.d_pad / 32);
-      if (lv == 2) W_TRY((launch_gemm_t<EvalSymEpi<2>, 3, 32, 8, 3>(pq, pc, sh, sp, s)));
-      else if (lv == 4) W_TRY((launch_gemm_t<EvalSymEpi<4>, 3, 32, 8, 3>(pq, pc, sh, sp, s)));
-      else W_TRY((launch_gemm_t<EvalSymEpi<3>, 3, 32, 8, 3>(pq, pc, sh, sp, s)));
-    } else {
-      W_TRY((launch_gemm_t<EvalSymEpi<3>, 1, 64, 8, 3>(pq, pc, sh, sp, s)));
-    }
+    // the CTA-pair kernel works on super row blocks (two adjacent row blocks per CTA pair)
+    sh.n_row_blocks = (sh.n_row_blocks + 1) / 2;
+    sh.group_rows = (sh.group_rows + 1) / 2;
+    shard_row_blocks(sh, shard_rank, shard_world);
+    W_TRY(launch_sym_sweep(passes, sym_topk, pq, sh, sp, s));
   } else if (chunks == 2) {
     W_TRY(launch_eval_tracks<2>(passes, pq, pc, sh, ep, s, sym_tracks, shard_rank, shard_world));
   } else if (chunks == 4) {
@@ -1550,11 +1523,6 @@ static cudaStream_t upload_stream() {
   std::lock_guard<std::mutex> lock(mu);
   if (!streams[dev] && cudaStreamCreateWithFlags(&streams[dev], cudaStreamNonBlocking) != cudaSuccess) streams[dev] = nullptr;
   return streams[dev];
-}
-
-template <int kLevels, int kPasses, int kBlockK>
-static int launch_sym_part(const Planes& pq, const GemmShape& sh, const EvalSymParams& sp, cudaStream_t s, int max_pairs) {
-  return launch_gemm_pair<EvalSymEpi<kLevels>, kPasses, kBlockK, 12, true>(pq, sh, sp, s, nullptr, max_pairs);
 }
 
 // The upload kernel and where it runs.  By default on U = 8 SMs of its own (WEALY_HOST_UP_SMS): CTAs of 512 threads whose
@@ -1789,22 +1757,8 @@ extern "C" int wealy_eval_run_host(wealy_eval_plan* p, const void* host_z, int64
   const int64_t reach = p->max_clique > 1 ? p->max_clique : 1;  // K_pos of a query reads the rows of its whole clique
 
   GemmShape sh0;
-  fill_shape(sh0, n, n, pq.d_pad, 64, 1 << 20, env_int("WEALY_TILES_PER_UNIT", 8));
-  const int total_rb = sh0.n_row_blocks;
-  sh0.sym = 1 | (env_int("WEALY_PAIR_INTERLEAVE", 1) != 0 ? 2 : 0);
-  if (passes == 3) sh0.k_blocks = (int)(pq.d_pad / 32);
-  EvalSymParams sp;
-  memset(&sp, 0, sizeof(sp));
-  sp.lvl = p->s_lvl;
-  sp.cinfo = p->s_cinfo;
-  sp.s_c = p->sorted_c;
-  sp.s_i = p->s_i;
-  sp.thr = p->thr;
-  sp.hist = p->hist;
-  sp.dirty = p->s_dirty;
-  sp.n_col_tiles = sh0.n_col_tiles;
-  sp.n_row_blocks = total_rb;
-  sp.total_pairs = (unsigned)p->total_pairs;
+  fill_shape(sh0, n, n, pq.d_pad, 64, 1 << 20, kEvalTilesPerUnit);
+  const EvalSymParams sp = sym_params(p, sh0);
 
   CU_TRY(cudaEventRecord(p->evs[0], s));
   CU_TRY(cudaEventRecord(p->evs[1], s));
@@ -1862,10 +1816,8 @@ extern "C" int wealy_eval_run_host(wealy_eval_plan* p, const void* host_z, int64
       sh.n_row_blocks = sb_hi - sb_lo;
       sh.rb_offset = sb_lo;
       sh.rb_stride = 1;
-      sh.group_rows = std::max(1, std::min(num_sms() / 4, sh.n_row_blocks));
       const int max_pairs = (up_sms > 0 && k + 1 < n_parts) ? (num_sms() - up_sms) / 2 : 0;
-      if (passes == 3) W_TRY((launch_sym_part<4, 3, 32>(pq, sh, sp, s, max_pairs)));
-      else W_TRY((launch_sym_part<3, 1, 64>(pq, sh, sp, s, max_pairs)));
+      W_TRY(launch_sym_sweep(passes, false, pq, sh, sp, s, max_pairs));
     }
     else stamp(s);
     stamp(s);

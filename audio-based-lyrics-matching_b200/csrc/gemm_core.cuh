@@ -55,7 +55,8 @@ struct GemmShape {
   int* unit_counter;    // global work counter of this launch: dynamic unit scheduling.  unit_counter[1] counts the
                         //   CTAs that are through; the last one zeroes both again, so the host never has to (no memset
                         //   in front of every launch; the slots start out zero)
-  int sym;              // symmetric all-vs-all: only tiles that reach above the diagonal are computed
+  int sym;              // CTA-pair core (gemm_core2.cuh) only -- bit 0: symmetric all-vs-all, only tiles that reach
+                        //   above the diagonal are computed; bit 1: the pair's CTAs take alternate rows
   int rb_stride;        // multi-GPU symmetric sweep: this launch owns row blocks rb_offset + k * rb_stride
   int rb_offset;        //   (n_row_blocks counts the owned ones)
   // column-tile window of this launch: only tiles in [win0, win1) and outside [skip0, skip1) are contracted (the
@@ -66,13 +67,6 @@ struct GemmShape {
 
 __device__ __forceinline__ bool tile_selected(const GemmShape& sh, int t) {
   return t >= sh.win0 && t < sh.win1 && !(t >= sh.skip0 && t < sh.skip1);
-}
-
-// First column tile a row block needs in symmetric mode: tile t holds columns [256 t, 256 t + 256) and row
-// block rb rows [128 rb, 128 rb + 128); it contains an element with col > row iff t >= rb / 2.
-__device__ __forceinline__ int first_tile(const GemmShape& sh, int rb, int t0) {
-  static_assert(kTileN == 2 * kTileM, "symmetric tile range assumes 256-wide column tiles over 128-row blocks");
-  return sh.sym ? max(t0, rb >> 1) : t0;
 }
 
 // Unit order.  Units are handed out in sequence from a global atomic counter (the TMA warp fetches the
@@ -104,7 +98,7 @@ __device__ __forceinline__ void release_unit_counter(const GemmShape& sh) {
   }
 }
 
-template <int kPasses, int kBlockK, int kMaxStages = 8>
+template <int kPasses, int kBlockK>
 struct GemmSmem {
   static constexpr int kSwizzle = kBlockK * 2;  // bytes per smem row == swizzle span
   static constexpr int kABytes = kTileM * kBlockK * 2;
@@ -112,6 +106,7 @@ struct GemmSmem {
   static constexpr int kPlanes = kPasses == 3 ? 2 : 1;
   static constexpr int kStageBytes = kPlanes * (kABytes + kBBytes);
   static constexpr int kBudget = 227 * 1024 - 2048 - 30 * 1024;  // alignment slack + barriers + epilogue scratch
+  static constexpr int kMaxStages = 8;
   static constexpr int kStages = (kBudget / kStageBytes) > kMaxStages ? kMaxStages : (kBudget / kStageBytes);
   static constexpr int kBarBytes = 512;
   static constexpr int kCore = kStages * kStageBytes + kBarBytes;  // + per-warp epilogue scratch + 1024 align slack
@@ -159,10 +154,10 @@ struct ColSlotTraits<Epi, decltype((void)Epi::kColSlots)> {
 // `row` is the global query row owned by the thread, `part` identifies the partial result slot
 // (column chunk x epilogue half) when a row is split over several units / warps.
 
-template <class Epi, int kPasses, int kBlockK, int kEpiWarps, int kMaxStages = 8>
+template <class Epi, int kPasses, int kBlockK, int kEpiWarps>
 __global__ void __launch_bounds__(64 + kEpiWarps * 32, 1)
 gemm_kernel(const __grid_constant__ GemmTmaps tmaps, const GemmShape shape, const typename Epi::Params ep) {
-  using SM = GemmSmem<kPasses, kBlockK, kMaxStages>;
+  using SM = GemmSmem<kPasses, kBlockK>;
   constexpr int kStages = SM::kStages;
   constexpr int kHalves = kEpiWarps / 4;  // epilogue warps per TMEM lane quadrant
   static_assert(kEpiWarps == 4 || kEpiWarps == 8 || kEpiWarps == 12 || kEpiWarps == 16, "4, 8, 12 or 16 epilogue warps");
@@ -242,7 +237,7 @@ gemm_kernel(const __grid_constant__ GemmTmaps tmaps, const GemmShape shape, cons
         int chunk, rb;
         decode_unit(shape, u, chunk, rb);
         const int t1 = min((chunk + 1) * shape.tiles_per_chunk, shape.n_col_tiles);
-        const int t0 = first_tile(shape, rb, chunk * shape.tiles_per_chunk);
+        const int t0 = chunk * shape.tiles_per_chunk;
         for (int t = t0; t < t1; ++t) {
           if (!tile_selected(shape, t)) continue;
           if constexpr (kColSlots > 0) {
@@ -296,7 +291,7 @@ gemm_kernel(const __grid_constant__ GemmTmaps tmaps, const GemmShape shape, cons
         int chunk, rb;
         decode_unit(shape, u, chunk, rb);
         const int t1 = min((chunk + 1) * shape.tiles_per_chunk, shape.n_col_tiles);
-        const int t0 = first_tile(shape, rb, chunk * shape.tiles_per_chunk);
+        const int t0 = chunk * shape.tiles_per_chunk;
         for (int t = t0; t < t1; ++t) {
           if (!tile_selected(shape, t)) continue;
           ptx::mbar_wait(&tmem_empty[acc], acc_phase ^ 1u);  // epilogue has drained this accumulator
@@ -349,8 +344,7 @@ gemm_kernel(const __grid_constant__ GemmTmaps tmaps, const GemmShape shape, cons
       int chunk, rb;
       decode_unit(shape, u, chunk, rb);
       const int t1 = min((chunk + 1) * shape.tiles_per_chunk, shape.n_col_tiles);
-      const int t0 = first_tile(shape, rb, chunk * shape.tiles_per_chunk);
-      if (t0 >= t1) continue;  // symmetric mode: the whole unit lies below the diagonal
+      const int t0 = chunk * shape.tiles_per_chunk;
       const int row = rb * kTileM + row_in_tile;
       const int part = chunk * kHalves + half;
       typename Epi::RowState rs;

@@ -15,12 +15,13 @@
 //     barriers of both CTAs, the epilogue warps of both CTAs arrive on the leader's `tmem_empty`;
 //   * units are (super row block) x (chunk of column tiles), handed out dynamically by the leader's TMA thread,
 //     which publishes the unit index into the mailboxes of both CTAs (st.shared::cluster + remote mbarrier arrive);
-//   * kDynChunks: the epilogue warps of a TMEM lane quadrant do not own fixed 32-column chunks of a tile; they CLAIM
-//     the chunks of the unit's tiles one by one from a shared-memory counter (chunk stream g -> tile g / 8, chunk
-//     g % 8).  The rows of a quadrant are the same for all its warps, so any of them can score any chunk; a warp
-//     held up by a hot chunk (deep queue, dirty tile) simply claims fewer, and a fast one runs ahead into the next
-//     tile as soon as its accumulator is ready.  The accumulator hand-over then waits for the SUM of the warps'
-//     work, not for the slowest warp of 2 x kEpiWarps: every chunk arrives on `tmem_empty` on its own.
+//   * kDynChunks (every epilogue with per-tile column slots, i.e. the symmetric evaluation's EvalSymEpi): the epilogue
+//     warps of a TMEM lane quadrant do not own fixed 32-column chunks of a tile; they CLAIM the chunks of the unit's
+//     tiles one by one from a shared-memory counter (chunk stream g -> tile g / 8, chunk g % 8).  The rows of a
+//     quadrant are the same for all its warps, so any of them can score any chunk; a warp held up by a hot chunk
+//     (deep queue, dirty tile) simply claims fewer, and a fast one runs ahead into the next tile as soon as its
+//     accumulator is ready.  The accumulator hand-over then waits for the SUM of the warps' work, not for the
+//     slowest warp of 2 x kEpiWarps: every chunk arrives on `tmem_empty` on its own.
 #pragma once
 #include "gemm_core.cuh"
 
@@ -39,20 +40,16 @@ struct PairSmem {
   }
 };
 
-template <class Epi, int kPasses, int kBlockK, int kEpiWarps, int kStages, bool kDynChunks = false>
+template <class Epi, int kPasses, int kBlockK, int kEpiWarps, int kStages>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(64 + kEpiWarps * 32, 1)
 gemm_pair_kernel(const __grid_constant__ GemmTmaps tmaps, const GemmShape shape, const typename Epi::Params ep) {
   using SM = PairSmem<kPasses, kBlockK, kStages>;
   using CS = ColSlotTraits<Epi>;
   constexpr int kHalves = kEpiWarps / 4;
   constexpr int kColSlots = CS::kSlots;
-#ifdef WEALY_LATE_RELEASE
-  constexpr bool kEarlyRelease = false;  // (A/B builds: release the accumulator after the chunk has been scored)
-#else
-  constexpr bool kEarlyRelease = true;
-#endif
+  constexpr bool kDynChunks = kColSlots > 0;  // dynamic chunk claiming; the other epilogues own fixed chunks
   static_assert(kEpiWarps == 8 || kEpiWarps == 12, "8 or 12 epilogue warps (2 or 3 per TMEM lane quadrant)");
-  static_assert(kColSlots > 0 || !kDynChunks, "dynamic chunk claiming belongs to the symmetric evaluation epilogue");
+  static_assert(kTileN == 2 * kTileM, "symmetric tile range assumes 256-wide column tiles over 256-row super blocks");
 
   extern __shared__ uint8_t smem_raw[];
   // (the dynamic shared memory of both CTAs starts at the same offset, so the aligned layouts coincide)
@@ -98,7 +95,7 @@ gemm_pair_kernel(const __grid_constant__ GemmTmaps tmaps, const GemmShape shape,
     }
     for (int c = 0; c < kColSlots; ++c) {
       ptx::mbar_init(&col_full[c], 1);
-      ptx::mbar_init(&col_empty[c], kDynChunks ? 4 * kChunksPerTile : kEpiWarps);
+      ptx::mbar_init(&col_empty[c], 4 * kChunksPerTile);  // per claimed chunk
     }
     for (int k = 0; k < 8; ++k) chunk_ctr[k] = 0;
     ptx::fence_mbar_init();
@@ -267,8 +264,6 @@ gemm_pair_kernel(const __grid_constant__ GemmTmaps tmaps, const GemmShape shape,
     uint32_t acc_phase = 0;
     int us = 0;
     uint32_t uphase = 0;
-    int cs = 0;
-    uint32_t cphase = 0;
     const uint32_t leader_unit_empty0 = ptx::map_to_cta(&unit_empty[0], 0);
     const uint32_t leader_tmem_empty0 = ptx::map_to_cta(&tmem_empty[0], 0);
     unsigned tile_seq = 0;  // kDynChunks: tiles this CTA has been through (every role counts the same)
@@ -340,22 +335,15 @@ gemm_pair_kernel(const __grid_constant__ GemmTmaps tmaps, const GemmShape shape,
           // chunk (queue drain, dirty tile) never holds up the tensor pipe; only the column slot stays in use
           ptx::tc_fence_before_sync();
           __syncwarp();
-          if (kEarlyRelease && lane == 0) ptx::mbar_arrive_cluster_relaxed(leader_tmem_empty0 + 8u * a_cur);
+          if (lane == 0) ptx::mbar_arrive_cluster_relaxed(leader_tmem_empty0 + 8u * a_cur);
           Epi::chunk32(ep, rs, row, (t0 + tile) * kTileN + c * kChunkCols, v, shape, ctx);
           __syncwarp();
-          if (lane == 0) {
-            if (!kEarlyRelease) ptx::mbar_arrive_cluster_relaxed(leader_tmem_empty0 + 8u * a_cur);
-            ptx::mbar_arrive(&col_empty[c_cur]);
-          }
+          if (lane == 0) ptx::mbar_arrive(&col_empty[c_cur]);
         }
         if (cur >= 0) Epi::tile_end(ep, rs, shape, ctx);
         tile_seq += (unsigned)n_tiles;
       } else {
       for (int t = t0; t < t1; ++t) {
-        if constexpr (kColSlots > 0) {
-          ptx::mbar_wait_warp(&col_full[cs], cphase);
-          ctx.col_slot = col_slots + cs * CS::kBytes;
-        }
         Epi::tile_begin(ep, rs, shape, ctx, t);
         ptx::mbar_wait_cluster_warp(&tmem_full[acc], acc_phase);
         ptx::tc_fence_after_sync();
@@ -369,14 +357,8 @@ gemm_pair_kernel(const __grid_constant__ GemmTmaps tmaps, const GemmShape shape,
         }
         ptx::tc_fence_before_sync();
         __syncwarp();
-        if (lane == 0) {
-          ptx::mbar_arrive_cluster_relaxed(leader_tmem_empty0 + 8u * acc);
-          if constexpr (kColSlots > 0) ptx::mbar_arrive(&col_empty[cs]);
-        }
+        if (lane == 0) ptx::mbar_arrive_cluster_relaxed(leader_tmem_empty0 + 8u * acc);
         if (++acc == 2) { acc = 0; acc_phase ^= 1u; }
-        if constexpr (kColSlots > 0) {
-          if (++cs == kColSlots) { cs = 0; cphase ^= 1u; }
-        }
         Epi::tile_end(ep, rs, shape, ctx);
       }
       }

@@ -45,17 +45,10 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
 // Waiting warps burn issue slots and power that the tensor pipe could use (the sweeps run at the power cap): the
 // poll carries a suspend-time hint (the hardware parks the thread until the phase completes or the hint expires) and
 // a waiting WARP polls with one lane only (mbar_wait_warp).  Measured on the MMA-bound symmetric sweep: 1-2 %.
-#ifndef WEALY_WAIT_HINT_NS
-#define WEALY_WAIT_HINT_NS 1000
-#endif
-#ifndef WEALY_WAIT_ALL_LANES
-#define WEALY_WAIT_LANE0
-#endif
+constexpr uint32_t kWaitHintNs = 1000;
 
 __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
   uint32_t ok;
-#if WEALY_WAIT_HINT_NS > 0
-  // suspend-time hint: the hardware parks the thread until the phase completes or the hint expires
   asm volatile(
       "{\n"
       ".reg .pred P;\n"
@@ -63,19 +56,8 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
       "selp.u32 %0, 1, 0, P;\n"
       "}\n"
       : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)WEALY_WAIT_HINT_NS)
+      : "r"(smem_u32(bar)), "r"(parity), "r"(kWaitHintNs)
       : "memory");
-#else
-  asm volatile(
-      "{\n"
-      ".reg .pred P;\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 P, [%1], %2;\n"
-      "selp.u32 %0, 1, 0, P;\n"
-      "}\n"
-      : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-#endif
   return ok != 0;
 }
 
@@ -114,12 +96,8 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 
 // The same for a whole warp: one lane polls, the others wait at the warp barrier (32x fewer polling lanes)
 __device__ __forceinline__ void mbar_wait_warp(uint64_t* bar, uint32_t parity) {
-#ifdef WEALY_WAIT_LANE0
   if (lane_id() == 0) mbar_wait(bar, parity);
   __syncwarp();
-#else
-  mbar_wait(bar, parity);
-#endif
 }
 
 // barrier among a subset of the CTA's warps (id 0 is __syncthreads)
@@ -264,7 +242,7 @@ __device__ __forceinline__ bool mbar_try_wait_cluster(uint64_t* bar, uint32_t pa
       "selp.u32 %0, 1, 0, P;\n"
       "}\n"
       : "=r"(ok)
-      : "r"(smem_u32(bar)), "r"(parity), "r"((uint32_t)(WEALY_WAIT_HINT_NS > 0 ? WEALY_WAIT_HINT_NS : 1))
+      : "r"(smem_u32(bar)), "r"(parity), "r"(kWaitHintNs)
       : "memory");
   return ok != 0;
 }

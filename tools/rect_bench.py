@@ -1,5 +1,5 @@
 """Timing of the rectangle sweeps (everything that is not the symmetric all-vs-all sweep): queries != corpus, chunked
-tracks, all-vs-all top-k forced onto the streaming path.  Prints one JSON line; WEALY_RECT_PAIR=0/1 selects the core."""
+tracks, all-vs-all top-k forced onto the streaming path.  Prints one JSON line."""
 import json
 import os
 import sys
@@ -26,7 +26,7 @@ def timed(fn, warm=2, reps=4):
 
 
 def main():
-    out = {"core": "pair" if os.environ.get("WEALY_RECT_PAIR", "1") != "0" else "single"}
+    out = {}
     s = synth.make_eval_set(200_000, 1024, seed=0, device="cuda", md5_ids=False)
     q, c = slice(0, 100_000), slice(100_000, 200_000)
     keep = torch.isin(s["c"][q], s["c"][c])               # queries with a relevant item in the corpus half

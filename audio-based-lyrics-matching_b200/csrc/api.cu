@@ -870,7 +870,7 @@ using WideCounts = cub::TransformInputIterator<long long, WidenI32, const int*>;
 
 static int plan_build(wealy_eval_plan* p, const int64_t* queries_c, const int64_t* queries_i,
                       const int64_t* candidates_c, const int64_t* candidates_i, cudaStream_t s,
-                      const std::function<int()>& after_sort = nullptr) {
+                      const std::function<int(wealy_eval_plan*)>& after_sort = nullptr) {
   const int nq = (int)p->nq, nc = (int)p->nc;
   const int T = 256;
   TempAllocs tmps(s);
@@ -917,7 +917,7 @@ static int plan_build(wealy_eval_plan* p, const int64_t* queries_c, const int64_
   CU_TRY(cub::DeviceRadixSort::SortPairs(tmp, tmp_bytes, p->c_c, p->sorted_c, iota, p->sorted_idx, nc, 0, 32, s));
   // (wealy_eval_plan_create_host: the sorted order is all the upload of the first rows needs -- it starts here, under
   // the rest of the plan)
-  if (after_sort && p->same_ids) W_TRY(after_sort());
+  if (after_sort && p->same_ids) W_TRY(after_sort(p));
 
   CU_TRY(dev_alloc((void**)&p->seg_lo, (size_t)nq * 4 + 4, s));
   CU_TRY(dev_alloc((void**)&p->seg_len, (size_t)nq * 4 + 4, s));
@@ -1000,9 +1000,9 @@ static int plan_build(wealy_eval_plan* p, const int64_t* queries_c, const int64_
   return WEALY_OK;
 }
 
-extern "C" int wealy_eval_plan_create(const int64_t* queries_c, const int64_t* queries_i, int64_t nq,
-                                      const int64_t* candidates_c, const int64_t* candidates_i, int64_t nc,
-                                      void* stream, wealy_eval_plan** plan) {
+static int plan_create(const int64_t* queries_c, const int64_t* queries_i, int64_t nq, const int64_t* candidates_c,
+                       const int64_t* candidates_i, int64_t nc, cudaStream_t s, wealy_eval_plan** plan,
+                       const std::function<int(wealy_eval_plan*)>& after_sort = nullptr) {
   if (!plan) return fail(WEALY_ERR_BAD_ARG, "plan output pointer is null");
   *plan = nullptr;
   if (nq <= 0 || nc <= 0) return fail(WEALY_ERR_BAD_ARG, "empty query or candidate set (nq=%lld nc=%lld)", (long long)nq, (long long)nc);
@@ -1011,14 +1011,20 @@ extern "C" int wealy_eval_plan_create(const int64_t* queries_c, const int64_t* q
   wealy_eval_plan* p = new wealy_eval_plan();
   p->nq = nq;
   p->nc = nc;
-  p->stream = (cudaStream_t)stream;
-  int st = plan_build(p, queries_c, queries_i, candidates_c, candidates_i, (cudaStream_t)stream);
+  p->stream = s;
+  int st = plan_build(p, queries_c, queries_i, candidates_c, candidates_i, s, after_sort);
   if (st != WEALY_OK) {
     wealy_eval_plan_destroy(p);
     return st;
   }
   *plan = p;
   return WEALY_OK;
+}
+
+extern "C" int wealy_eval_plan_create(const int64_t* queries_c, const int64_t* queries_i, int64_t nq,
+                                      const int64_t* candidates_c, const int64_t* candidates_i, int64_t nc,
+                                      void* stream, wealy_eval_plan** plan) {
+  return plan_create(queries_c, queries_i, nq, candidates_c, candidates_i, nc, (cudaStream_t)stream, plan);
 }
 
 extern "C" int wealy_eval_plan_info(const wealy_eval_plan* p, int64_t* total_pairs, int64_t* queries_without_relevant,
@@ -1114,250 +1120,338 @@ static int launch_sym_sweep(int passes, bool topk, const Planes& pq, GemmShape s
   return launch_gemm_pair<EvalSymEpi<3>, 1, 64, 12>(pq, sh, sp, s, nullptr, max_pairs);
 }
 
-static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q, const void* candidates_z,
-                         int64_t ld_c, int64_t d, int dtype, float eps, int passes, int topk, float* aps,
-                         float* r1s, double* sums, int64_t* topk_idx, float* topk_sim, int shard_rank,
-                         int shard_world, bool finish, void* stream, int chunks = 1, int redux = WEALY_REDUX_MIN,
-                         const int* q_len = nullptr, const int* c_len = nullptr, bool allow_sym_topk = true, int stage = 0,
-                         int* local_idx = nullptr, int* local_cnt = nullptr) {
-  // stage (sharded all-vs-all sweeps only): 0 = everything in one call; 1 = prep + the relevant similarities of THIS
-  // rank's share of the queries, then return (the caller sums the threshold buffer over the ranks); 2 = the sweep,
-  // on the planes and thresholds stage 1 left in the plan
-  // local_cnt != NULL (wealy_eval_sweep_shard_topk): the symmetric top-k sweep over this rank's row blocks, its lists
-  // finalized locally into topk_sim / local_idx / local_cnt; the rank counters stay in the plan (finish == false)
-  const bool local = local_cnt != nullptr;
-  cudaStream_t s = (cudaStream_t)stream;
-  if (!p) return fail(WEALY_ERR_BAD_ARG, "null plan");
-  if (p->early_lo >= 0) {
-    // a plan created by wealy_eval_plan_create_host that is run on device embeddings after all: its early upload may
-    // still be writing the planes this run is about to fill -- order the run behind it
-    cudaStream_t up = upload_stream();
-    if (up && p->host_ev[1]) {
-      CU_TRY(cudaEventRecord(p->host_ev[1], up));
-      CU_TRY(cudaStreamWaitEvent(s, p->host_ev[1], 0));
-    }
-    p->early_lo = -1;
-  }
-  if (stage != 2 && (!queries_z || !candidates_z)) return fail(WEALY_ERR_BAD_ARG, "null pointer");
-  if (stage == 2) {
-    if (!p->planes_buf || !p->lvl_thr_buf) return fail(WEALY_ERR_BAD_ARG, "wealy_eval_shard_sweep needs wealy_eval_shard_prepare first");
-    if (chunks > 1 ? p->staged_chunks != chunks : p->staged_chunks > 1)
-      return fail(WEALY_ERR_BAD_ARG, "the staged sweep needs a prepare of the same layout (%d chunks per track)", chunks);
-    queries_z = candidates_z = p;  // (not dereferenced: the planes are in the plan)
-  }
-  if (finish && (!aps || !r1s || !sums)) return fail(WEALY_ERR_BAD_ARG, "null pointer");
-  if (shard_world < 1 || shard_rank < 0 || shard_rank >= shard_world) return fail(WEALY_ERR_BAD_ARG, "bad shard %d/%d", shard_rank, shard_world);
-  if (d <= 0) return fail(WEALY_ERR_BAD_ARG, "bad embedding size %lld", (long long)d);
-  if (passes != 1 && passes != 3) return fail(WEALY_ERR_BAD_ARG, "passes must be 1 or 3");
-  if (topk < 0 || topk > 800) return fail(WEALY_ERR_UNSUPPORTED, "topk must be in [0, 800], got %d", topk);
-  if (topk > 0 && (!(local ? (void*)local_idx : (void*)topk_idx) || !topk_sim)) return fail(WEALY_ERR_BAD_ARG, "topk outputs are null");
-  const int64_t nq = p->nq, nc = p->nc;
-  const bool same = (queries_z == candidates_z && nq == nc && ld_q == ld_c);
-  if (chunks != 1 && chunks != 2 && chunks != 4 && chunks != 8 && chunks != 16)
-    return fail(WEALY_ERR_UNSUPPORTED, "chunks per track must be 1, 2, 4, 8 or 16, got %d", chunks);
-  if (redux < WEALY_REDUX_MIN || redux > WEALY_REDUX_MINMEAN) return fail(WEALY_ERR_BAD_ARG, "unknown redux %d", redux);
-  if ((q_len == nullptr) != (c_len == nullptr)) return fail(WEALY_ERR_BAD_ARG, "q_len and c_len go together");
-  if (q_len && chunks == 1) return fail(WEALY_ERR_BAD_ARG, "chunk counts need chunks > 1");
-  if ((nq * chunks) >= (1ll << 31) - 256 || (nc * chunks) >= (1ll << 31) - 256) return fail(WEALY_ERR_UNSUPPORTED, "more than 2^31 rows");
+// One evaluation call: what the caller hands over, which stage of a staged run it is, and where the results go.
+enum class EvalStage {
+  kWhole,    // everything in one call
+  kPrepare,  // sharded all-vs-all, stage 1: prep + the relevant similarities of THIS rank's share of the queries, then
+             // return (the caller sums the threshold buffer over the ranks)
+  kSweep,    // stage 2: the sweep, on the planes and thresholds stage 1 left in the plan
+};
+
+struct EvalCall {
+  const void* q_z = nullptr;  // (kSweep: unused, the planes are in the plan)
+  const void* c_z = nullptr;
+  int64_t ld_q = 0, ld_c = 0, d = 0;
+  int dtype = WEALY_F32;
+  float eps = 0.f;
+  int passes = 1;
+  int topk = 0;
+  int chunks = 1;  // > 1: every track has `chunks` embeddings (rows t * chunks ..), reduced per track pair by `redux`
+  int redux = WEALY_REDUX_MIN;
+  const int* q_len = nullptr;  // ragged tracks: valid chunks of every query / candidate track
+  const int* c_len = nullptr;
+  // shard_world > 1: the row blocks rb = shard_rank (mod shard_world) of the sweep; the rank counts stay in the plan's
+  // histogram for the caller to sum over the ranks
+  int shard_rank = 0, shard_world = 1;
+  EvalStage stage = EvalStage::kWhole;
+  // outputs.  aps / r1s / sums present: finish in this call (AP, R1 and the running sums)
+  float *aps = nullptr, *r1s = nullptr;
+  double* sums = nullptr;
+  int64_t* topk_idx = nullptr;
+  float* topk_sim = nullptr;
+  // local_cnt present (wealy_eval_sweep_shard_topk): the symmetric top-k sweep over this rank's row blocks, its lists
+  // finalized locally into topk_sim / local_idx / local_cnt
+  int *local_idx = nullptr, *local_cnt = nullptr;
+
+  EvalCall(const void* q_z, int64_t ld_q, const void* c_z, int64_t ld_c, int64_t d, int dtype, float eps, int passes)
+      : q_z(q_z), c_z(c_z), ld_q(ld_q), ld_c(ld_c), d(d), dtype(dtype), eps(eps), passes(passes) {}
+};
+
+enum class EvalSweep {
+  kSym,         // symmetric all-vs-all sweep in the clique-sorted view (tiles above the diagonal, both directions)
+  kSymTopk,     // ... with top-k lists behind sampled per-query bounds
+  kTracksHalf,  // chunked tracks, all-vs-all, a reduction with d(q, c) == d(c, q): tiles above the diagonal
+  kTracksRect,  // chunked tracks, every query against every candidate
+  kRect,        // plain embeddings, every query against every candidate (streaming top-k)
+};
+
+struct EvalRoute {
+  EvalSweep sweep = EvalSweep::kRect;
+  bool same = false;  // one embedding matrix on both sides: one set of planes
   // similarity space: distance min <-> similarity max; {inner over the candidate's chunks, outer over the query's}
   int red_inner = kRedMax, red_outer = kRedMax;
   float red_scale = 1.f;
-  switch (redux) {
+  int64_t rows_q = 0;  // plane rows of the queries
+  bool sym() const { return sweep == EvalSweep::kSym || sweep == EvalSweep::kSymTopk; }
+};
+
+static size_t pair_slots(const wealy_eval_plan* p) { return (size_t)(p->total_pairs > 0 ? p->total_pairs : 1); }
+
+// Checks a call against the plan and picks its sweep.  try_sym_topk == false keeps top-k on the rectangle sweep (the run
+// that replaces symmetric top-k lists which missed some query's k best).
+static int eval_route(const wealy_eval_plan* p, const EvalCall& c, bool try_sym_topk, EvalRoute& r) {
+  const bool staged_sweep = c.stage == EvalStage::kSweep;
+  const bool local = c.local_cnt != nullptr;
+  if (!staged_sweep && (!c.q_z || !c.c_z)) return fail(WEALY_ERR_BAD_ARG, "null pointer");
+  if (staged_sweep) {
+    if (!p->planes_buf || !p->lvl_thr_buf) return fail(WEALY_ERR_BAD_ARG, "wealy_eval_shard_sweep needs wealy_eval_shard_prepare first");
+    if (c.chunks > 1 ? p->staged_chunks != c.chunks : p->staged_chunks > 1)
+      return fail(WEALY_ERR_BAD_ARG, "the staged sweep needs a prepare of the same layout (%d chunks per track)", c.chunks);
+  }
+  if (c.shard_world < 1 || c.shard_rank < 0 || c.shard_rank >= c.shard_world)
+    return fail(WEALY_ERR_BAD_ARG, "bad shard %d/%d", c.shard_rank, c.shard_world);
+  if (c.stage != EvalStage::kWhole && c.shard_world < 2) return fail(WEALY_ERR_BAD_ARG, "staged sweeps are for two or more ranks");
+  if (c.d <= 0) return fail(WEALY_ERR_BAD_ARG, "bad embedding size %lld", (long long)c.d);
+  if (c.passes != 1 && c.passes != 3) return fail(WEALY_ERR_BAD_ARG, "passes must be 1 or 3");
+  if (c.topk < 0 || c.topk > 800) return fail(WEALY_ERR_UNSUPPORTED, "topk must be in [0, 800], got %d", c.topk);
+  if (c.topk > 0 && (!(local ? (void*)c.local_idx : (void*)c.topk_idx) || !c.topk_sim))
+    return fail(WEALY_ERR_BAD_ARG, "topk outputs are null");
+  const int64_t nq = p->nq, nc = p->nc;
+  const int chunks = c.chunks;
+  // (the staged sweep has no embeddings of its own: those of the prepare, queries == candidates)
+  r.same = (staged_sweep || (c.q_z == c.c_z && c.ld_q == c.ld_c)) && nq == nc;
+  if (chunks != 1 && chunks != 2 && chunks != 4 && chunks != 8 && chunks != 16)
+    return fail(WEALY_ERR_UNSUPPORTED, "chunks per track must be 1, 2, 4, 8 or 16, got %d", chunks);
+  if (c.redux < WEALY_REDUX_MIN || c.redux > WEALY_REDUX_MINMEAN) return fail(WEALY_ERR_BAD_ARG, "unknown redux %d", c.redux);
+  if ((c.q_len == nullptr) != (c.c_len == nullptr)) return fail(WEALY_ERR_BAD_ARG, "q_len and c_len go together");
+  if (c.q_len && chunks == 1) return fail(WEALY_ERR_BAD_ARG, "chunk counts need chunks > 1");
+  if ((nq * chunks) >= (1ll << 31) - 256 || (nc * chunks) >= (1ll << 31) - 256) return fail(WEALY_ERR_UNSUPPORTED, "more than 2^31 rows");
+  r.red_inner = r.red_outer = kRedMax;
+  r.red_scale = 1.f;
+  switch (c.redux) {
     case WEALY_REDUX_MIN: break;
-    case WEALY_REDUX_MAX: red_inner = red_outer = kRedMin; break;
-    case WEALY_REDUX_MEAN: red_inner = red_outer = kRedSum; red_scale = 1.f / (float)(chunks * chunks); break;
-    case WEALY_REDUX_MEANMIN: red_inner = kRedMax; red_outer = kRedSum; red_scale = 1.f / (float)chunks; break;
-    case WEALY_REDUX_MINMEAN: red_inner = kRedSum; red_outer = kRedMax; red_scale = 1.f / (float)chunks; break;
+    case WEALY_REDUX_MAX: r.red_inner = r.red_outer = kRedMin; break;
+    case WEALY_REDUX_MEAN: r.red_inner = r.red_outer = kRedSum; r.red_scale = 1.f / (float)(chunks * chunks); break;
+    case WEALY_REDUX_MEANMIN: r.red_inner = kRedMax; r.red_outer = kRedSum; r.red_scale = 1.f / (float)chunks; break;
+    case WEALY_REDUX_MINMEAN: r.red_inner = kRedSum; r.red_outer = kRedMax; r.red_scale = 1.f / (float)chunks; break;
   }
 
   // Symmetric all-vs-all: queries ARE the candidates (same ids, same embeddings), no top-k.  Only the tiles
   // that reach above the diagonal are contracted (half the tensor work); every element scores both its row
   // query and its column query.  Runs in the plan's clique-sorted row order (eval_sym_epilogue.cuh).
-  const bool can_sym = same && p->same_ids && chunks == 1 && p->total_pairs < (1ll << 31) - 8;
+  const bool can_sym = r.same && p->same_ids && chunks == 1 && p->total_pairs < (1ll << 31) - 8;
   // ... with top-k (topk_sym_kernels.cuh): a sampled pre-pass bounds every query's k-th best similarity from below, the
   // sweep appends what lies above the bound to per-query lists in both directions.  Worth it (and statistically sound)
   // for large sets and moderate k; everything else keeps the rectangle sweep with its streaming top-k.
-  const bool sym_topk = can_sym && topk > 0 && topk <= 128 && nq >= env_int("WEALY_SYM_TOPK_MIN_ROWS", 16384) &&
-                        nq >= 192ll * topk && (local || (finish && shard_world == 1)) &&
-                        allow_sym_topk && env_int("WEALY_SYM_TOPK", 1) != 0;
-  const bool sym = can_sym && (topk == 0 || sym_topk);
+  const bool sym_topk = can_sym && c.topk > 0 && c.topk <= 128 && nq >= env_int("WEALY_SYM_TOPK_MIN_ROWS", 16384) &&
+                        nq >= 192ll * c.topk && (local || (c.aps && c.shard_world == 1)) && try_sym_topk &&
+                        env_int("WEALY_SYM_TOPK", 1) != 0;
   // chunked tracks, all-vs-all: the same halving for reductions that give d(q, c) == d(c, q) (min / max / mean)
-  const bool all_tracks = same && p->same_ids && chunks > 1 && topk == 0;
-  const bool sym_tracks = all_tracks && red_inner == red_outer && nq * chunks > 2 * kTileM && env_int("WEALY_SYM_TRACKS", 1) != 0;
+  const bool all_tracks = r.same && p->same_ids && chunks > 1 && c.topk == 0;
+  const bool sym_tracks = all_tracks && r.red_inner == r.red_outer && nq * chunks > 2 * kTileM && env_int("WEALY_SYM_TRACKS", 1) != 0;
+  if (sym_topk) r.sweep = EvalSweep::kSymTopk;
+  else if (can_sym && c.topk == 0) r.sweep = EvalSweep::kSym;
+  else if (chunks > 1) r.sweep = sym_tracks ? EvalSweep::kTracksHalf : EvalSweep::kTracksRect;
+  else r.sweep = EvalSweep::kRect;
   if (local && !sym_topk)
     return fail(WEALY_ERR_UNSUPPORTED, "the sharded top-k sweep needs queries == candidates (ids and embeddings), plain "
-                "embeddings, k <= 128 and N >= max(WEALY_SYM_TOPK_MIN_ROWS, 192 k), got N = %lld, k = %d", (long long)nq, topk);
-  if (shard_world > 1 && !sym && !all_tracks)
+                "embeddings, k <= 128 and N >= max(WEALY_SYM_TOPK_MIN_ROWS, 192 k), got N = %lld, k = %d", (long long)nq, c.topk);
+  if (c.shard_world > 1 && !r.sym() && !all_tracks)
     return fail(WEALY_ERR_BAD_ARG, "a sharded sweep needs queries == candidates (ids and embeddings) and no top-k");
-
-  // operand planes (cached allocation)
-  const int64_t rq = nq * chunks, rc = nc * chunks;  // embedding rows
   // the symmetric sweep stores its planes in spread order over whole 128-row blocks (gemm_core.cuh)
-  const int64_t rows_q = sym ? ceil_div(nq, kTileM) * kTileM : rq;
-  const size_t need = planes_bytes(rows_q, d, passes) + (same ? 0 : planes_bytes(rc, d, passes)) + 2048;
-  if (need > p->planes_cap) {
-    big_free(p->planes_buf, p->planes_cap, s);
-    p->planes_buf = nullptr;
-    p->planes_cap = 0;
-    CU_TRY(big_alloc((void**)&p->planes_buf, &p->planes_cap, need, s));
-  }
-  uint8_t* cur = reinterpret_cast<uint8_t*>(align_up((size_t)p->planes_buf, 1024));
-  Planes pq, pc;
-  carve_planes(pq, cur, rows_q, d, passes);
-  if (same) pc = pq; else carve_planes(pc, cur, rc, d, passes);
-  if (!p->ev0) {
-    CU_TRY(cudaEventCreate(&p->ev0));
-    CU_TRY(cudaEventCreate(&p->ev1));
-    for (cudaEvent_t& e : p->evs) CU_TRY(cudaEventCreate(&e));
-  }
-  if (stage != 0 && !((sym || all_tracks) && shard_world > 1))
-    return fail(WEALY_ERR_BAD_ARG, "staged runs belong to the sharded all-vs-all sweep");
-  if (stage != 2) CU_TRY(cudaEventRecord(p->evs[0], s));
-  if (stage != 2) {
-    W_TRY(launch_prep(queries_z, ld_q, rows_q, d, dtype, kPrepL2AddEps, eps, pq, nullptr, nullptr, 0, nullptr, 0, s,
-                      sym ? p->sorted_idx : nullptr, sym ? (int)nq : 0));
-    if (!same) W_TRY(launch_prep(candidates_z, ld_c, rc, d, dtype, kPrepL2AddEps, eps, pc, nullptr, nullptr, 0, nullptr, 0, s));
-  }
+  r.rows_q = r.sym() ? ceil_div(nq, kTileM) * kTileM : nq * chunks;
+  return WEALY_OK;
+}
 
-  // K_pos: relevant similarities, sorted per query
-  if (stage != 2) CU_TRY(cudaEventRecord(p->evs[1], s));
-  if (stage != 2) {
-    const int threads = 256;
-    if (sym) {
-      // stage 1: this rank's share of the 16-query blocks only; the buffer {lvl, thr} is zeroed first so that the sum
-      // over the ranks assembles the whole of it
-      int q_lo = 0, q_hi = (int)nq;
-      if (stage == 1) {
-        const int64_t nblk = ceil_div(nq, 16);
-        q_lo = (int)(nblk * shard_rank / shard_world) * 16;
-        q_hi = (int)std::min<int64_t>((nblk * (shard_rank + 1) / shard_world) * 16, nq);
-        CU_TRY(cudaMemsetAsync(p->lvl_thr_buf, 0, (size_t)p->s_padded * 16 + (size_t)(p->total_pairs > 0 ? p->total_pairs : 1) * 4, s));
-      }
-      // the plan's cnt array doubles as the per-query fill counter of step 1 (step 2 rewrites it)
-      CU_TRY(cudaMemsetAsync(p->cnt, 0, (size_t)nq * 4, s));
-      if (q_hi > q_lo)
-        pos_pairs_sorted_kernel<false><<<(unsigned)ceil_div(q_hi - q_lo, 16), threads, 0, s>>>(
-            pq.hi, pq.lo, (int)pq.d_pad, p->sorted_c, p->s_i, (int)nq, p->s_seg_lo, p->s_seg_len, p->s_off, p->raw, p->cnt, nullptr,
-            q_lo, q_hi);
-      const unsigned blocks = (unsigned)ceil_div(p->s_padded * 32, threads);
-      pos_sort_sorted_kernel<<<blocks, threads, 0, s>>>(p->s_npos, (int)nq, (int)p->s_padded, p->s_off, p->raw, p->thr,
-                                                        p->cnt, p->s_lvl, p->s_cinfo, q_lo, q_hi);
-    } else if (chunks > 1) {
-      // stage 1: this rank's contiguous share of the query tracks, on a zeroed thr (its CSR rows are disjoint from the
-      // other ranks', so the sum over the ranks assembles the whole of it); cnt / lim are rebuilt by stage 2
-      int q_lo = 0, q_hi = (int)nq;
-      if (stage == 1) {
-        q_lo = (int)(nq * shard_rank / shard_world);
-        q_hi = (int)(nq * (shard_rank + 1) / shard_world);
-        CU_TRY(cudaMemsetAsync(p->thr, 0, (size_t)(p->total_pairs > 0 ? p->total_pairs : 1) * 4, s));
-      }
-      if (q_hi > q_lo)
-        pos_thresholds_tracks_kernel<<<(unsigned)(q_hi - q_lo), threads, 0, s>>>(
-            pq.hi, pq.lo, pc.hi, pc.lo, (int)pq.d_pad, chunks, red_inner, red_outer, red_scale, p->q_i, (int)nq, p->sorted_idx,
-            p->c_i, p->seg_lo, p->seg_len, p->off, p->raw, p->thr, p->lim, p->cnt, q_len, c_len, q_lo);
-    } else if (same && p->same_ids && nq > 0) {
-      // all-vs-all through the rectangle sweep (top-k requested): the clique-block tensor-core K_pos of the symmetric
-      // path on the caller's row order (every unordered pair's operands are read once per 16 x 8 block, not per pair)
-      CU_TRY(cudaMemsetAsync(p->cnt, 0, (size_t)nq * 4, s));
-      pos_pairs_sorted_kernel<true><<<(unsigned)ceil_div(nq, 16), threads, 0, s>>>(
-          pq.hi, pq.lo, (int)pq.d_pad, p->sorted_c, p->s_i, (int)nq, p->s_seg_lo, p->s_seg_len, p->off, p->raw, p->cnt,
-          p->sorted_idx);
-      pos_sort_kernel<<<(unsigned)ceil_div(nq * 32, threads), threads, 0, s>>>((int)nq, p->off, p->raw, p->thr, p->lim, p->cnt);
-    } else {
-      const unsigned blocks = (unsigned)ceil_div(nq * 32, threads);
-      pos_thresholds_kernel<<<blocks, threads, 0, s>>>(pq.hi, pq.lo, pc.hi, pc.lo, (int)pq.d_pad, p->q_i, (int)nq,
-                                                       p->sorted_idx, p->c_i, p->seg_lo, p->seg_len, p->off, p->raw,
-                                                       p->thr, p->lim, p->cnt);
-    }
-    CU_TRY(cudaGetLastError());
+// Grows an embedding-dependent plan buffer to `need` bytes (its contents are not kept).
+static int grow_buffer(void** buf, size_t* cap, size_t need, cudaStream_t s) {
+  if (need <= *cap) return WEALY_OK;
+  big_free(*buf, *cap, s);
+  *buf = nullptr;
+  *cap = 0;
+  CU_TRY(big_alloc(buf, cap, need, s));
+  return WEALY_OK;
+}
+
+// Operand planes of a run (cached in the plan): rows_q query rows, and rows_c candidate rows of their own unless rows_c
+// is 0 (one matrix on both sides: *pc = pq).
+static int eval_planes(wealy_eval_plan* p, int64_t rows_q, int64_t rows_c, int64_t d, int passes, cudaStream_t s, Planes& pq,
+                       Planes* pc = nullptr) {
+  const size_t need = planes_bytes(rows_q, d, passes) + (rows_c ? planes_bytes(rows_c, d, passes) : 0) + 2048;
+  W_TRY(grow_buffer(&p->planes_buf, &p->planes_cap, need, s));
+  uint8_t* cur = reinterpret_cast<uint8_t*>(align_up((size_t)p->planes_buf, 1024));
+  carve_planes(pq, cur, rows_q, d, passes);
+  if (pc) {
+    if (rows_c) carve_planes(*pc, cur, rows_c, d, passes);
+    else *pc = pq;
   }
-  if (stage == 1) {
-    p->last_sym = sym;
-    p->last_stream = s;
-    p->staged_chunks = chunks;
-    return WEALY_OK;
-  }
-  if (stage == 2 && chunks > 1) {
-    track_limits_kernel<<<(unsigned)ceil_div(nq, 256), 256, 0, s>>>(p->off, p->thr, (int)nq, p->lim, p->cnt);
-    CU_TRY(cudaGetLastError());
-  }
-  // ---- top-k in the symmetric sweep: sampled pre-pass -> per-query lower bound of the k-th best similarity
-  float* tk_val = nullptr;
-  int *tk_idx = nullptr, *tk_cnt = nullptr, *tk_fail = nullptr;
-  float* tk_beta = nullptr;
-  int tk_cap2 = 0;
-  if (sym_topk) {
-    const int n = (int)nq, rows = (int)rows_q;
-    // sample ~N/16 rows (>= 4096): the pre-pass is one fp16 pass of N x S pairs.  Target: t = max(24, 3 k S / N) of the
-    // sample's similarities above the bound, i.e. about t N / S >= 3 k of the corpus; the bound is the m-th largest of
-    // the G = S / 32 group maxima, and the top t of S values occupy about G (1 - exp(-t / G)) distinct groups.
-    int S = (int)ceil_div(nq / 16, kTileN) * kTileN;
-    if (S < 4096) S = 4096;
-    if (S > 32768) S = 32768;
-    if (S > n) S = n / kTileN * kTileN;
-    const double fr = (double)S / (double)n, G = (double)(S / kChunkCols);
-    double t = 3.0 * topk * fr;
-    if (t < 24.0) t = 24.0;
-    const int r = (int)ceil(G * (1.0 - exp(-t / G)));
-    const double mean = t / fr, sd = 1.15 * sqrt(t * (1.0 - fr)) / fr;
-    tk_cap2 = (int)align_up((size_t)(mean + 8.0 * sd + 32.0), 32);
-    if (tk_cap2 > 1024) tk_cap2 = 1024;
-    const int n_groups = S / kChunkCols;
-    // carve the scratch
-    size_t need_tk = 0;
-    auto reserve = [&](size_t bytes) { const size_t o = need_tk; need_tk += align_up(bytes, 1024); return o; };
-    const size_t o_samp = reserve((size_t)S * pq.d_pad * 2);
-    const size_t o_gmax = reserve((size_t)rows * n_groups * 4);
-    const size_t o_beta = reserve((size_t)rows * 4);
-    const size_t o_tv = reserve((size_t)rows * tk_cap2 * 4);
-    const size_t o_ti = reserve((size_t)rows * tk_cap2 * 4);
-    const size_t o_tc = reserve((size_t)rows * 4);
-    const size_t o_fail = reserve(256);
-    if (need_tk + 1024 > p->tks_cap) {
-      big_free(p->tks_buf, p->tks_cap, s);
-      p->tks_buf = nullptr;
-      p->tks_cap = 0;
-      CU_TRY(big_alloc(&p->tks_buf, &p->tks_cap, need_tk + 1024, s));
-    }
-    uint8_t* tb = reinterpret_cast<uint8_t*>(align_up((size_t)p->tks_buf, 1024));
-    __half* samp = reinterpret_cast<__half*>(tb + o_samp);
-    float* gmax = reinterpret_cast<float*>(tb + o_gmax);
-    tk_beta = reinterpret_cast<float*>(tb + o_beta);
-    tk_val = reinterpret_cast<float*>(tb + o_tv);
-    tk_idx = reinterpret_cast<int*>(tb + o_ti);
-    tk_cnt = reinterpret_cast<int*>(tb + o_tc);
-    tk_fail = reinterpret_cast<int*>(tb + o_fail);
-    const int T = 256;
-    CU_TRY(cudaMemsetAsync(tk_fail, 0, 4, s));
-    sample_rows_kernel<<<(unsigned)ceil_div((int64_t)S * 32, T), T, 0, s>>>(pq.hi, (int)pq.d_pad, n, S, samp);
-    CU_TRY(cudaGetLastError());
-    Planes pa = pq, pb;
-    pa.lo = nullptr;
-    pb.hi = samp; pb.lo = nullptr; pb.rows = S; pb.d_pad = pq.d_pad;
-    pb.norm = pb.scale = pb.sq = nullptr;
-    GemmShape shp;
-    fill_shape(shp, rows, S, pq.d_pad, 64, 1 << 20, 8);
-    GroupMaxParams gp;
-    gp.gmax = gmax;
-    gp.n_groups = n_groups;
-    W_TRY(launch_gemm<GroupMaxEpi>(1, pa, pb, shp, gp, s));  // (the CTA-pair core was measured no faster here: 1.385 vs 1.387 ms for K_pos + pre-pass)
-    topk_beta_kernel<<<(unsigned)ceil_div(p->s_padded * 32, 128), 128, 0, s>>>(gmax, n_groups, rows, r + 1, n, tk_beta, p->s_lvl,
-                                                                              (int)p->s_padded, tk_cnt);
-    CU_TRY(cudaGetLastError());
-  }
-  p->last_topk_path = topk > 0 ? (sym_topk ? 1 : 2) : 0;
-  p->last_sym = sym;
+  return WEALY_OK;
+}
+
+// The events that time a run's stages (created with the first run)
+static int plan_events(wealy_eval_plan* p) {
+  if (p->ev0) return WEALY_OK;
+  CU_TRY(cudaEventCreate(&p->ev0));
+  CU_TRY(cudaEventCreate(&p->ev1));
+  for (cudaEvent_t& e : p->evs) CU_TRY(cudaEventCreate(&e));
+  return WEALY_OK;
+}
+
+// What later calls (finish, ranks, stage_ms, thresholds, destroy) read about the run just enqueued.  swept: the run
+// recorded the sweep's events (then `finished`: also those of ap_reduce and the top-k finalize).
+static void note_run(wealy_eval_plan* p, cudaStream_t s, bool sym, bool swept, bool finished = false, int topk_path = 0) {
   p->last_stream = s;
-  CU_TRY(cudaMemsetAsync(p->hist, 0, (size_t)(p->total_pairs > 0 ? p->total_pairs : 1) * 4, s));
-  if (finish) CU_TRY(cudaMemsetAsync(sums, 0, 3 * sizeof(double), s));
+  p->last_sym = sym;
+  if (!swept) return;
+  p->timed = true;
+  p->finished = finished;
+  p->last_topk_path = topk_path;
+}
+
+// K_pos of the clique-sorted view for the sorted queries [q_lo, q_hi): their relevant similarities (step 1), sorted into
+// thr, lvl and cinfo (step 2).  partial == false: step 2 covers every row (the rows of other queries get their id-only
+// data); partial: only [q_lo, q_hi), plus the padding rows when the range reaches n (a part of a host run).
+static int kpos_sorted(const wealy_eval_plan* p, const Planes& pq, int q_lo, int q_hi, bool partial, cudaStream_t s) {
+  const int threads = 256, n = (int)p->nq;
+  if (q_hi > q_lo)
+    pos_pairs_sorted_kernel<false><<<(unsigned)ceil_div(q_hi - q_lo, 16), threads, 0, s>>>(
+        pq.hi, pq.lo, (int)pq.d_pad, p->sorted_c, p->s_i, n, p->s_seg_lo, p->s_seg_len, p->s_off, p->raw, p->cnt, nullptr,
+        q_lo, q_hi);
+  const int64_t sort_lo = partial ? q_lo : 0, sort_hi = partial && q_hi < n ? q_hi : p->s_padded;
+  pos_sort_sorted_kernel<<<(unsigned)ceil_div((sort_hi - sort_lo) * 32, threads), threads, 0, s>>>(
+      p->s_npos, n, (int)p->s_padded, p->s_off, p->raw, p->thr, p->cnt, p->s_lvl, p->s_cinfo, q_lo, q_hi, partial ? 1 : 0);
+  CU_TRY(cudaGetLastError());
+  return WEALY_OK;
+}
+
+// AP / R1 of every query from the rank counters; sym: the counters are in the clique-sorted view's CSR order
+static int ap_reduce(const wealy_eval_plan* p, bool sym, float* aps, float* r1s, double* sums, cudaStream_t s) {
+  const int threads = 256;
+  ap_reduce_kernel<<<(unsigned)ceil_div(p->nq * 32, threads), threads, 0, s>>>(
+      p->hist, sym ? p->s_off : p->off, p->cnt, (int)p->nq, aps, r1s, sums, sym ? p->sorted_idx : nullptr);
+  CU_TRY(cudaGetLastError());
+  return WEALY_OK;
+}
+
+// Operand planes of the queries (and of the candidates unless they are the same matrix)
+static int eval_prep(const wealy_eval_plan* p, const EvalCall& c, const EvalRoute& r, const Planes& pq, const Planes& pc,
+                     cudaStream_t s) {
+  const bool sym = r.sym();
+  W_TRY(launch_prep(c.q_z, c.ld_q, r.rows_q, c.d, c.dtype, kPrepL2AddEps, c.eps, pq, nullptr, nullptr, 0, nullptr, 0, s,
+                    sym ? p->sorted_idx : nullptr, sym ? (int)p->nq : 0));
+  if (!r.same)
+    W_TRY(launch_prep(c.c_z, c.ld_c, p->nc * c.chunks, c.d, c.dtype, kPrepL2AddEps, c.eps, pc, nullptr, nullptr, 0, nullptr, 0, s));
+  return WEALY_OK;
+}
+
+// K_pos: relevant similarities, sorted per query
+static int eval_kpos(wealy_eval_plan* p, const EvalCall& c, const EvalRoute& r, const Planes& pq, const Planes& pc,
+                     cudaStream_t s) {
+  const int threads = 256;
+  const int64_t nq = p->nq;
+  const bool prepare = c.stage == EvalStage::kPrepare;
+  if (r.sym()) {
+    // stage 1: this rank's share of the 16-query blocks only; the buffer {lvl, thr} is zeroed first so that the sum
+    // over the ranks assembles the whole of it
+    int q_lo = 0, q_hi = (int)nq;
+    if (prepare) {
+      const int64_t nblk = ceil_div(nq, 16);
+      q_lo = (int)(nblk * c.shard_rank / c.shard_world) * 16;
+      q_hi = (int)std::min<int64_t>((nblk * (c.shard_rank + 1) / c.shard_world) * 16, nq);
+      CU_TRY(cudaMemsetAsync(p->lvl_thr_buf, 0, (size_t)p->s_padded * 16 + pair_slots(p) * 4, s));
+    }
+    // the plan's cnt array doubles as the per-query fill counter of step 1 (step 2 rewrites it)
+    CU_TRY(cudaMemsetAsync(p->cnt, 0, (size_t)nq * 4, s));
+    return kpos_sorted(p, pq, q_lo, q_hi, false, s);
+  }
+  if (c.chunks > 1) {
+    // stage 1: this rank's contiguous share of the query tracks, on a zeroed thr (its CSR rows are disjoint from the
+    // other ranks', so the sum over the ranks assembles the whole of it); cnt / lim are rebuilt by stage 2
+    int q_lo = 0, q_hi = (int)nq;
+    if (prepare) {
+      q_lo = (int)(nq * c.shard_rank / c.shard_world);
+      q_hi = (int)(nq * (c.shard_rank + 1) / c.shard_world);
+      CU_TRY(cudaMemsetAsync(p->thr, 0, pair_slots(p) * 4, s));
+    }
+    if (q_hi > q_lo)
+      pos_thresholds_tracks_kernel<<<(unsigned)(q_hi - q_lo), threads, 0, s>>>(
+          pq.hi, pq.lo, pc.hi, pc.lo, (int)pq.d_pad, c.chunks, r.red_inner, r.red_outer, r.red_scale, p->q_i, (int)nq,
+          p->sorted_idx, p->c_i, p->seg_lo, p->seg_len, p->off, p->raw, p->thr, p->lim, p->cnt, c.q_len, c.c_len, q_lo);
+  } else if (r.same && p->same_ids && nq > 0) {
+    // all-vs-all through the rectangle sweep (top-k requested): the clique-block tensor-core K_pos of the symmetric
+    // path on the caller's row order (every unordered pair's operands are read once per 16 x 8 block, not per pair)
+    CU_TRY(cudaMemsetAsync(p->cnt, 0, (size_t)nq * 4, s));
+    pos_pairs_sorted_kernel<true><<<(unsigned)ceil_div(nq, 16), threads, 0, s>>>(
+        pq.hi, pq.lo, (int)pq.d_pad, p->sorted_c, p->s_i, (int)nq, p->s_seg_lo, p->s_seg_len, p->off, p->raw, p->cnt,
+        p->sorted_idx);
+    pos_sort_kernel<<<(unsigned)ceil_div(nq * 32, threads), threads, 0, s>>>((int)nq, p->off, p->raw, p->thr, p->lim, p->cnt);
+  } else {
+    pos_thresholds_kernel<<<(unsigned)ceil_div(nq * 32, threads), threads, 0, s>>>(
+        pq.hi, pq.lo, pc.hi, pc.lo, (int)pq.d_pad, p->q_i, (int)nq, p->sorted_idx, p->c_i, p->seg_lo, p->seg_len, p->off,
+        p->raw, p->thr, p->lim, p->cnt);
+  }
+  CU_TRY(cudaGetLastError());
+  return WEALY_OK;
+}
+
+// Candidate lists of a top-k run, for its finalize
+struct TopkLists {
+  float *val = nullptr, *beta = nullptr;  // beta: the symmetric sweep's per-query bounds from the pre-pass
+  int *idx = nullptr, *cnt = nullptr, *fail = nullptr;  // fail: a symmetric list missed its query's k best
+  int cap = 0, parts = 0;  // slots per list; lists per query (rectangle sweep)
+};
+
+// Top-k in the symmetric sweep: sampled pre-pass -> per-query lower bound of the k-th best similarity
+static int topk_prepass(wealy_eval_plan* p, int topk, int64_t rows_q, const Planes& pq, cudaStream_t s, TopkLists& tl) {
+  const int64_t nq = p->nq;
+  const int n = (int)nq, rows = (int)rows_q;
+  // sample ~N/16 rows (>= 4096): the pre-pass is one fp16 pass of N x S pairs.  Target: t = max(24, 3 k S / N) of the
+  // sample's similarities above the bound, i.e. about t N / S >= 3 k of the corpus; the bound is the m-th largest of
+  // the G = S / 32 group maxima, and the top t of S values occupy about G (1 - exp(-t / G)) distinct groups.
+  int S = (int)ceil_div(nq / 16, kTileN) * kTileN;
+  if (S < 4096) S = 4096;
+  if (S > 32768) S = 32768;
+  if (S > n) S = n / kTileN * kTileN;
+  const double fr = (double)S / (double)n, G = (double)(S / kChunkCols);
+  double t = 3.0 * topk * fr;
+  if (t < 24.0) t = 24.0;
+  const int r = (int)ceil(G * (1.0 - exp(-t / G)));
+  const double mean = t / fr, sd = 1.15 * sqrt(t * (1.0 - fr)) / fr;
+  tl.cap = (int)align_up((size_t)(mean + 8.0 * sd + 32.0), 32);
+  if (tl.cap > 1024) tl.cap = 1024;
+  const int n_groups = S / kChunkCols;
+  // carve the scratch
+  size_t need_tk = 0;
+  auto reserve = [&](size_t bytes) { const size_t o = need_tk; need_tk += align_up(bytes, 1024); return o; };
+  const size_t o_samp = reserve((size_t)S * pq.d_pad * 2);
+  const size_t o_gmax = reserve((size_t)rows * n_groups * 4);
+  const size_t o_beta = reserve((size_t)rows * 4);
+  const size_t o_tv = reserve((size_t)rows * tl.cap * 4);
+  const size_t o_ti = reserve((size_t)rows * tl.cap * 4);
+  const size_t o_tc = reserve((size_t)rows * 4);
+  const size_t o_fail = reserve(256);
+  W_TRY(grow_buffer(&p->tks_buf, &p->tks_cap, need_tk + 1024, s));
+  uint8_t* tb = reinterpret_cast<uint8_t*>(align_up((size_t)p->tks_buf, 1024));
+  __half* samp = reinterpret_cast<__half*>(tb + o_samp);
+  float* gmax = reinterpret_cast<float*>(tb + o_gmax);
+  tl.beta = reinterpret_cast<float*>(tb + o_beta);
+  tl.val = reinterpret_cast<float*>(tb + o_tv);
+  tl.idx = reinterpret_cast<int*>(tb + o_ti);
+  tl.cnt = reinterpret_cast<int*>(tb + o_tc);
+  tl.fail = reinterpret_cast<int*>(tb + o_fail);
+  const int T = 256;
+  CU_TRY(cudaMemsetAsync(tl.fail, 0, 4, s));
+  sample_rows_kernel<<<(unsigned)ceil_div((int64_t)S * 32, T), T, 0, s>>>(pq.hi, (int)pq.d_pad, n, S, samp);
+  CU_TRY(cudaGetLastError());
+  Planes pa = pq, pb;
+  pa.lo = nullptr;
+  pb.hi = samp; pb.lo = nullptr; pb.rows = S; pb.d_pad = pq.d_pad;
+  pb.norm = pb.scale = pb.sq = nullptr;
+  GemmShape shp;
+  fill_shape(shp, rows, S, pq.d_pad, 64, 1 << 20, 8);
+  GroupMaxParams gp;
+  gp.gmax = gmax;
+  gp.n_groups = n_groups;
+  W_TRY(launch_gemm<GroupMaxEpi>(1, pa, pb, shp, gp, s));  // (the CTA-pair core was measured no faster here: 1.385 vs 1.387 ms for K_pos + pre-pass)
+  topk_beta_kernel<<<(unsigned)ceil_div(p->s_padded * 32, 128), 128, 0, s>>>(gmax, n_groups, rows, r + 1, n, tl.beta, p->s_lvl,
+                                                                            (int)p->s_padded, tl.cnt);
+  CU_TRY(cudaGetLastError());
+  return WEALY_OK;
+}
+
+// The fused sweep, bracketed by ev0 / ev1.  Rectangle top-k: its candidate lists go to tl.
+static int eval_sweep(wealy_eval_plan* p, const EvalCall& c, const EvalRoute& r, const Planes& pq, const Planes& pc,
+                      TopkLists& tl, cudaStream_t s) {
+  const int64_t nq = p->nq;
+  CU_TRY(cudaMemsetAsync(p->hist, 0, pair_slots(p) * 4, s));
+  if (c.aps) CU_TRY(cudaMemsetAsync(c.sums, 0, 3 * sizeof(double), s));
 
   const int halves = 2;  // two epilogue warps per TMEM lane quadrant (16 warps and 4 warps were measured no better)
   GemmShape sh;
   // top-k keeps <= 4 candidate lists per query (column chunks x epilogue warps per row)
-  const bool rect_topk = topk > 0 && !sym_topk;
-  fill_shape(sh, rq, rc, pq.d_pad, 64, rect_topk ? (4 / halves) : (1 << 20), rect_topk ? 0 : kEvalTilesPerUnit);
-  const int parts = sh.n_col_chunks * halves;
-  const int cap = rect_topk ? topk_capacity(topk) : 0;
+  const bool rect_topk = c.topk > 0 && r.sweep != EvalSweep::kSymTopk;
+  fill_shape(sh, nq * c.chunks, p->nc * c.chunks, pq.d_pad, 64, rect_topk ? (4 / halves) : (1 << 20),
+             rect_topk ? 0 : kEvalTilesPerUnit);
 
   EvalParams ep;
   memset(&ep, 0, sizeof(ep));
@@ -1370,107 +1464,148 @@ static int eval_run_impl(wealy_eval_plan* p, const void* queries_z, int64_t ld_q
   ep.off = p->off;
   ep.cnt = p->cnt;
   ep.hist = p->hist;
-  ep.topk = topk;
-  ep.cap = cap;
+  ep.topk = c.topk;
   ep.nq_total = (int)nq;
-  ep.red_inner = red_inner;
-  ep.red_outer = red_outer;
-  ep.red_scale = red_scale;
-  ep.q_len = q_len;
-  ep.c_len = c_len;
+  ep.red_inner = r.red_inner;
+  ep.red_outer = r.red_outer;
+  ep.red_scale = r.red_scale;
+  ep.q_len = c.q_len;
+  ep.c_len = c.c_len;
   if (rect_topk) {
-    const size_t slots = (size_t)parts * nq * cap;
-    const size_t tneed = slots * 16 + (size_t)parts * nq * 4 + 1024;  // candidate lists + finalize staging
-    if (tneed > p->topk_cap) {
-      big_free(p->topk_buf, p->topk_cap, s);
-      p->topk_buf = nullptr;
-      p->topk_cap = 0;
-      CU_TRY(big_alloc((void**)&p->topk_buf, &p->topk_cap, tneed, s));
-    }
-    ep.cand_val = reinterpret_cast<float*>(p->topk_buf);
-    ep.cand_idx = reinterpret_cast<int*>(ep.cand_val + slots);
-    ep.cand_cnt = ep.cand_idx + slots;
-    CU_TRY(cudaMemsetAsync(ep.cand_cnt, 0, (size_t)parts * nq * 4, s));
+    tl.parts = sh.n_col_chunks * halves;
+    tl.cap = ep.cap = topk_capacity(c.topk);
+    const size_t slots = (size_t)tl.parts * nq * tl.cap;
+    const size_t tneed = slots * 16 + (size_t)tl.parts * nq * 4 + 1024;  // candidate lists + finalize staging
+    W_TRY(grow_buffer(&p->topk_buf, &p->topk_cap, tneed, s));
+    tl.val = ep.cand_val = reinterpret_cast<float*>(p->topk_buf);
+    tl.idx = ep.cand_idx = reinterpret_cast<int*>(ep.cand_val + slots);
+    tl.cnt = ep.cand_cnt = ep.cand_idx + slots;
+    CU_TRY(cudaMemsetAsync(ep.cand_cnt, 0, (size_t)tl.parts * nq * 4, s));
   }
   CU_TRY(cudaEventRecord(p->ev0, s));
-  if (sym) {
+  const bool half = r.sweep == EvalSweep::kTracksHalf;
+  if (r.sym()) {
     EvalSymParams sp = sym_params(p, sh);
-    sp.beta = tk_beta;
-    sp.tk_val = tk_val;
-    sp.tk_idx = tk_idx;
-    sp.tk_cnt = tk_cnt;
-    sp.tk_cap = tk_cap2;
+    sp.beta = tl.beta;
+    sp.tk_val = tl.val;
+    sp.tk_idx = tl.idx;
+    sp.tk_cnt = tl.cnt;
+    sp.tk_cap = tl.cap;
     // the CTA-pair kernel works on super row blocks (two adjacent row blocks per CTA pair)
     sh.n_row_blocks = (sh.n_row_blocks + 1) / 2;
     sh.group_rows = (sh.group_rows + 1) / 2;
-    shard_row_blocks(sh, shard_rank, shard_world);
-    W_TRY(launch_sym_sweep(passes, sym_topk, pq, sh, sp, s));
-  } else if (chunks == 2) {
-    W_TRY(launch_eval_tracks<2>(passes, pq, pc, sh, ep, s, sym_tracks, shard_rank, shard_world));
-  } else if (chunks == 4) {
-    W_TRY(launch_eval_tracks<4>(passes, pq, pc, sh, ep, s, sym_tracks, shard_rank, shard_world));
-  } else if (chunks == 8) {
-    W_TRY(launch_eval_tracks<8>(passes, pq, pc, sh, ep, s, sym_tracks, shard_rank, shard_world));
-  } else if (chunks == 16) {
-    W_TRY(launch_eval_tracks<16>(passes, pq, pc, sh, ep, s, sym_tracks, shard_rank, shard_world));
+    shard_row_blocks(sh, c.shard_rank, c.shard_world);
+    W_TRY(launch_sym_sweep(c.passes, r.sweep == EvalSweep::kSymTopk, pq, sh, sp, s));
+  } else if (c.chunks == 2) {
+    W_TRY(launch_eval_tracks<2>(c.passes, pq, pc, sh, ep, s, half, c.shard_rank, c.shard_world));
+  } else if (c.chunks == 4) {
+    W_TRY(launch_eval_tracks<4>(c.passes, pq, pc, sh, ep, s, half, c.shard_rank, c.shard_world));
+  } else if (c.chunks == 8) {
+    W_TRY(launch_eval_tracks<8>(c.passes, pq, pc, sh, ep, s, half, c.shard_rank, c.shard_world));
+  } else if (c.chunks == 16) {
+    W_TRY(launch_eval_tracks<16>(c.passes, pq, pc, sh, ep, s, half, c.shard_rank, c.shard_world));
   } else {
-    W_TRY(launch_gemm_rect<EvalEpi>(passes, pq, pc, sh, ep, s));
+    W_TRY(launch_gemm_rect<EvalEpi>(c.passes, pq, pc, sh, ep, s));
   }
   CU_TRY(cudaEventRecord(p->ev1, s));
-  p->timed = true;
-  p->finished = finish;
+  return WEALY_OK;
+}
 
-  if (local) {
+// After the sweep: AP / R1 and the top-k lists (finishing calls), or the local lists of the sharded top-k sweep.
+// *overflow: a symmetric top-k list missed its query's k best (the caller reruns on the rectangle sweep).
+static int eval_finish(wealy_eval_plan* p, const EvalCall& c, const EvalRoute& r, const TopkLists& tl, cudaStream_t s,
+                       bool* overflow) {
+  const int64_t nq = p->nq;
+  const unsigned sym_blocks = (unsigned)ceil_div(r.rows_q * 32, 128);
+  if (c.local_cnt) {
     // (stage events: ap_reduce stays empty -- it runs in wealy_eval_finish once the counters are summed --, topk_finalize
     //  times the local finalize)
     CU_TRY(cudaEventRecord(p->evs[2], s));
-    topk_sym_local_kernel<<<(unsigned)ceil_div(rows_q * 32, 128), 128, 0, s>>>(tk_val, tk_idx, tk_cnt, tk_cap2, (int)rows_q, (int)nq,
-                                                                              topk, p->sorted_idx, topk_sim, local_idx, local_cnt);
+    topk_sym_local_kernel<<<sym_blocks, 128, 0, s>>>(tl.val, tl.idx, tl.cnt, tl.cap, (int)r.rows_q, (int)nq, c.topk,
+                                                     p->sorted_idx, c.topk_sim, c.local_idx, c.local_cnt);
     CU_TRY(cudaGetLastError());
     CU_TRY(cudaEventRecord(p->evs[3], s));
-    p->finished = true;
     return WEALY_OK;
   }
-
-  if (finish) {
-    const int threads = 256;
-    const unsigned blocks = (unsigned)ceil_div(nq * 32, threads);
-    if (sym) ap_reduce_kernel<<<blocks, threads, 0, s>>>(p->hist, p->s_off, p->cnt, (int)nq, aps, r1s, sums, p->sorted_idx);
-    else ap_reduce_kernel<<<blocks, threads, 0, s>>>(p->hist, p->off, p->cnt, (int)nq, aps, r1s, sums);
+  if (!c.aps) return WEALY_OK;
+  W_TRY(ap_reduce(p, r.sym(), c.aps, c.r1s, c.sums, s));
+  CU_TRY(cudaEventRecord(p->evs[2], s));
+  if (r.sweep == EvalSweep::kSymTopk) {
+    topk_sym_finalize_kernel<<<sym_blocks, 128, 0, s>>>(tl.val, tl.idx, tl.cnt, tl.cap, (int)r.rows_q, (int)nq, c.topk,
+                                                        p->sorted_idx, (long long*)c.topk_idx, c.topk_sim, tl.fail);
     CU_TRY(cudaGetLastError());
-    CU_TRY(cudaEventRecord(p->evs[2], s));
-    if (sym_topk) {
-      topk_sym_finalize_kernel<<<(unsigned)ceil_div(rows_q * 32, 128), 128, 0, s>>>(tk_val, tk_idx, tk_cnt, tk_cap2, (int)rows_q, (int)nq,
-                                                                                   topk, p->sorted_idx, (long long*)topk_idx, topk_sim,
-                                                                                   tk_fail);
-      CU_TRY(cudaGetLastError());
-      CU_TRY(cudaEventRecord(p->evs[3], s));
-      // the one host round trip of this path: 4 bytes that say whether every list held its k best (see topk_sym_kernels.cuh)
-      int failed = 0;
-      CU_TRY(cudaMemcpyAsync(&failed, tk_fail, 4, cudaMemcpyDeviceToHost, s));
-      CU_TRY(cudaStreamSynchronize(s));
-      if (failed != 0) {
-        W_TRY(eval_run_impl(p, queries_z, ld_q, candidates_z, ld_c, d, dtype, eps, passes, topk, aps, r1s, sums, topk_idx, topk_sim,
-                            shard_rank, shard_world, finish, stream, chunks, redux, q_len, c_len, false));
-        p->last_topk_path = 3;
-      }
-      return WEALY_OK;
-    }
-    if (topk > 0) {
-      if (parts * cap <= 32 * kFinPerLane) {
-        float* stage_val = reinterpret_cast<float*>(ep.cand_cnt + (size_t)parts * nq);
-        int* stage_idx = reinterpret_cast<int*>(stage_val + (size_t)parts * nq * cap);
-        topk_finalize_select_kernel<<<(unsigned)ceil_div(nq * 32, 128), 128, 0, s>>>(
-            ep.cand_val, ep.cand_idx, ep.cand_cnt, parts, (int)nq, cap, topk, stage_val, stage_idx,
-            (long long*)topk_idx, topk_sim);
-      } else {
-        topk_finalize_kernel<<<blocks, threads, 0, s>>>(ep.cand_val, ep.cand_idx, ep.cand_cnt, parts, (int)nq, cap, topk,
-                                                        (long long*)topk_idx, topk_sim);
-      }
-      CU_TRY(cudaGetLastError());
-    }
     CU_TRY(cudaEventRecord(p->evs[3], s));
+    // the one host round trip of this path: 4 bytes that say whether every list held its k best (see topk_sym_kernels.cuh)
+    int failed = 0;
+    CU_TRY(cudaMemcpyAsync(&failed, tl.fail, 4, cudaMemcpyDeviceToHost, s));
+    CU_TRY(cudaStreamSynchronize(s));
+    *overflow = failed != 0;
+    return WEALY_OK;
   }
+  if (c.topk > 0) {
+    if (tl.parts * tl.cap <= 32 * kFinPerLane) {
+      float* stage_val = reinterpret_cast<float*>(tl.cnt + (size_t)tl.parts * nq);
+      int* stage_idx = reinterpret_cast<int*>(stage_val + (size_t)tl.parts * nq * tl.cap);
+      topk_finalize_select_kernel<<<(unsigned)ceil_div(nq * 32, 128), 128, 0, s>>>(
+          tl.val, tl.idx, tl.cnt, tl.parts, (int)nq, tl.cap, c.topk, stage_val, stage_idx, (long long*)c.topk_idx, c.topk_sim);
+    } else {
+      topk_finalize_kernel<<<(unsigned)ceil_div(nq * 32, 256), 256, 0, s>>>(tl.val, tl.idx, tl.cnt, tl.parts, (int)nq, tl.cap,
+                                                                           c.topk, (long long*)c.topk_idx, c.topk_sim);
+    }
+    CU_TRY(cudaGetLastError());
+  }
+  CU_TRY(cudaEventRecord(p->evs[3], s));
+  return WEALY_OK;
+}
+
+// One run on a decided route, stage by stage
+static int eval_run_route(wealy_eval_plan* p, const EvalCall& c, const EvalRoute& r, cudaStream_t s, bool* overflow) {
+  Planes pq, pc;
+  W_TRY(eval_planes(p, r.rows_q, r.same ? 0 : p->nc * c.chunks, c.d, c.passes, s, pq, &pc));
+  W_TRY(plan_events(p));
+  if (c.stage != EvalStage::kSweep) {
+    CU_TRY(cudaEventRecord(p->evs[0], s));
+    W_TRY(eval_prep(p, c, r, pq, pc, s));
+    CU_TRY(cudaEventRecord(p->evs[1], s));
+    W_TRY(eval_kpos(p, c, r, pq, pc, s));
+  }
+  if (c.stage == EvalStage::kPrepare) {
+    note_run(p, s, r.sym(), false);
+    p->staged_chunks = c.chunks;
+    return WEALY_OK;
+  }
+  if (c.stage == EvalStage::kSweep && c.chunks > 1) {
+    track_limits_kernel<<<(unsigned)ceil_div(p->nq, 256), 256, 0, s>>>(p->off, p->thr, (int)p->nq, p->lim, p->cnt);
+    CU_TRY(cudaGetLastError());
+  }
+  TopkLists tl;
+  if (r.sweep == EvalSweep::kSymTopk) W_TRY(topk_prepass(p, c.topk, r.rows_q, pq, s, tl));
+  W_TRY(eval_sweep(p, c, r, pq, pc, tl, s));
+  note_run(p, s, r.sym(), true, c.aps || c.local_cnt, c.topk > 0 ? (r.sweep == EvalSweep::kSymTopk ? 1 : 2) : 0);
+  return eval_finish(p, c, r, tl, s, overflow);
+}
+
+static int eval_run(wealy_eval_plan* p, const EvalCall& c, cudaStream_t s) {
+  if (!p) return fail(WEALY_ERR_BAD_ARG, "null plan");
+  if (p->early_lo >= 0) {
+    // a plan created by wealy_eval_plan_create_host that is run on device embeddings after all: its early upload may
+    // still be writing the planes this run is about to fill -- order the run behind it
+    cudaStream_t up = upload_stream();
+    if (up && p->host_ev[1]) {
+      CU_TRY(cudaEventRecord(p->host_ev[1], up));
+      CU_TRY(cudaStreamWaitEvent(s, p->host_ev[1], 0));
+    }
+    p->early_lo = -1;
+  }
+  EvalRoute r;
+  W_TRY(eval_route(p, c, true, r));
+  bool overflow = false;
+  W_TRY(eval_run_route(p, c, r, s, &overflow));
+  if (!overflow) return WEALY_OK;
+  // some symmetric top-k list missed its query's k best: the whole run again, top-k on the rectangle sweep
+  W_TRY(eval_route(p, c, false, r));
+  W_TRY(eval_run_route(p, c, r, s, &overflow));
+  p->last_topk_path = 3;
   return WEALY_OK;
 }
 
@@ -1501,8 +1636,8 @@ extern "C" int wealy_eval_plan_stage_ms(const wealy_eval_plan* p, float* ms) {
 extern "C" int wealy_eval_run(wealy_eval_plan* p, const void* queries_z, int64_t ld_q, const void* candidates_z,
                               int64_t ld_c, int64_t d, int dtype, float eps, int passes, int topk, float* aps,
                               float* r1s, double* sums, int64_t* topk_idx, float* topk_sim, void* stream) {
-  return eval_run_impl(p, queries_z, ld_q, candidates_z, ld_c, d, dtype, eps, passes, topk, aps, r1s, sums, topk_idx,
-                       topk_sim, 0, 1, true, stream);
+  return wealy_eval_run_chunked(p, queries_z, ld_q, candidates_z, ld_c, d, dtype, eps, passes, topk, 1, WEALY_REDUX_MIN, aps,
+                                r1s, sums, topk_idx, topk_sim, stream);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1525,22 +1660,22 @@ static cudaStream_t upload_stream() {
   return streams[dev];
 }
 
-// The upload kernel and where it runs.  By default on U = 8 SMs of its own (WEALY_HOST_UP_SMS): CTAs of 512 threads whose
-// shared-memory request keeps the sweep off their SM, while the parts of the sweep that can overlap with the upload run
-// on the remaining SMs.  Measured at 100 000 x 1024 (profiles/r02_host_pipeline.md): 8 SMs already saturate PCIe
-// (51 GB/s).  U = 0 puts two upload warps per SM NEXT to the sweep's CTAs (they fit beside a resident sweep CTA; the
-// largest shared-memory carve-out is requested for them and for the K_pos kernels between the parts, because an SM whose
-// L1 / shared-memory split was chosen for a kernel without shared memory cannot take a sweep CTA until it has drained):
-// that slowed the sweep and K_pos 2-3x while rows were in flight -- the SM's memory pipeline queues behind the
-// microsecond-long host reads.  K_pos also slows down with the number of SMs that read host memory (U = 4: not at all,
-// U = 16: 4x).
+// The upload kernel runs on kHostUpSms SMs of its own: CTAs of kHostUpThreads threads whose shared-memory request keeps
+// the sweep off their SM, while the parts of the sweep that overlap with the upload run on the remaining SMs.  Measured
+// at 100 000 x 1024 on one B200 (profiles/r02_host_pipeline.md, r02_host_knobs.json):
+// - 8 SMs already saturate PCIe (51 GB/s; 4 SMs: 10.1 instead of 8.1 ms for the upload).  K_pos slows down with the
+//   number of SMs that read host memory (U = 4: not at all, U = 16: 4x); 6 to 12 SMs gave the same call time.
+// - 512 threads per CTA: 24.6-25.6 ms per call; 256 the same (25.3-25.7), 128 slower (29.0-29.2, PCIe under-fed).
+// - Upload warps NEXT to the sweep's CTAs (two per SM, no shared memory) slowed the sweep and K_pos 2-3x while rows
+//   were in flight -- the SM's memory pipeline queues behind the microsecond-long host reads: 26.9-27.4 ms per call.
+constexpr int kHostUpSms = 8, kHostUpThreads = 512;
+constexpr size_t kHostUpSmem = 120 * 1024;
+
 struct HostUpload {
   const void* z = nullptr;  // device-side address of the pinned host matrix
   int64_t ld = 0, d = 0;
   int dtype = 0;
   float eps = 0.f;
-  int up_sms = 0, grid = 0, threads = 0;
-  size_t smem = 0;
   cudaStream_t up = nullptr;
 };
 
@@ -1570,95 +1705,55 @@ static int host_upload_setup(HostUpload& h, const void* host_z, int64_t ld, int6
   h.eps = eps;
   h.up = upload_stream();
   if (!h.up) return fail(WEALY_ERR_CUDA, "no upload stream");
-  h.up_sms = std::min(std::max(env_int("WEALY_HOST_UP_SMS", 8), 0), num_sms() / 2);
-  h.smem = h.up_sms > 0 ? 120 * 1024 : 0;
-  h.grid = h.up_sms > 0 ? h.up_sms : num_sms() * std::max(1, env_int("WEALY_HOST_UP_GRID", 1));
-  if (h.up_sms > 0) {
-    h.threads = std::min(512, std::max(32, env_int("WEALY_HOST_UP_THREADS", 512) / 32 * 32));  // (bytes in flight per upload SM)
-  } else {
-    h.threads = env_int("WEALY_HOST_UP_THREADS", 64) <= 32 ? 32 : 64;
-  }
-  const void* up_kernel =
-      h.up_sms > 0 ? (dtype == WEALY_F32 ? (const void*)prep_rows_stream_kernel<float, 512>
-                      : dtype == WEALY_F16 ? (const void*)prep_rows_stream_kernel<__half, 512>
-                                           : (const void*)prep_rows_stream_kernel<__nv_bfloat16, 512>)
-                   : (dtype == WEALY_F32 ? (const void*)prep_rows_stream_kernel<float, 64>
-                      : dtype == WEALY_F16 ? (const void*)prep_rows_stream_kernel<__half, 64>
-                                           : (const void*)prep_rows_stream_kernel<__nv_bfloat16, 64>);
+  const void* up_kernel = dtype == WEALY_F32   ? (const void*)prep_rows_stream_kernel<float, kHostUpThreads>
+                          : dtype == WEALY_F16 ? (const void*)prep_rows_stream_kernel<__half, kHostUpThreads>
+                                               : (const void*)prep_rows_stream_kernel<__nv_bfloat16, kHostUpThreads>;
   CU_TRY(cudaFuncSetAttribute(up_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  if (h.smem) CU_TRY(cudaFuncSetAttribute(up_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h.smem));
+  CU_TRY(cudaFuncSetAttribute(up_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kHostUpSmem));
   return WEALY_OK;
+}
+
+template <typename T>
+static void host_upload_launch(const HostUpload& h, const Planes& pq, const int* sorted_idx, int64_t n, int64_t lo, int64_t hi) {
+  prep_rows_stream_kernel<T, kHostUpThreads><<<kHostUpSms, kHostUpThreads, kHostUpSmem, h.up>>>(
+      (const T*)h.z, (long long)h.ld, (int)lo, (int)hi, (int)h.d, (int)pq.d_pad, h.eps, pq.hi, pq.lo, pq.norm, pq.scale, pq.sq,
+      sorted_idx, (int)n);
 }
 
 // plane rows [lo, hi) (whole 128-row blocks of the spread order) <- the caller's rows, on the upload stream
 static int host_upload_rows(const HostUpload& h, const Planes& pq, const int* sorted_idx, int64_t n, int64_t lo, int64_t hi) {
   if (hi <= lo) return WEALY_OK;
-#define STREAM_ARGS (long long)h.ld, (int)lo, (int)hi, (int)h.d, (int)pq.d_pad, h.eps, pq.hi, pq.lo, pq.norm, pq.scale, pq.sq, sorted_idx, (int)n
-#define STREAM_LAUNCH(T)                                                                                                     \
-  do {                                                                                                                       \
-    if (h.up_sms > 0) prep_rows_stream_kernel<T, 512><<<h.grid, h.threads, h.smem, h.up>>>((const T*)h.z, STREAM_ARGS);       \
-    else prep_rows_stream_kernel<T, 64><<<h.grid, h.threads, 0, h.up>>>((const T*)h.z, STREAM_ARGS);                          \
-  } while (0)
   switch (h.dtype) {
-    case WEALY_F32: STREAM_LAUNCH(float); break;
-    case WEALY_F16: STREAM_LAUNCH(__half); break;
-    default: STREAM_LAUNCH(__nv_bfloat16); break;
+    case WEALY_F32: host_upload_launch<float>(h, pq, sorted_idx, n, lo, hi); break;
+    case WEALY_F16: host_upload_launch<__half>(h, pq, sorted_idx, n, lo, hi); break;
+    default: host_upload_launch<__nv_bfloat16>(h, pq, sorted_idx, n, lo, hi); break;
   }
-#undef STREAM_LAUNCH
-#undef STREAM_ARGS
   CU_TRY(cudaGetLastError());
   return WEALY_OK;
 }
 
 // operand planes of an all-vs-all plan in the sweep's spread order over whole 128-row blocks, and the events of a host run
 static int host_planes(wealy_eval_plan* p, int64_t d, int passes, cudaStream_t s, Planes& pq) {
-  const int64_t rows_q = ceil_div(p->nq, kTileM) * kTileM;
-  const size_t need = planes_bytes(rows_q, d, passes) + 2048;
-  if (need > p->planes_cap) {
-    big_free(p->planes_buf, p->planes_cap, s);
-    p->planes_buf = nullptr;
-    p->planes_cap = 0;
-    CU_TRY(big_alloc((void**)&p->planes_buf, &p->planes_cap, need, s));
-  }
-  uint8_t* cur = reinterpret_cast<uint8_t*>(align_up((size_t)p->planes_buf, 1024));
-  carve_planes(pq, cur, rows_q, d, passes);
-  if (!p->ev0) {
-    CU_TRY(cudaEventCreate(&p->ev0));
-    CU_TRY(cudaEventCreate(&p->ev1));
-    for (cudaEvent_t& e : p->evs) CU_TRY(cudaEventCreate(&e));
-  }
+  W_TRY(eval_planes(p, ceil_div(p->nq, kTileM) * kTileM, 0, d, passes, s, pq));
+  W_TRY(plan_events(p));
   for (cudaEvent_t& e : p->host_ev)
     if (!e) CU_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
   return WEALY_OK;
 }
 
-// parts of a host run, in super row blocks (256 rows) counted from the END: cumulative fractions of the rows
-static float kHostCum[5][8] = {{1.f}, {0.30f, 1.f}, {0.10f, 0.20f, 0.35f, 0.55f, 1.f}, {0.06f, 0.14f, 0.24f, 0.36f, 0.5f, 0.7f, 1.f}, {1.f}};
-static int kHostCount[5] = {1, 2, 5, 7, 1};
+// Parts of a host run, in super row blocks (256 rows) counted from the END: cumulative fractions of the rows.  The
+// 5-part schedule measured best at 100 000 x 1024 on one B200 (r02_host_knobs.json, ms per call): 24.6-25.6, against
+// 25.0-25.4 for 5 / 12 / 22 / 35 / 55 %, 25.5-25.9 for 10 / 25 / 50 %, 26.0-26.7 for 8 / 20 / 40 % and 15 / 40 %,
+// 25.6-25.7 with a part at 80 %; 7 parts: 25.8-26.7.
+static const float kHostCum[4][8] = {{1.f}, {0.30f, 1.f}, {0.10f, 0.20f, 0.35f, 0.55f, 1.f}, {0.06f, 0.14f, 0.24f, 0.36f, 0.5f, 0.7f, 1.f}};
+static const int kHostCount[4] = {1, 2, 5, 7};
+// The schedule by size; WEALY_HOST_PARTS = 1 / 2 / 5 / 7 picks one at any size (the tests use it to reach every schedule
+// with small sets).
 static int host_preset(int64_t n) {
   const int nsb = (int)ceil_div(n, 2 * kTileM);
-  int preset = nsb >= 96 ? 2 : (nsb >= 24 ? 1 : 0);  // (24 k / 6 k rows)
   const int forced = env_int("WEALY_HOST_PARTS", 0);
-  if (forced > 0) preset = forced >= 7 ? 3 : (forced >= 5 ? 2 : (forced >= 2 ? 1 : 0));
-  // WEALY_HOST_CUM="0.1,0.25,0.5" (tuning): a schedule of its own, up to 7 increasing fractions; 1.0 is appended
-  if (const char* cum = getenv("WEALY_HOST_CUM")) {
-    static std::mutex mu;
-    std::lock_guard<std::mutex> lock(mu);
-    int cnt = 0;
-    float last = 0.f;
-    for (const char* q = cum; *q && cnt < 7;) {
-      char* end = nullptr;
-      const float v = strtof(q, &end);
-      if (end == q) break;
-      if (v > last && v < 1.f) kHostCum[4][cnt++] = last = v;
-      q = *end == ',' ? end + 1 : end;
-      if (*end != ',' && *end != 0) break;
-    }
-    kHostCum[4][cnt++] = 1.f;
-    kHostCount[4] = cnt;
-    preset = 4;
-  }
-  return preset;
+  if (forced > 0) return forced >= 7 ? 3 : (forced >= 5 ? 2 : (forced >= 2 ? 1 : 0));
+  return nsb >= 96 ? 2 : (nsb >= 24 ? 1 : 0);  // (24 k / 6 k rows)
 }
 // first super row block of part k
 static int host_part_begin(int64_t n, int preset, int k) {
@@ -1670,24 +1765,16 @@ static int host_part_begin(int64_t n, int preset, int k) {
 
 // As wealy_eval_plan_create for an all-vs-all evaluation of pinned host embeddings (to be run with wealy_eval_run_host on
 // the same matrix): the upload of the first part starts as soon as the sorted order exists, under the rest of the plan.
+// (Measured at 100 000 x 1024: 24.30 / 24.52 ms per call with, 24.97 / 24.31 ms without -- never slower.)
 extern "C" int wealy_eval_plan_create_host(const int64_t* queries_c, const int64_t* queries_i, int64_t nq,
                                            const int64_t* candidates_c, const int64_t* candidates_i, int64_t nc,
                                            const void* host_z, int64_t ld, int64_t d, int dtype, float eps, int passes,
                                            void* stream, wealy_eval_plan** plan) {
-  if (!plan) return fail(WEALY_ERR_BAD_ARG, "plan output pointer is null");
-  *plan = nullptr;
-  if (nq <= 0 || nc <= 0) return fail(WEALY_ERR_BAD_ARG, "empty query or candidate set (nq=%lld nc=%lld)", (long long)nq, (long long)nc);
-  if (!queries_c || !queries_i || !candidates_c || !candidates_i) return fail(WEALY_ERR_BAD_ARG, "null id pointer");
-  if (nq >= (1ll << 31) - 256 || nc >= (1ll << 31) - 256) return fail(WEALY_ERR_UNSUPPORTED, "more than 2^31 rows");
   cudaStream_t s = (cudaStream_t)stream;
-  wealy_eval_plan* p = new wealy_eval_plan();
-  p->nq = nq;
-  p->nc = nc;
-  p->stream = s;
-  auto early = [&]() -> int {
+  auto early = [&](wealy_eval_plan* p) -> int {
     HostUpload h;
     bool on_device = false;
-    if (!host_z || (passes != 1 && passes != 3) || env_int("WEALY_HOST_EARLY", 1) == 0) return WEALY_OK;
+    if (!host_z || (passes != 1 && passes != 3)) return WEALY_OK;
     if (host_upload_setup(h, host_z, ld, d, dtype, eps, &on_device) != WEALY_OK || on_device) return WEALY_OK;  // nothing to start early
     Planes pq;
     W_TRY(host_planes(p, d, passes, s, pq));
@@ -1704,13 +1791,7 @@ extern "C" int wealy_eval_plan_create_host(const int64_t* queries_c, const int64
     p->early_eps = eps;
     return WEALY_OK;
   };
-  int st = plan_build(p, queries_c, queries_i, candidates_c, candidates_i, s, early);
-  if (st != WEALY_OK) {
-    wealy_eval_plan_destroy(p);
-    return st;
-  }
-  *plan = p;
-  return WEALY_OK;
+  return plan_create(queries_c, queries_i, nq, candidates_c, candidates_i, nc, s, plan, early);
 }
 
 extern "C" int wealy_eval_run_host(wealy_eval_plan* p, const void* host_z, int64_t ld, int64_t d, int dtype, float eps,
@@ -1724,29 +1805,17 @@ extern "C" int wealy_eval_run_host(wealy_eval_plan* p, const void* host_z, int64
   HostUpload h;
   bool on_device = false;
   W_TRY(host_upload_setup(h, host_z, ld, d, dtype, eps, &on_device));
-  if (on_device)  // already on the device: the plain run
-    return eval_run_impl(p, host_z, ld, host_z, ld, d, dtype, eps, passes, 0, aps, r1s, sums, nullptr, nullptr, 0, 1, true, stream);
-  const void* z = h.z;
-  cudaStream_t up = h.up;
-  const int up_sms = h.up_sms;
-  const void* kpos_kernels[2] = {(const void*)pos_pairs_sorted_kernel<false>, (const void*)pos_sort_sorted_kernel};
-  struct RestoreCarveout {
-    const void* const* k;
-    bool on;
-    ~RestoreCarveout() {
-      for (int i = 0; on && i < 2; ++i) cudaFuncSetAttribute(k[i], cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutDefault);
-    }
-  } restore{kpos_kernels, up_sms == 0};
-  if (up_sms == 0)  // (upload CTAs on SMs of their own never share an SM with these kernels; the attribute is read at launch)
-    for (const void* k : kpos_kernels)
-      CU_TRY(cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  if (on_device) {  // already on the device: the plain run
+    EvalCall c(host_z, ld, host_z, ld, d, dtype, eps, passes);
+    c.aps = aps, c.r1s = r1s, c.sums = sums;
+    return eval_run(p, c, s);
+  }
 
   Planes pq;
   W_TRY(host_planes(p, d, passes, s, pq));
-  const int64_t rows_q = pq.rows;
   // rows an early upload (wealy_eval_plan_create_host) of exactly this matrix has already put in flight
   int64_t early_lo = -1;
-  if (p->early_lo >= 0 && p->early_z == z && p->early_ld == ld && p->early_d == d && p->early_dtype == dtype &&
+  if (p->early_lo >= 0 && p->early_z == h.z && p->early_ld == ld && p->early_d == d && p->early_dtype == dtype &&
       p->early_passes == passes && p->early_eps == eps)
     early_lo = p->early_lo;
   p->early_lo = -1;
@@ -1762,26 +1831,15 @@ extern "C" int wealy_eval_run_host(wealy_eval_plan* p, const void* host_z, int64
 
   CU_TRY(cudaEventRecord(p->evs[0], s));
   CU_TRY(cudaEventRecord(p->evs[1], s));
-  CU_TRY(cudaMemsetAsync(p->hist, 0, (size_t)(p->total_pairs > 0 ? p->total_pairs : 1) * 4, s));
+  CU_TRY(cudaMemsetAsync(p->hist, 0, pair_slots(p) * 4, s));
   CU_TRY(cudaMemsetAsync(p->cnt, 0, (size_t)n * 4, s));
   CU_TRY(cudaMemsetAsync(sums, 0, 3 * sizeof(double), s));
   CU_TRY(cudaEventRecord(p->host_ev[0], s));           // the upload may touch the planes from here on
-  CU_TRY(cudaStreamWaitEvent(up, p->host_ev[0], 0));
+  CU_TRY(cudaStreamWaitEvent(h.up, p->host_ev[0], 0));
   CU_TRY(cudaEventRecord(p->ev0, s));
 
-  // WEALY_HOST_TRACE=1 (diagnostics): time stamps of every part on both streams, printed to stderr after a synchronize
-  const bool trace = env_int("WEALY_HOST_TRACE", 0) != 0;
-  std::vector<cudaEvent_t> tev;
-  auto stamp = [&](cudaStream_t st) {
-    if (!trace) return;
-    cudaEvent_t e = nullptr;
-    cudaEventCreate(&e);
-    cudaEventRecord(e, st);
-    tev.push_back(e);
-  };
-  stamp(s);
   int sb_hi = nsb;
-  int64_t prep_hi = rows_q;
+  int64_t prep_hi = pq.rows;
   for (int k = 0; k < n_parts; ++k) {
     int sb_lo = host_part_begin(n, preset, k);
     if (sb_lo > sb_hi) sb_lo = sb_hi;
@@ -1789,60 +1847,28 @@ extern "C" int wealy_eval_run_host(wealy_eval_plan* p, const void* host_z, int64
     int64_t prep_lo = k + 1 == n_parts ? 0 : ((int64_t)sb_lo * 2 * kTileM - reach) / kTileM * kTileM;
     if (prep_lo < 0) prep_lo = 0;
     if (prep_lo > prep_hi) prep_lo = prep_hi;
-    stamp(up);
     // (what an early upload already has in flight is not fetched again)
     W_TRY(host_upload_rows(h, pq, p->sorted_idx, n, prep_lo, early_lo >= 0 ? std::min(prep_hi, early_lo) : prep_hi));
-    if (trace) fprintf(stderr, "[wealy host run] part %d: rows [%lld, %lld) arrive, super row blocks [%d, %d) swept\n", k,
-                       (long long)prep_lo, (long long)prep_hi, sb_lo, sb_hi);
     prep_hi = prep_lo;
-    stamp(up);
-    CU_TRY(cudaEventRecord(p->host_ev[1 + k], up));
+    CU_TRY(cudaEventRecord(p->host_ev[1 + k], h.up));
     CU_TRY(cudaStreamWaitEvent(s, p->host_ev[1 + k], 0));
-    stamp(s);
     // ---- caller's stream: K_pos of the part's queries, then its row blocks of the sweep
     const int q_lo = sb_lo * 2 * kTileM;
     const int q_hi = (int)std::min<int64_t>((int64_t)sb_hi * 2 * kTileM, n);
     if (q_hi > q_lo) {
-      const int threads = 256;
-      pos_pairs_sorted_kernel<false><<<(unsigned)ceil_div(q_hi - q_lo, 16), threads, 0, s>>>(
-          pq.hi, pq.lo, (int)pq.d_pad, p->sorted_c, p->s_i, (int)n, p->s_seg_lo, p->s_seg_len, p->s_off, p->raw, p->cnt, nullptr,
-          q_lo, q_hi);
-      const int64_t sort_end = k == 0 ? p->s_padded : q_hi;  // (the first part reaches n: it owns the padding rows)
-      pos_sort_sorted_kernel<<<(unsigned)ceil_div((sort_end - q_lo) * 32, threads), threads, 0, s>>>(
-          p->s_npos, (int)n, (int)p->s_padded, p->s_off, p->raw, p->thr, p->cnt, p->s_lvl, p->s_cinfo, q_lo, q_hi, 1);
-      CU_TRY(cudaGetLastError());
-      stamp(s);
+      W_TRY(kpos_sorted(p, pq, q_lo, q_hi, true, s));
       GemmShape sh = sh0;
       sh.n_row_blocks = sb_hi - sb_lo;
       sh.rb_offset = sb_lo;
       sh.rb_stride = 1;
-      const int max_pairs = (up_sms > 0 && k + 1 < n_parts) ? (num_sms() - up_sms) / 2 : 0;
+      const int max_pairs = k + 1 < n_parts ? (num_sms() - kHostUpSms) / 2 : 0;
       W_TRY(launch_sym_sweep(passes, false, pq, sh, sp, s, max_pairs));
     }
-    else stamp(s);
-    stamp(s);
     sb_hi = sb_lo;
   }
   CU_TRY(cudaEventRecord(p->ev1, s));
-  if (trace) {
-    cudaStreamSynchronize(s);
-    cudaStreamSynchronize(up);
-    // per part: {upload begin, upload end} on the upload stream, {wait over, K_pos done, sweep done} on the run's stream
-    for (int k = 0; k < n_parts && (size_t)(1 + 5 * k + 4) < tev.size(); ++k) {
-      float t[5];
-      for (int j = 0; j < 5; ++j) cudaEventElapsedTime(&t[j], tev[0], tev[1 + 5 * k + j]);
-      fprintf(stderr, "[wealy host run] part %d: upload %.3f -> %.3f ms | ready %.3f, K_pos done %.3f, sweep done %.3f ms\n", k, t[0],
-              t[1], t[2], t[3], t[4]);
-    }
-    for (cudaEvent_t e : tev) cudaEventDestroy(e);
-  }
-  p->timed = true;
-  p->finished = true;
-  p->last_sym = true;
-  p->last_stream = s;
-  p->last_topk_path = 0;
-  ap_reduce_kernel<<<(unsigned)ceil_div(n * 32, 256), 256, 0, s>>>(p->hist, p->s_off, p->cnt, (int)n, aps, r1s, sums, p->sorted_idx);
-  CU_TRY(cudaGetLastError());
+  note_run(p, s, true, true, true);
+  W_TRY(ap_reduce(p, true, aps, r1s, sums, s));
   CU_TRY(cudaEventRecord(p->evs[2], s));
   CU_TRY(cudaEventRecord(p->evs[3], s));
   return WEALY_OK;
@@ -1852,8 +1878,11 @@ extern "C" int wealy_eval_run_chunked(wealy_eval_plan* p, const void* queries_z,
                                       int64_t ld_c, int64_t d, int dtype, float eps, int passes, int topk, int chunks,
                                       int redux, float* aps, float* r1s, double* sums, int64_t* topk_idx, float* topk_sim,
                                       void* stream) {
-  return eval_run_impl(p, queries_z, ld_q, candidates_z, ld_c, d, dtype, eps, passes, topk, aps, r1s, sums, topk_idx,
-                       topk_sim, 0, 1, true, stream, chunks, redux);
+  if (!aps || !r1s || !sums) return fail(WEALY_ERR_BAD_ARG, "null pointer");
+  EvalCall c(queries_z, ld_q, candidates_z, ld_c, d, dtype, eps, passes);
+  c.topk = topk, c.chunks = chunks, c.redux = redux;
+  c.aps = aps, c.r1s = r1s, c.sums = sums, c.topk_idx = topk_idx, c.topk_sim = topk_sim;
+  return eval_run(p, c, (cudaStream_t)stream);
 }
 
 extern "C" int wealy_eval_run_ragged(wealy_eval_plan* p, const void* queries_z, int64_t ld_q, const void* candidates_z,
@@ -1861,8 +1890,19 @@ extern "C" int wealy_eval_run_ragged(wealy_eval_plan* p, const void* queries_z, 
                                      int redux, const int32_t* q_len, const int32_t* c_len, float* aps, float* r1s,
                                      double* sums, int64_t* topk_idx, float* topk_sim, void* stream) {
   if (!q_len || !c_len) return fail(WEALY_ERR_BAD_ARG, "null chunk counts");
-  return eval_run_impl(p, queries_z, ld_q, candidates_z, ld_c, d, dtype, eps, passes, topk, aps, r1s, sums, topk_idx,
-                       topk_sim, 0, 1, true, stream, chunks, redux, q_len, c_len);
+  if (!aps || !r1s || !sums) return fail(WEALY_ERR_BAD_ARG, "null pointer");
+  EvalCall c(queries_z, ld_q, candidates_z, ld_c, d, dtype, eps, passes);
+  c.topk = topk, c.chunks = chunks, c.redux = redux, c.q_len = q_len, c.c_len = c_len;
+  c.aps = aps, c.r1s = r1s, c.sums = sums, c.topk_idx = topk_idx, c.topk_sim = topk_sim;
+  return eval_run(p, c, (cudaStream_t)stream);
+}
+
+// multi-GPU all-vs-all: every rank sweeps its share of the row blocks of the SAME symmetric problem ...
+extern "C" int wealy_eval_sweep_shard(wealy_eval_plan* p, const void* z, int64_t ld, int64_t d, int dtype, float eps,
+                                      int passes, int shard_rank, int shard_world, void* stream) {
+  EvalCall c(z, ld, z, ld, d, dtype, eps, passes);
+  c.shard_rank = shard_rank, c.shard_world = shard_world;
+  return eval_run(p, c, (cudaStream_t)stream);
 }
 
 // The same in two stages, so that the relevant similarities (K_pos) are computed ONCE across the ranks instead of once
@@ -1871,9 +1911,15 @@ extern "C" int wealy_eval_run_ragged(wealy_eval_plan* p, const void* queries_z, 
 // share of the row blocks on the result.
 extern "C" int wealy_eval_shard_prepare(wealy_eval_plan* p, const void* z, int64_t ld, int64_t d, int dtype, float eps,
                                         int passes, int shard_rank, int shard_world, void* stream) {
-  if (shard_world < 2) return fail(WEALY_ERR_BAD_ARG, "staged sweeps are for two or more ranks");
-  return eval_run_impl(p, z, ld, z, ld, d, dtype, eps, passes, 0, nullptr, nullptr, nullptr, nullptr, nullptr, shard_rank,
-                       shard_world, false, stream, 1, WEALY_REDUX_MIN, nullptr, nullptr, true, 1);
+  EvalCall c(z, ld, z, ld, d, dtype, eps, passes);
+  c.shard_rank = shard_rank, c.shard_world = shard_world, c.stage = EvalStage::kPrepare;
+  return eval_run(p, c, (cudaStream_t)stream);
+}
+
+extern "C" int wealy_eval_shard_sweep(wealy_eval_plan* p, int64_t d, int passes, int shard_rank, int shard_world, void* stream) {
+  EvalCall c(nullptr, 0, nullptr, 0, d, WEALY_F32, 0.f, passes);
+  c.shard_rank = shard_rank, c.shard_world = shard_world, c.stage = EvalStage::kSweep;
+  return eval_run(p, c, (cudaStream_t)stream);
 }
 
 extern "C" int wealy_eval_plan_thresholds(const wealy_eval_plan* p, void** values, int64_t* count) {
@@ -1881,62 +1927,52 @@ extern "C" int wealy_eval_plan_thresholds(const wealy_eval_plan* p, void** value
   if (!p->lvl_thr_buf) return fail(WEALY_ERR_BAD_ARG, "the plan is not an all-vs-all plan");
   if (p->staged_chunks > 1) {  // chunked tracks: the thresholds in the caller's CSR order, nothing else
     *values = p->thr;
-    *count = p->total_pairs > 0 ? p->total_pairs : 1;
+    *count = (int64_t)pair_slots(p);
     return WEALY_OK;
   }
   *values = p->lvl_thr_buf;
-  *count = p->s_padded * 4 + (p->total_pairs > 0 ? p->total_pairs : 1);
+  *count = p->s_padded * 4 + (int64_t)pair_slots(p);
   return WEALY_OK;
 }
 
 // Chunked tracks (chunks in {2, 4, 8, 16}, redux WEALY_REDUX_*, lens = NULL or the ragged chunk counts of every track):
 // the same three steps.  min / max / mean take the half sweep, the other reductions (and small sets, WEALY_SYM_TRACKS=0)
 // the rectangle sweep; either way sharded by row blocks.
-static int check_shard_tracks(const wealy_eval_plan* p, int chunks, int shard_rank, int shard_world) {
+static int check_shard_tracks(const wealy_eval_plan* p, int chunks) {
   if (!p) return fail(WEALY_ERR_BAD_ARG, "null plan");
   if (!p->same_ids) return fail(WEALY_ERR_BAD_ARG, "a sharded sweep needs queries == candidates (ids and embeddings) and no top-k");
   if (chunks != 2 && chunks != 4 && chunks != 8 && chunks != 16)
     return fail(WEALY_ERR_UNSUPPORTED, "chunked tracks have 2, 4, 8 or 16 chunks, got %d", chunks);
-  if (shard_world < 1 || shard_rank < 0 || shard_rank >= shard_world) return fail(WEALY_ERR_BAD_ARG, "bad shard %d/%d", shard_rank, shard_world);
   return WEALY_OK;
 }
 
 extern "C" int wealy_eval_sweep_shard_tracks(wealy_eval_plan* p, const void* z, int64_t ld, int64_t d, int dtype, float eps,
                                              int passes, int chunks, int redux, const int32_t* lens, int shard_rank,
                                              int shard_world, void* stream) {
-  W_TRY(check_shard_tracks(p, chunks, shard_rank, shard_world));
-  return eval_run_impl(p, z, ld, z, ld, d, dtype, eps, passes, 0, nullptr, nullptr, nullptr, nullptr, nullptr, shard_rank,
-                       shard_world, false, stream, chunks, redux, lens, lens);
+  W_TRY(check_shard_tracks(p, chunks));
+  EvalCall c(z, ld, z, ld, d, dtype, eps, passes);
+  c.chunks = chunks, c.redux = redux, c.q_len = c.c_len = lens;
+  c.shard_rank = shard_rank, c.shard_world = shard_world;
+  return eval_run(p, c, (cudaStream_t)stream);
 }
 
 extern "C" int wealy_eval_shard_prepare_tracks(wealy_eval_plan* p, const void* z, int64_t ld, int64_t d, int dtype, float eps,
                                                int passes, int chunks, int redux, const int32_t* lens, int shard_rank,
                                                int shard_world, void* stream) {
-  W_TRY(check_shard_tracks(p, chunks, shard_rank, shard_world));
-  if (shard_world < 2) return fail(WEALY_ERR_BAD_ARG, "staged sweeps are for two or more ranks");
-  return eval_run_impl(p, z, ld, z, ld, d, dtype, eps, passes, 0, nullptr, nullptr, nullptr, nullptr, nullptr, shard_rank,
-                       shard_world, false, stream, chunks, redux, lens, lens, true, 1);
+  W_TRY(check_shard_tracks(p, chunks));
+  EvalCall c(z, ld, z, ld, d, dtype, eps, passes);
+  c.chunks = chunks, c.redux = redux, c.q_len = c.c_len = lens;
+  c.shard_rank = shard_rank, c.shard_world = shard_world, c.stage = EvalStage::kPrepare;
+  return eval_run(p, c, (cudaStream_t)stream);
 }
 
 extern "C" int wealy_eval_shard_sweep_tracks(wealy_eval_plan* p, int64_t d, int passes, int chunks, int redux,
                                              const int32_t* lens, int shard_rank, int shard_world, void* stream) {
-  W_TRY(check_shard_tracks(p, chunks, shard_rank, shard_world));
-  if (shard_world < 2) return fail(WEALY_ERR_BAD_ARG, "staged sweeps are for two or more ranks");
-  return eval_run_impl(p, nullptr, 0, nullptr, 0, d, WEALY_F32, 0.f, passes, 0, nullptr, nullptr, nullptr, nullptr, nullptr,
-                       shard_rank, shard_world, false, stream, chunks, redux, lens, lens, true, 2);
-}
-
-extern "C" int wealy_eval_shard_sweep(wealy_eval_plan* p, int64_t d, int passes, int shard_rank, int shard_world, void* stream) {
-  if (shard_world < 2) return fail(WEALY_ERR_BAD_ARG, "staged sweeps are for two or more ranks");
-  return eval_run_impl(p, nullptr, 0, nullptr, 0, d, WEALY_F32, 0.f, passes, 0, nullptr, nullptr, nullptr, nullptr, nullptr,
-                       shard_rank, shard_world, false, stream, 1, WEALY_REDUX_MIN, nullptr, nullptr, true, 2);
-}
-
-// multi-GPU all-vs-all: every rank sweeps its share of the row blocks of the SAME symmetric problem ...
-extern "C" int wealy_eval_sweep_shard(wealy_eval_plan* p, const void* z, int64_t ld, int64_t d, int dtype, float eps,
-                                      int passes, int shard_rank, int shard_world, void* stream) {
-  return eval_run_impl(p, z, ld, z, ld, d, dtype, eps, passes, 0, nullptr, nullptr, nullptr, nullptr, nullptr,
-                       shard_rank, shard_world, false, stream);
+  W_TRY(check_shard_tracks(p, chunks));
+  EvalCall c(nullptr, 0, nullptr, 0, d, WEALY_F32, 0.f, passes);
+  c.chunks = chunks, c.redux = redux, c.q_len = c.c_len = lens;
+  c.shard_rank = shard_rank, c.shard_world = shard_world, c.stage = EvalStage::kSweep;
+  return eval_run(p, c, (cudaStream_t)stream);
 }
 
 // ... with top-k lists: the same sweep with the symmetric top-k epilogue, this rank's lists finalized locally (caller's
@@ -1949,8 +1985,10 @@ extern "C" int wealy_eval_sweep_shard_topk(wealy_eval_plan* p, const void* z, in
   if ((int64_t)shard_world * k > 1024)
     return fail(WEALY_ERR_UNSUPPORTED, "the sharded top-k merge needs world * k <= 1024, got %d x %d", shard_world, k);
   if (!p || !z || !val || !idx || !cnt) return fail(WEALY_ERR_BAD_ARG, "null pointer");
-  return eval_run_impl(p, z, ld, z, ld, d, dtype, eps, passes, k, nullptr, nullptr, nullptr, nullptr, val, shard_rank,
-                       shard_world, false, stream, 1, WEALY_REDUX_MIN, nullptr, nullptr, true, 0, idx, cnt);
+  EvalCall c(z, ld, z, ld, d, dtype, eps, passes);
+  c.topk = k, c.topk_sim = val, c.local_idx = idx, c.local_cnt = cnt;
+  c.shard_rank = shard_rank, c.shard_world = shard_world;
+  return eval_run(p, c, (cudaStream_t)stream);
 }
 
 // The k best of every query's lists of all ranks (val / idx [world][n][k], cnt [world][n]: the local lists of the ranks,
@@ -1980,7 +2018,7 @@ extern "C" int wealy_eval_topk_merge(const float* val, const int32_t* idx, const
 extern "C" int wealy_eval_plan_counts(const wealy_eval_plan* p, void** counts, int64_t* count) {
   if (!p || !counts || !count) return fail(WEALY_ERR_BAD_ARG, "null pointer");
   *counts = p->hist;
-  *count = p->total_pairs > 0 ? p->total_pairs : 1;
+  *count = (int64_t)pair_slots(p);
   return WEALY_OK;
 }
 
@@ -1989,12 +2027,7 @@ extern "C" int wealy_eval_finish(wealy_eval_plan* p, float* aps, float* r1s, dou
   cudaStream_t s = (cudaStream_t)stream;
   if (!p || !aps || !r1s || !sums) return fail(WEALY_ERR_BAD_ARG, "null pointer");
   CU_TRY(cudaMemsetAsync(sums, 0, 3 * sizeof(double), s));
-  const int threads = 256;
-  const unsigned blocks = (unsigned)ceil_div(p->nq * 32, threads);
-  if (p->last_sym) ap_reduce_kernel<<<blocks, threads, 0, s>>>(p->hist, p->s_off, p->cnt, (int)p->nq, aps, r1s, sums, p->sorted_idx);
-  else ap_reduce_kernel<<<blocks, threads, 0, s>>>(p->hist, p->off, p->cnt, (int)p->nq, aps, r1s, sums);
-  CU_TRY(cudaGetLastError());
-  return WEALY_OK;
+  return ap_reduce(p, p->last_sym, aps, r1s, sums, s);
 }
 
 // Per-item ranks of the last run (all ranks' counters summed first in a sharded run): offsets [nq + 1] int64 = CSR

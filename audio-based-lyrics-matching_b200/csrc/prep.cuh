@@ -216,9 +216,9 @@ __global__ void __launch_bounds__(256) prep_rows_kernel(const T* __restrict__ x,
 // K0 for embeddings that still live in PINNED HOST memory (wealy_eval_run_host): the same arithmetic as
 // prep_rows_kernel (identical summation order, IEEE division -> bit-identical planes), but every input row is read
 // exactly ONCE -- it crosses PCIe -- and kept in registers between the norm and the split.  A small persistent grid,
-// rows dealt warp by warp: by default 8 CTAs of kThreads = 512 on SMs of their own (api.cu: host_upload_setup), so that
-// the upload of the next rows runs while the tensor cores of the other SMs sweep the rows that have arrived; the
-// kThreads = 64 instance (72 registers, no shared memory) fits NEXT TO a resident CTA of the sweep -- measured slower.
+// rows dealt warp by warp: 8 CTAs of kThreads = 512 on SMs of their own (api.cu: host_upload_setup), so that the
+// upload of the next rows runs while the tensor cores of the other SMs sweep the rows that have arrived (upload warps
+// NEXT TO the sweep's CTAs were measured slower: api.cu, kHostUpSms).
 // Plane rows [row_lo, row_hi), whole 128-row blocks of the spread order; d <= 128 kRowVecs.
 constexpr int kRowVecs = 8;  // float4 per lane: rows of up to 1024 elements
 template <typename T, int kThreads>

@@ -143,17 +143,12 @@ STAGED_MIN_WORLD = 4
 def _chunks_per_track(z, chunks, redux, q_chunks):
     """Chunks per track of `z` ([N, s, D], or [N * s, D] with chunks=s; 1 for plain [N, D] embeddings).  Every rank
     passes the same arguments, so whatever this refuses is refused on every rank, before any collective."""
-    from . import _native as N
+    from .evaluation import _check_tracks
     shape = tuple(torch.as_tensor(z).shape)
     s = shape[1] if len(shape) == 3 else (1 if chunks is None else int(chunks))
     if len(shape) == 3 and chunks is not None and int(chunks) != s:
         raise ValueError(f"chunks={chunks}, but z holds {s} chunks per track")
-    if s not in (1, 2, 4, 8, 16):
-        raise NotImplementedError("chunks per track must be 1, 2, 4, 8 or 16")
-    if redux not in N.REDUX:
-        raise NotImplementedError(f"redux {redux!r} is not fused into the evaluation (min / max / mean / meanmin / minmean)")
-    if q_chunks is not None and s == 1:
-        raise ValueError("chunk counts need chunked tracks")
+    _check_tracks(s, redux, q_chunks)
     return s
 
 
@@ -231,9 +226,7 @@ def evaluate_all_vs_all(c, i, z, *, precision=None, eps=1e-6, group=None, plan=N
     if side is not None:
         torch.cuda.current_stream(plan.device).wait_stream(side)
         z.record_stream(torch.cuda.current_stream(plan.device))
-    if plan.queries_without_relevant and not allow_empty:
-        raise ValueError(f"{plan.queries_without_relevant} queries have no relevant candidate "
-                         "(every clique needs >= 2 versions; pass allow_empty=True to score the rest)")
+    plan._check_relevant(allow_empty)
     if world == 1:
         res = plan.run(z, z, eps=eps, precision=precision, allow_empty=allow_empty, topk=topk, chunks=chunks, redux=redux,
                        q_chunks=q_chunks)

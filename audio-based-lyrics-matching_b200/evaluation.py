@@ -31,6 +31,24 @@ def _to_device(t, device, dtype=None):
     return t
 
 
+def _check_tracks(s, redux, q_chunks):
+    """What the fused evaluation takes of chunked tracks: s chunks per track, the reduction, and chunk counts only with
+    s > 1."""
+    if s not in (1, 2, 4, 8, 16):
+        raise NotImplementedError("chunks per track must be 1, 2, 4, 8 or 16")
+    if redux not in N.REDUX:
+        raise NotImplementedError(f"redux {redux!r} is not fused into the evaluation (min / max / mean / meanmin / minmean)")
+    if q_chunks is not None and s == 1:
+        raise ValueError("chunk counts need chunked tracks")
+
+
+def _device_view(ptr, n, typestr, device):
+    """1-D tensor over `n` elements of library memory at `ptr` (no copy)."""
+    class _Dev:
+        __cuda_array_interface__ = {"shape": (n,), "typestr": typestr, "data": (ptr, False), "version": 2}
+    return torch.as_tensor(_Dev(), device=device)
+
+
 class EvalPlan:
     """Everything that depends on ids only (clique-sorted candidate order, per-query relevant
     segments, CSR offsets) -- build once per (queries, candidates) id set, run for any embeddings."""
@@ -78,6 +96,11 @@ class EvalPlan:
         except Exception:
             pass
 
+    def _check_relevant(self, allow_empty):
+        if self.queries_without_relevant and not allow_empty:
+            raise ValueError(f"{self.queries_without_relevant} queries have no relevant candidate "
+                             "(every clique needs >= 2 versions; pass allow_empty=True to score the rest)")
+
     # ---- multi-GPU all-vs-all: symmetric sweep sharded by row blocks, rank counts summed over ranks ----
     def _shard_input(self, z, chunks, redux, q_chunks):
         """-> (z [rows, D] on the device, chunks per track, device int32 chunk counts or None) for the sharded entries;
@@ -90,12 +113,7 @@ class EvalPlan:
             chunks = z.shape[1]
             z = z.reshape(-1, z.shape[-1])
         s = 1 if chunks is None else int(chunks)
-        if s not in (1, 2, 4, 8, 16):
-            raise NotImplementedError("chunks per track must be 1, 2, 4, 8 or 16")
-        if redux not in N.REDUX:
-            raise NotImplementedError(f"redux {redux!r} is not fused into the evaluation (min / max / mean / meanmin / minmean)")
-        if q_chunks is not None and s == 1:
-            raise ValueError("chunk counts need chunked tracks")
+        _check_tracks(s, redux, q_chunks)
         assert z.ndim == 2 and z.shape[0] == self.nq * s and self.nq == self.nc
         if z.stride(1) != 1:
             z = z.contiguous()
@@ -168,10 +186,7 @@ class EvalPlan:
         shard_sweep()."""
         ptr, n = ctypes.c_void_p(), ctypes.c_int64()
         N.check(N.lib.wealy_eval_plan_thresholds(self._handle, ctypes.byref(ptr), ctypes.byref(n)))
-
-        class _Dev:
-            __cuda_array_interface__ = {"shape": (n.value,), "typestr": "<f4", "data": (ptr.value, False), "version": 2}
-        return torch.as_tensor(_Dev(), device=self.device)
+        return _device_view(ptr.value, n.value, "<f4", self.device)
 
     def shard_sweep(self, shard_rank, shard_world, *, redux=None, q_chunks=None, chunks=None):
         """Stage 2: this rank's row blocks of the symmetric sweep on the planes / thresholds stage 1 left in the plan.
@@ -201,10 +216,7 @@ class EvalPlan:
         multi-GPU run all-reduces between sweep_shard() and finish()."""
         ptr, n = ctypes.c_void_p(), ctypes.c_int64()
         N.check(N.lib.wealy_eval_plan_counts(self._handle, ctypes.byref(ptr), ctypes.byref(n)))
-
-        class _Dev:
-            __cuda_array_interface__ = {"shape": (n.value,), "typestr": "<i4", "data": (ptr.value, False), "version": 2}
-        return torch.as_tensor(_Dev(), device=self.device)
+        return _device_view(ptr.value, n.value, "<i4", self.device)
 
     def finish(self):
         """Rank counts -> dict(aps, r1s, sums) for ALL queries."""
@@ -253,9 +265,7 @@ class EvalPlan:
         what has arrived (wealy_eval_run_host) -- no separate upload.  Raises NotImplementedError where that pipeline
         does not apply (then upload and call run()); `z` must stay alive until the current stream has drained (the plan
         keeps a reference until its next run)."""
-        if self.queries_without_relevant and not allow_empty:
-            raise ValueError(f"{self.queries_without_relevant} queries have no relevant candidate "
-                             "(every clique needs >= 2 versions; pass allow_empty=True to score the rest)")
+        self._check_relevant(allow_empty)
         assert z.ndim == 2 and z.shape[0] == self.nq == self.nc
         if z.stride(1) != 1:
             raise NotImplementedError("run_host needs contiguous rows")
@@ -281,9 +291,7 @@ class EvalPlan:
         Ragged tracks: `q_chunks[Nq]` / `c_chunks[Nc]` = valid chunks of every track (1 .. s; the remaining rows are
         padding): reduced like `distance_tensor_redux(dist, redux, mask)` with mask = query chunk invalid | candidate
         chunk invalid."""
-        if self.queries_without_relevant and not allow_empty:
-            raise ValueError(f"{self.queries_without_relevant} queries have no relevant candidate "
-                             "(every clique needs >= 2 versions; pass allow_empty=True to score the rest)")
+        self._check_relevant(allow_empty)
         same = queries_z is candidates_z
         qz = _to_device(queries_z, self.device)
         cz = qz if same else _to_device(candidates_z, self.device)
@@ -296,10 +304,7 @@ class EvalPlan:
             qz = qz.reshape(-1, qz.shape[-1])
             cz = qz if same else cz.reshape(-1, cz.shape[-1])
         s = 1 if chunks is None else int(chunks)
-        if s not in (1, 2, 4, 8, 16):
-            raise NotImplementedError("chunks per track must be 1, 2, 4, 8 or 16")
-        if redux not in N.REDUX:
-            raise NotImplementedError(f"redux {redux!r} is not fused into the evaluation (min / max / mean / meanmin / minmean)")
+        _check_tracks(s, redux, q_chunks if q_chunks is not None else c_chunks)
         assert qz.ndim == 2 and cz.ndim == 2 and qz.shape[1] == cz.shape[1]
         assert qz.shape[0] == self.nq * s and cz.shape[0] == self.nc * s
         if qz.dtype != cz.dtype:
@@ -319,30 +324,20 @@ class EvalPlan:
             if not same:
                 raise ValueError("q_chunks and c_chunks go together")
             q_chunks = c_chunks = q_chunks if c_chunks is None else c_chunks
-        if q_chunks is not None:
-            if s == 1:
-                raise ValueError("chunk counts need chunked tracks")
+        entry, lens = N.lib.wealy_eval_run_chunked, ()
+        if q_chunks is not None:                          # ragged tracks: the entry that takes the chunk counts
             ql = torch.as_tensor(q_chunks).to(self.device, torch.int32).contiguous()
             cl = ql if c_chunks is q_chunks else torch.as_tensor(c_chunks).to(self.device, torch.int32).contiguous()
             assert ql.shape == (self.nq,) and cl.shape == (self.nc,)
-            with torch.cuda.device(self.device):
-                N.check(N.lib.wealy_eval_run_ragged(
-                    self._handle, qz.data_ptr(), qz.stride(0), cz.data_ptr(), cz.stride(0), qz.shape[1],
-                    N.dtype_code(qz.dtype), float(eps), passes_of(precision), k, s, N.REDUX[redux], ql.data_ptr(),
-                    cl.data_ptr(), aps.data_ptr(), r1s.data_ptr(), sums.data_ptr(), tk_idx.data_ptr() if k else None,
-                    tk_sim.data_ptr() if k else None, N.stream_ptr(self.device)))
-            ql.record_stream(torch.cuda.current_stream(self.device))
-            cl.record_stream(torch.cuda.current_stream(self.device))
-            out = {"aps": aps, "r1s": r1s, "sums": sums}
-            if k:
-                out["topk_idx"], out["topk_sim"] = tk_idx, tk_sim
-            return out
+            entry, lens = N.lib.wealy_eval_run_ragged, (ql, cl)
         with torch.cuda.device(self.device):
-            N.check(N.lib.wealy_eval_run_chunked(
+            N.check(entry(
                 self._handle, qz.data_ptr(), qz.stride(0), cz.data_ptr(), cz.stride(0), qz.shape[1],
-                N.dtype_code(qz.dtype), float(eps), passes_of(precision), k, s, N.REDUX[redux], aps.data_ptr(),
-                r1s.data_ptr(), sums.data_ptr(), tk_idx.data_ptr() if k else None, tk_sim.data_ptr() if k else None,
-                N.stream_ptr(self.device)))
+                N.dtype_code(qz.dtype), float(eps), passes_of(precision), k, s, N.REDUX[redux],
+                *(t.data_ptr() for t in lens), aps.data_ptr(), r1s.data_ptr(), sums.data_ptr(),
+                tk_idx.data_ptr() if k else None, tk_sim.data_ptr() if k else None, N.stream_ptr(self.device)))
+        for t in lens:
+            t.record_stream(torch.cuda.current_stream(self.device))
         out = {"aps": aps, "r1s": r1s, "sums": sums}
         if k:
             out["topk_idx"], out["topk_sim"] = tk_idx, tk_sim

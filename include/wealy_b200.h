@@ -133,9 +133,7 @@ int wealy_eval_run(wealy_eval_plan* plan, const void* queries_z, int64_t ld_q, c
  * wealy_eval_run on a device copy of host_z.  Work is enqueued on `stream` and on an internal upload stream ordered
  * with it; host_z must stay valid until `stream` has drained.  A device pointer is accepted and takes the plain path;
  * WEALY_ERR_UNSUPPORTED for pageable memory, other shapes or plans (callers then upload and use wealy_eval_run).
- * Environment: WEALY_HOST_UP_SMS (SMs of the upload kernel, default 8; 0 = next to the sweep's CTAs),
- * WEALY_HOST_PARTS (1 / 2 / 5 / 7 parts instead of the size-based choice), WEALY_HOST_TRACE=1 (per-part time stamps
- * on stderr; synchronises).                                                                                    */
+ * Environment: WEALY_HOST_PARTS (1 / 2 / 5 / 7 parts instead of the size-based choice).                          */
 int wealy_eval_run_host(wealy_eval_plan* plan, const void* host_z, int64_t ld, int64_t d, int dtype, float eps, int passes,
                         float* aps, float* r1s, double* sums, void* stream);
 /* wealy_eval_plan_create for a plan that wealy_eval_run_host will run on host_z (same ld / d / dtype / eps / passes): the

@@ -1,5 +1,5 @@
 """Randomised comparison of wealy_eval_run_host (pinned host embeddings, upload / prep / sweep pipeline) with wealy_eval_run
-on a device copy: random sizes / dims / dtypes / row strides / clique structures / part schedules / upload placements.
+on a device copy: random sizes / dims / dtypes / row strides / clique structures / part schedules / early uploads.
 AP, R1, the running sums and the rank of every relevant item must be IDENTICAL (the planes are bit-identical); every
 tenth case is also held against the oracle's rank bands.  One JSON line.  Usage: python tools/fuzz_host.py [seconds] [seed]"""
 import json
@@ -36,8 +36,8 @@ def main():
         if n > 9000:
             d = min(d, 256)
         dtype = rng.choice([torch.float32, torch.float32, torch.float16, torch.bfloat16])
-        parts, up_sms = rng.choice([0, 1, 2, 5, 7]), rng.choice([8, 8, 0, 1, 3, 16])
-        os.environ["WEALY_HOST_PARTS"], os.environ["WEALY_HOST_UP_SMS"] = str(parts), str(up_sms)
+        parts = rng.choice([0, 1, 2, 5, 7])
+        os.environ["WEALY_HOST_PARTS"] = str(parts)
         dist = rng.choice(["shs100k_test", "lyric_covers_test"])
         s = synth.make_eval_set(max(n, 4), d, seed=7000 + k, dist=dist, md5_ids=rng.random() < 0.5)
         c, i, z = s["c"], s["i"], s["z"].to(dtype)
@@ -64,7 +64,7 @@ def main():
         out["relevant_items"] += int(ref_plan.total_pairs)
         out["early_upload_cases"] += int(early)
         if not ok:
-            out["mismatches"].append({"case": k, "n": n, "d": d, "dtype": str(dtype), "parts": parts, "up_sms": up_sms, "early": early})
+            out["mismatches"].append({"case": k, "n": n, "d": d, "dtype": str(dtype), "parts": parts, "early": early})
         if k % 10 == 0 and n <= 6000:
             zf = z.float()
             off_o, _, exact, lo, hi = oev.rank_bands(c, i, zf, c, i, zf, gap=1e-5)

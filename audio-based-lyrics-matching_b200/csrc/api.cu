@@ -1200,8 +1200,8 @@ static int eval_route(const wealy_eval_plan* p, const EvalCall& c, bool try_sym_
   const int chunks = c.chunks;
   // (the staged sweep has no embeddings of its own: those of the prepare, queries == candidates)
   r.same = (staged_sweep || (c.q_z == c.c_z && c.ld_q == c.ld_c)) && nq == nc;
-  if (chunks != 1 && chunks != 2 && chunks != 4 && chunks != 8 && chunks != 16)
-    return fail(WEALY_ERR_UNSUPPORTED, "chunks per track must be 1, 2, 4, 8 or 16, got %d", chunks);
+  if (chunks != 1 && chunks != 2 && chunks != 4 && chunks != 8 && chunks != 16 && chunks != 32)
+    return fail(WEALY_ERR_UNSUPPORTED, "chunks per track must be 1, 2, 4, 8, 16 or 32, got %d", chunks);
   if (c.redux < WEALY_REDUX_MIN || c.redux > WEALY_REDUX_MINMEAN) return fail(WEALY_ERR_BAD_ARG, "unknown redux %d", c.redux);
   if ((c.q_len == nullptr) != (c.c_len == nullptr)) return fail(WEALY_ERR_BAD_ARG, "q_len and c_len go together");
   if (c.q_len && chunks == 1) return fail(WEALY_ERR_BAD_ARG, "chunk counts need chunks > 1");
@@ -1353,8 +1353,9 @@ static int eval_kpos(wealy_eval_plan* p, const EvalCall& c, const EvalRoute& r, 
       q_hi = (int)(nq * (c.shard_rank + 1) / c.shard_world);
       CU_TRY(cudaMemsetAsync(p->thr, 0, pair_slots(p) * 4, s));
     }
+    auto kpos_tracks = c.chunks == 32 ? pos_thresholds_tracks_kernel<true> : pos_thresholds_tracks_kernel<false>;
     if (q_hi > q_lo)
-      pos_thresholds_tracks_kernel<<<(unsigned)(q_hi - q_lo), threads, 0, s>>>(
+      kpos_tracks<<<(unsigned)(q_hi - q_lo), threads, 0, s>>>(
           pq.hi, pq.lo, pc.hi, pc.lo, (int)pq.d_pad, c.chunks, r.red_inner, r.red_outer, r.red_scale, p->q_i, (int)nq,
           p->sorted_idx, p->c_i, p->seg_lo, p->seg_len, p->off, p->raw, p->thr, p->lim, p->cnt, c.q_len, c.c_len, q_lo);
   } else if (r.same && p->same_ids && nq > 0) {
@@ -1504,6 +1505,8 @@ static int eval_sweep(wealy_eval_plan* p, const EvalCall& c, const EvalRoute& r,
     W_TRY(launch_eval_tracks<8>(c.passes, pq, pc, sh, ep, s, half, c.shard_rank, c.shard_world));
   } else if (c.chunks == 16) {
     W_TRY(launch_eval_tracks<16>(c.passes, pq, pc, sh, ep, s, half, c.shard_rank, c.shard_world));
+  } else if (c.chunks == 32) {
+    W_TRY(launch_eval_tracks<32>(c.passes, pq, pc, sh, ep, s, half, c.shard_rank, c.shard_world));
   } else {
     W_TRY(launch_gemm_rect<EvalEpi>(c.passes, pq, pc, sh, ep, s));
   }
@@ -1935,14 +1938,14 @@ extern "C" int wealy_eval_plan_thresholds(const wealy_eval_plan* p, void** value
   return WEALY_OK;
 }
 
-// Chunked tracks (chunks in {2, 4, 8, 16}, redux WEALY_REDUX_*, lens = NULL or the ragged chunk counts of every track):
+// Chunked tracks (chunks in {2, 4, 8, 16, 32}, redux WEALY_REDUX_*, lens = NULL or the ragged chunk counts of every track):
 // the same three steps.  min / max / mean take the half sweep, the other reductions (and small sets, WEALY_SYM_TRACKS=0)
 // the rectangle sweep; either way sharded by row blocks.
 static int check_shard_tracks(const wealy_eval_plan* p, int chunks) {
   if (!p) return fail(WEALY_ERR_BAD_ARG, "null plan");
   if (!p->same_ids) return fail(WEALY_ERR_BAD_ARG, "a sharded sweep needs queries == candidates (ids and embeddings) and no top-k");
-  if (chunks != 2 && chunks != 4 && chunks != 8 && chunks != 16)
-    return fail(WEALY_ERR_UNSUPPORTED, "chunked tracks have 2, 4, 8 or 16 chunks, got %d", chunks);
+  if (chunks != 2 && chunks != 4 && chunks != 8 && chunks != 16 && chunks != 32)
+    return fail(WEALY_ERR_UNSUPPORTED, "chunked tracks have 2, 4, 8, 16 or 32 chunks, got %d", chunks);
   return WEALY_OK;
 }
 

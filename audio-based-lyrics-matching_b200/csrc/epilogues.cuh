@@ -308,8 +308,12 @@ __device__ __forceinline__ float red_neutral(int op) {
 // thresholds of their column query).
 template <int kQueueCapT, int kCachePairsT, int kS = 1, bool kSym = false>
 struct EvalEpiT {
-  static_assert(kS == 1 || kS == 2 || kS == 4 || kS == 8 || kS == 16, "chunks per track: a power of two <= 16");
-  static constexpr int kGroups = 32 / kS;  // tracks per 32-row / 32-column chunk
+  static_assert(kS == 1 || kS == 2 || kS == 4 || kS == 8 || kS == 16 || kS == 32, "chunks per track: a power of two <= 32");
+  // tracks per 32-row / 32-column chunk.  kS = 32 (kGroups = 1): a warp's 32 rows are one query track and a chunk's 32
+  // columns one candidate track -- the reduction over the candidate's chunks stays in the lane's 32 registers, the one
+  // over the query's chunks takes the whole warp's shuffles, lane 0 carries the track's state, and every expression
+  // below holds with a single group (64 chunks would put one track's rows in two epilogue warps)
+  static constexpr int kGroups = 32 / kS;
   using Params = EvalParams;
   // Shared-memory scratch of the epilogue.
   //  * per warp, a work queue: the elements that pass the per-row limit are scattered unevenly over

@@ -142,14 +142,100 @@ __device__ __forceinline__ void mma_16x8x16(float (&c)[4], const unsigned (&a)[4
       : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b[0]), "r"(b[1]));
 }
 
+// K_pos of one query track at 32 chunks per track (pos_thresholds_tracks_kernel below): warp `warp` of the CTA takes the
+// relevant candidates warp, warp + 8, ..., one at a time.  A candidate's 32 chunks fill the rows of TWO m16n8k16 tiles
+// (rows g and g + 8 of row tile rt are its chunks 16 rt + g and 16 rt + g + 8), the query's 32 chunks the columns of FOUR
+// (column 2 tig + e of query tile t is its chunk 8 t + 2 tig + e).  Every (query tile, row tile) is contracted exactly as
+// in the 16-chunk layout -- two accumulators on alternate k windows, summed -- so a chunk pair's similarity is the one the
+// narrower layouts compute.  The reduction over the candidate's chunks folds the lane's two rows of each row tile, then
+// the 8 row groups g; it goes into the reduction over the query's chunks (the lane's two columns of every query tile,
+// then the 4 lanes tig).  Ragged counts select, so padding rows may hold anything; lane 0 writes the value.
+__device__ __forceinline__ void pos_tracks32_candidates(
+    const __half* __restrict__ q_hi, const __half* __restrict__ q_lo, const __half* __restrict__ c_hi,
+    const __half* __restrict__ c_lo, int d_pad, int red_inner, int red_outer, float red_scale, int q, int qi, int lq,
+    int first, int len, const int* __restrict__ sorted_idx, const int* __restrict__ c_i, const int* __restrict__ c_len,
+    float* __restrict__ raw, long long o, int* n_sh, int lane, int warp) {
+  constexpr int ks = 32;
+  const int g = lane >> 2, tig = lane & 3;
+  const bool ragged = c_len != nullptr;
+  const float n_in = red_neutral(red_inner), n_out = red_neutral(red_outer);
+  for (int m = warp; m < len; m += 8) {
+    const int j = sorted_idx[first + m];
+    if (c_i[j] == qi) continue;  // self / id collision: not a candidate (the whole warp skips it)
+    const int lc = ragged ? min(max(c_len[j], 1), ks) : ks;
+    float w = n_out;  // outer reduction (over the query's chunks)
+    for (int t = 0; t < 4; ++t) {
+      const long long rq = ((long long)q * ks + t * 8 + g) * d_pad;  // B column g = query chunk t * 8 + g
+      float in[2];  // inner reduction (over the candidate's chunks) of query chunks t * 8 + 2 tig + e
+      for (int rt = 0; rt < 2; ++rt) {
+        const int cA = 16 * rt + g, cB = cA + 8;  // the candidate's chunks in tile rows g, g + 8
+        const long long rA = ((long long)j * ks + cA) * d_pad, rB = rA + 8ll * d_pad;
+        float c0[4] = {0.f, 0.f, 0.f, 0.f}, c1[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll 2  // (ptxas unrolls further on its own, to 80 registers with spills)
+        for (int k = 0; k < d_pad; k += 64) {
+#pragma unroll
+          for (int u = 0; u < 2; ++u) {
+            float (&c)[4] = u ? c1 : c0;
+            const int ko = k + u * 32 + tig * 8;
+            const uint4 ah0 = __ldg(reinterpret_cast<const uint4*>(c_hi + rA + ko));
+            const uint4 ah1 = __ldg(reinterpret_cast<const uint4*>(c_hi + rB + ko));
+            const uint4 bh = __ldg(reinterpret_cast<const uint4*>(q_hi + rq + ko));
+            const unsigned a1[4] = {ah0.x, ah1.x, ah0.y, ah1.y}, a2[4] = {ah0.z, ah1.z, ah0.w, ah1.w};
+            const unsigned b1[2] = {bh.x, bh.y}, b2[2] = {bh.z, bh.w};
+            mma_16x8x16(c, a1, b1);
+            mma_16x8x16(c, a2, b2);
+            if (q_lo) {
+              const uint4 al0 = __ldg(reinterpret_cast<const uint4*>(c_lo + rA + ko));
+              const uint4 al1 = __ldg(reinterpret_cast<const uint4*>(c_lo + rB + ko));
+              const uint4 bl = __ldg(reinterpret_cast<const uint4*>(q_lo + rq + ko));
+              const unsigned l1[4] = {al0.x, al1.x, al0.y, al1.y}, l2[4] = {al0.z, al1.z, al0.w, al1.w};
+              const unsigned m1[2] = {bl.x, bl.y}, m2[2] = {bl.z, bl.w};
+              mma_16x8x16(c, a1, m1);
+              mma_16x8x16(c, a2, m2);
+              mma_16x8x16(c, l1, b1);
+              mma_16x8x16(c, l2, b2);
+            }
+          }
+        }
+        // c[e], c[2 + e]: tile rows g, g + 8 against query chunk t * 8 + 2 tig + e
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+          const float vA = cA < lc ? c0[e] + c1[e] : n_in;
+          const float vB = cB < lc ? c0[2 + e] + c1[2 + e] : n_in;
+          const float v = red_op(vA, vB, red_inner);
+          in[e] = rt == 0 ? v : red_op(in[e], v, red_inner);
+        }
+      }
+#pragma unroll
+      for (int e = 0; e < 2; ++e) {
+        float v = in[e];
+#pragma unroll
+        for (int x = 4; x < 32; x <<= 1) v = red_op(v, __shfl_xor_sync(0xffffffffu, v, x), red_inner);
+        if (ragged) {
+          if (red_inner == kRedSum) v *= 1.f / (float)lc;
+        } else if (red_inner == kRedSum && red_outer != kRedSum) {
+          v *= red_scale;
+        }
+        if (t * 8 + 2 * tig + e < lq) w = red_op(w, v, red_outer);
+      }
+    }
+#pragma unroll
+    for (int x = 1; x < 4; x <<= 1) w = red_op(w, __shfl_xor_sync(0xffffffffu, w, x), red_outer);
+    if (red_outer == kRedSum) w *= ragged ? 1.f / (float)lq : red_scale;
+    if (lane == 0) raw[o + atomicAdd(n_sh, 1)] = w;
+  }
+}
+
 // K_pos for chunked tracks (row f1).  One CTA (8 warps) per query track: for every relevant candidate track the kS x kS chunk
 // similarities (same planes, same three products as the sweep) are reduced exactly like the sweep's epilogue does
 // (red_inner over the candidate's chunks, red_outer over the query's), then rank-sorted ascending.
 // The kS x kS blocks come from warp-level tensor-core tiles m16n8k16 read straight from the planes: the 16 tile ROWS
 // are candidate chunks -- 16 / kS whole candidates per tile for kS <= 8 (eight two-chunk tracks, two eight-chunk
-// tracks), one for kS = 16 -- and the 8 tile COLUMNS the query's chunks (two tiles for kS = 16), so a warp reads the
-// query's rows once for all the candidates of its tile.  Two accumulators take alternate k windows (the dependent MMA
-// chain is what bounds a warp).  Block b takes query track q_lo + b (a multi-GPU run gives every rank a share).
+// tracks), one for kS = 16, two tiles per candidate for kS = 32 (pos_tracks32_candidates) -- and the 8 tile COLUMNS the
+// query's chunks (two tiles for kS = 16, four for kS = 32), so a warp reads the query's rows once for all the candidates
+// of its tile.  Two accumulators take alternate k windows (the dependent MMA chain is what bounds a warp).  Block b takes
+// query track q_lo + b (a multi-GPU run gives every rank a share).
+template <bool k32>  // ks == 32 (pos_tracks32_candidates), else ks <= 16
 __global__ void __launch_bounds__(256) pos_thresholds_tracks_kernel(
     const __half* __restrict__ q_hi, const __half* __restrict__ q_lo, const __half* __restrict__ c_hi,
     const __half* __restrict__ c_lo, int d_pad, int ks, int red_inner, int red_outer, float red_scale,
@@ -178,7 +264,10 @@ __global__ void __launch_bounds__(256) pos_thresholds_tracks_kernel(
   const int sB = wide ? 0 : (g + 8) / ks, cB = wide ? g + 8 : (g + 8) % ks;
   const int ntile = wide ? 2 : 1;
   const float n_in = red_neutral(red_inner), n_out = red_neutral(red_outer);
-  for (int m0 = warp * per; m0 < len; m0 += 8 * per) {
+  if constexpr (k32)
+    pos_tracks32_candidates(q_hi, q_lo, c_hi, c_lo, d_pad, red_inner, red_outer, red_scale, q, qi, lq, first, len,
+                            sorted_idx, c_i, c_len, raw, o, &n_sh, lane, warp);
+  for (int m0 = warp * per; !k32 && m0 < len; m0 += 8 * per) {  // (kS <= 16: the layouts above)
     const int mA = m0 + sA, mB = m0 + sB;
     const int jA = mA < len ? sorted_idx[first + mA] : -1;
     const int jB = mB < len ? sorted_idx[first + mB] : -1;

@@ -34,8 +34,8 @@ def _to_device(t, device, dtype=None):
 def _check_tracks(s, redux, q_chunks):
     """What the fused evaluation takes of chunked tracks: s chunks per track, the reduction, and chunk counts only with
     s > 1."""
-    if s not in (1, 2, 4, 8, 16):
-        raise NotImplementedError("chunks per track must be 1, 2, 4, 8 or 16")
+    if s not in (1, 2, 4, 8, 16, 32):
+        raise NotImplementedError("chunks per track must be 1, 2, 4, 8, 16 or 32")
     if redux not in N.REDUX:
         raise NotImplementedError(f"redux {redux!r} is not fused into the evaluation (min / max / mean / meanmin / minmean)")
     if q_chunks is not None and s == 1:
@@ -284,7 +284,7 @@ class EvalPlan:
         """-> dict(aps, r1s, sums[, topk_idx, topk_sim]); `sums` = device doubles {sum AP, sum R1, #scored}.
 
         Chunked tracks (SURVEY.md 8(f) row f1): pass `[N, s, D]` embeddings (or `[N * s, D]` with `chunks=s`,
-        s in {2, 4, 8, 16}): the s x s chunk distances of every track pair are reduced like
+        s in {2, 4, 8, 16, 32}): the s x s chunk distances of every track pair are reduced like
         `distance_tensor_redux(dist, redux)` (lib/tensor_ops.py:288-373; redux in min / max / mean / meanmin /
         minmean) inside the sweep's epilogue before ranking; ids and results are per track.
 
@@ -373,7 +373,12 @@ def evaluate(queries_c, queries_i, queries_z, candidates_c, candidates_i, candid
     """-> (aps[Nq], r1s[Nq]) or (aps, r1s, topk_idx[Nq,k], topk_sim[Nq,k]) on the CUDA device.
 
     AP_q = 1/P sum_{p relevant} rank_rel(p) / rank_all(p); R1_q = rank of the best relevant item;
-    self (candidates_i == queries_i) is excluded, relevant = same clique and not self."""
+    self (candidates_i == queries_i) is excluded, relevant = same clique and not self.
+
+    Chunked tracks ([N, s, D] embeddings or chunks=s, s in {2, 4, 8, 16, 32}; redux, q_chunks / c_chunks as in
+    EvalPlan.run): up to 32 chunks per track.  Every track pays for s rows whatever its valid count, so the tensor work
+    grows with (N * s)^2: pass the smallest s that holds the longest track (a set whose longest track has 17 chunks
+    takes s = 32, one whose longest has 9 takes s = 16)."""
     if mode not in ("cos", "cossim"):
         raise NotImplementedError("wealy_b200.evaluate ranks by cosine distance (mode='cos')")
     own = plan is None

@@ -146,9 +146,9 @@ int wealy_eval_plan_create_host(const int64_t* queries_c, const int64_t* queries
                                 int64_t ld, int64_t d, int dtype, float eps, int passes, void* stream,
                                 wealy_eval_plan** plan);
 
-/* f1 (SURVEY.md section 8(f)): evaluation of CHUNKED tracks -- every track has `chunks` (1, 2, 4, 8 or 16) embeddings,
- * queries_z [nq * chunks, d] / candidates_z [nc * chunks, d] (the chunks of a track are consecutive rows), the plan's ids
- * are per track.  The chunk-level cosine distances of a track pair are reduced like
+/* f1 (SURVEY.md section 8(f)): evaluation of CHUNKED tracks -- every track has `chunks` (1, 2, 4, 8, 16 or 32)
+ * embeddings, queries_z [nq * chunks, d] / candidates_z [nc * chunks, d] (the chunks of a track are consecutive rows),
+ * the plan's ids are per track.  The chunk-level cosine distances of a track pair are reduced like
  * distance_tensor_redux(dist[b1, b2, s1, s2], redux) of lib/tensor_ops.py:288-373 INSIDE the sweep's epilogue (the 4-D
  * tensor is never materialised), then ranked as in wealy_eval_run.  topk_sim holds 1 - reduced distance.             */
 enum { WEALY_REDUX_MIN = 0, WEALY_REDUX_MAX = 1, WEALY_REDUX_MEAN = 2, WEALY_REDUX_MEANMIN = 3, WEALY_REDUX_MINMEAN = 4 };
@@ -181,9 +181,9 @@ int wealy_eval_shard_prepare(wealy_eval_plan* plan, const void* z, int64_t ld, i
                              int shard_rank, int shard_world, void* stream);
 int wealy_eval_plan_thresholds(const wealy_eval_plan* plan, void** values, int64_t* count);
 int wealy_eval_shard_sweep(wealy_eval_plan* plan, int64_t d, int passes, int shard_rank, int shard_world, void* stream);
-/* Multi-GPU all-vs-all of CHUNKED tracks (z [n * chunks, d], chunks in {2, 4, 8, 16}, redux WEALY_REDUX_*; lens NULL for
- * full tracks, else the device int32 [n] ragged chunk counts, used for both sides as in wealy_eval_run_ragged).  The
- * same protocol as above: every rank sweeps the row blocks rb = shard_rank (mod shard_world) of the chunked sweep --
+/* Multi-GPU all-vs-all of CHUNKED tracks (z [n * chunks, d], chunks in {2, 4, 8, 16, 32}, redux WEALY_REDUX_*; lens
+ * NULL for full tracks, else the device int32 [n] ragged chunk counts, used for both sides as in
+ * wealy_eval_run_ragged).  The same protocol as above: every rank sweeps the row blocks rb = shard_rank (mod shard_world) of the chunked sweep --
  * the half sweep for min / max / mean, the rectangle for meanmin / minmean (or WEALY_SYM_TRACKS=0) -- then the counts
  * are summed over the ranks and wealy_eval_finish yields the per-track AP / R1.  No top-k; queries must be the
  * candidates (WEALY_ERR_BAD_ARG otherwise), other chunk counts WEALY_ERR_UNSUPPORTED.

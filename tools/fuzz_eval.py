@@ -17,7 +17,7 @@ from wealy_b200.data import synth  # noqa: E402
 
 
 def one_case(rng, k):
-    chunks = rng.choice([1, 1, 1, 2, 4, 8, 16])
+    chunks = rng.choice([1, 1, 1, 2, 4, 8, 16, 32])
     n = rng.randint(260, 5000) if chunks == 1 else rng.randint(max(40, 300 // chunks), 2400 // chunks * 2)
     d = rng.choice([24, 48, 64, 100, 128, 200, 256, 333, 512, 1024])
     dtype = rng.choice([torch.float32, torch.float32, torch.float16, torch.bfloat16])
